@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Headline benchmark: LDE + Merkle commit throughput (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one PolynomialBatch::from_coeffs commit (plonky2/src/fri/oracle.rs:68-98) of
 135 polynomials of degree 2^20 at rate_bits 3, cap_height 4 (BASELINE.json configs[3]):
@@ -22,6 +22,12 @@ value = W*N elems / max-over-ranks time.
 
 --impl reference times the CPU port of the reference (oracle/) with all host threads on a bounded
 sample of the same workload; rank 0 only.
+
+--dump-outputs DIR writes what the last timed commit computed, so that two builds can be compared output for output
+(the inputs are the same seeded polynomials on every run): DIR/cap.npy [2^cap_height][4][2], and for a fixed, seeded
+sample of leaves DIR/leaf_indices.npy [k], DIR/leaves.npy [k][width][2] (the LDE rows) and DIR/merkle_paths.npy
+[k][log2 N - cap_height][4][2] (MerkleTree::prove).  Field elements are 64-bit, so every one is stored as its low and
+high 32-bit halves (last axis), which float64 holds exactly; the files stay below 64 MB in all.
 """
 import argparse
 import ctypes as C
@@ -99,7 +105,13 @@ def parse():
                          "geometrically growing groups, only the first 8-polynomial transfer is exposed")
     ap.add_argument("--exchange", default="auto", choices=["auto", "allgather", "peer", "alltoall"],
                     help="N > 1: how coefficient blocks reach the other ranks (plonky2_demo_b200/sharded.py)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed commit computed to DIR/<name>.npy (float64)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return a
 
 
 def workload_name(a):
@@ -133,6 +145,26 @@ def cpu_commit_once(width, lg_d, rate_bits, cap_height, keep=False):
     cap = out["cap"].copy()
     del out
     return dt, cap
+
+
+DUMP_BUDGET_BYTES = 48 << 20
+
+
+def dump_sample(n_leaves, leaf_len, depth):
+    """--dump-outputs: the same sorted leaf indices on every run, as many as fit the budget (4096 at most)."""
+    per_leaf = 8 + 16 * (leaf_len + 4 * depth)
+    k = max(1, min(n_leaves, 4096, DUMP_BUDGET_BYTES // per_leaf))
+    return np.sort(np.random.default_rng(0x5EED).choice(n_leaves, size=k, replace=False)).astype(np.uint64)
+
+
+def write_outputs(out_dir, leaf_indices, field_arrays):
+    """leaf_indices as float64 (exact below 2^53); field elements as float64 [..., 2] = (low, high) 32-bit halves."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "leaf_indices.npy"), leaf_indices.astype(np.float64))
+    for name, a in field_arrays.items():
+        a = np.asarray(a, dtype=np.uint64)
+        np.save(os.path.join(out_dir, name + ".npy"),
+                np.stack([a & np.uint64(0xFFFFFFFF), a >> np.uint64(32)], axis=-1).astype(np.float64))
 
 
 def _mem_available_bytes():
@@ -599,6 +631,7 @@ def run_ours(a):
     e1.record(stream)
     barrier()
     t_wall1 = time.perf_counter()
+    clocks = sampler.stop(t_wall0, t_wall1)
     ms_total = e0.elapsed_time(e1)
     cap_dev = np.empty((1 << cap_h, 4), dtype=np.uint64)
     prev_exchange = prev.b.exchange if world > 1 else "none"
@@ -606,13 +639,28 @@ def run_ours(a):
         cap_dev[:] = prev.b.cap
     else:
         _ffi.check(L.pcs_batch_cap(prev, _ffi.ptr(cap_dev)))
+    dump = None
+    if a.dump_outputs:
+        # read back while the last batch is alive; the reads launch no commit, so the phase totals below stay the timed ones
+        depth = lg_d + r - cap_h
+        idx = dump_sample(n, w, depth)
+        if world > 1:
+            rows = prev.b.get_rows(idx)
+            paths = np.stack([p.siblings for p in prev.b.prove_many(idx)])
+        else:
+            rows = np.empty((idx.size, w), dtype=np.uint64)
+            _ffi.check(L.pcs_batch_get_rows(prev, _ffi.ptr(idx), idx.size, _ffi.ptr(rows)))
+            paths = np.empty((idx.size, depth, 4), dtype=np.uint64)
+            _ffi.check(L.pcs_batch_prove_many(prev, _ffi.ptr(idx), idx.size, _ffi.ptr(paths)))
+        dump = (idx, {"cap": cap_dev.copy(), "leaves": rows, "merkle_paths": paths})
     free(prev)
     ms5 = (C.c_float * 5)()
     ncommit = C.c_uint()
     _ffi.check(L.pcs_timing_totals(ms5, C.byref(ncommit), 1))
     assert ncommit.value == a.steps, (ncommit.value, a.steps)
     phase = np.array(list(ms5)) / a.steps
-    clocks = sampler.stop(t_wall0, t_wall1)
+    if dump is not None and rank == 0:
+        write_outputs(a.dump_outputs, *dump)
 
     t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     if world > 1:

@@ -466,3 +466,39 @@ def test_coset_lde_dev_is_the_leaf_order_lde(pcs):
         _ffi.check(_ffi.lib().pcs_coset_lde_dev(ptrs, w, lg_d, r, 7, C.c_void_p(out.data_ptr())))
         pcs.synchronize()
         assert np.array_equal(out.cpu().numpy().view(np.uint64), ref)
+
+
+def test_bench_dump_outputs_hold_the_last_timed_commit(tmp_path):
+    """bench.py --dump-outputs at a small shape: the files hold the commitment of the benchmark's seeded inputs bit for bit
+    (cap, the sampled LDE rows and their Merkle paths, every element as float64 low / high 32-bit halves)."""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    w, lg_d, r, cap_h = 9, 10, 3, 4
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "0", "--width", str(w),
+                          "--lg-d", str(lg_d), "--rate-bits", str(r), "--cap-height", str(cap_h), "--no-fri", "--no-e2e",
+                          "--no-from-values", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == 2
+    files = {f: np.load(tmp_path / f"{f}.npy") for f in ("cap", "leaf_indices", "leaves", "merkle_paths")}
+    assert all(a.dtype == np.float64 for a in files.values())
+    assert sum(a.nbytes for a in files.values()) <= 64 << 20
+
+    def join(a):
+        assert np.all(a >= 0) and np.all(a < 2.0 ** 32) and np.all(a == np.floor(a))
+        return a[..., 0].astype(np.uint64) | (a[..., 1].astype(np.uint64) << np.uint64(32))
+
+    n = 1 << (lg_d + r)
+    ref = oracle.commit_from_coeffs(seeded_polys(w, 1 << lg_d), r, cap_h)
+    idx = files["leaf_indices"].astype(np.int64)
+    assert idx.size == 4096 and np.all(np.diff(idx) > 0) and idx[-1] < n
+    assert np.array_equal(join(files["cap"]), ref["cap"])
+    assert np.array_equal(join(files["leaves"]), ref["leaves"][idx])
+    paths = join(files["merkle_paths"])
+    assert paths.shape == (idx.size, lg_d + r - cap_h, 4)
+    for k in range(0, idx.size, 97):
+        assert np.array_equal(paths[k], oracle.merkle_prove(ref["digests"], n, cap_h, int(idx[k])))

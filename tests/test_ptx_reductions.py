@@ -16,15 +16,12 @@ M32, M64 = E.M32, E.M64
 BIAS = 0x43300000
 
 
-def _src():
+def _src(tmp_dir):
     text = "".join(l for l in open(HDR) if not l.startswith(("#include", "#pragma once")))
-    tmp = os.path.join("/tmp", f"gl64_{os.getpid()}.h")
+    tmp = os.path.join(tmp_dir, "gl64.h")
     with open(tmp, "w") as f:
         f.write(text)
-    try:
-        return E.preprocess(tmp, {})
-    finally:
-        os.unlink(tmp)
+    return E.preprocess(tmp, {})
 
 
 def _grid64():
@@ -53,8 +50,8 @@ def _rand64(rng, n):
 
 
 @pytest.fixture(scope="module")
-def src():
-    return _src()
+def src(tmp_path_factory):
+    return _src(str(tmp_path_factory.mktemp("ptx")))
 
 
 REDUCE128 = ["reduce128_limbs", "reduce128_limbs_sub", "reduce128_wide", "reduce128_mad"]   # forms 0, 1, 2 and the NTT's
