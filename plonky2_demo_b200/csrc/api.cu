@@ -61,20 +61,25 @@ static Ctx* ctx_enter(Ctx* c) {
     }
     return prev;
 }
+// The five phase times of a committed batch (or of the events a freed one left pending) from its six events.  Leaf hashing
+// that ran group by group inside the "FFT + blinding" phase (streaming sponge) is booked as leaf hashing.
+template <class Events>
+static int phase_times(const Events* b, float ms[5]) {
+    for (int i = 0; i < 5; i++) PCS_CUDA(cudaEventElapsedTime(&ms[i], b->ev[i], b->ev[i + 1]));
+    for (size_t k = 0; k + 1 < b->absorb_ev.size(); k += 2) {
+        float t = 0;
+        PCS_CUDA(cudaEventElapsedTime(&t, b->absorb_ev[k], b->absorb_ev[k + 1]));
+        ms[1] -= t;
+        ms[3] += t;
+    }
+    return PCS_OK;
+}
+
 // fold completed/pending event sets into the running totals (caller has synchronised the stream)
 static void drain_pending() {
     for (auto& pe : g_ctx.pending) {
-        bool ok = true;
         float ms[5];
-        for (int i = 0; i < 5 && ok; i++) ok = cudaEventElapsedTime(&ms[i], pe.ev[i], pe.ev[i + 1]) == cudaSuccess;
-        // leaf hashing that ran group by group inside the "FFT + blinding" phase (streaming sponge) is booked as leaf hashing
-        for (size_t k = 0; k + 1 < pe.absorb_ev.size() && ok; k += 2) {
-            float t = 0;
-            ok = cudaEventElapsedTime(&t, pe.absorb_ev[k], pe.absorb_ev[k + 1]) == cudaSuccess;
-            ms[1] -= t;
-            ms[3] += t;
-        }
-        if (ok) {
+        if (phase_times(&pe, ms) == PCS_OK) {
             for (int i = 0; i < 5; i++) g_ctx.totals[i] += ms[i];
             g_ctx.n_totals++;
         }
@@ -107,15 +112,11 @@ pcs_batch* batch_new() {
     return b;
 }
 
-#define PCS_NEED_INIT()                                                            \
-    do {                                                                           \
-        if (!g_ctx.init) {                                                         \
-            int _rc = pcs_init(-1, nullptr);                                       \
-            if (_rc) return _rc;                                                   \
-        } else {                                                                   \
-            cudaSetDevice(g_ctx.device); /* the caller (torch ...) may have switched this thread's device */ \
-        }                                                                          \
-    } while (0)
+int need_init() {
+    if (!g_ctx.init) return pcs_init(-1, nullptr);
+    cudaSetDevice(g_ctx.device);
+    return PCS_OK;
+}
 
 static int node_levels_dev(size_t n, unsigned lg_sub, uint64_t* digests, uint64_t* cap, cudaStream_t st) {
     // one launch per level while a level still fills the GPU (more than 256 nodes per cap subtree), then the top of every
@@ -166,6 +167,72 @@ static int absorb_columns(pcs_batch* b, size_t upto, bool last, cudaStream_t st,
     if (last && b->sponge) {
         cudaFreeAsync(b->sponge, st);
         b->sponge = nullptr;
+    }
+    return PCS_OK;
+}
+
+int batch_begin(size_t w, size_t salt_w, unsigned lg_d, unsigned rate_bits, unsigned coset_first, unsigned lg_cosets,
+                unsigned cap_height, unsigned kind, BatchOwner& out) {
+    if (int rc = check_two_adicity(lg_d + rate_bits)) return rc;
+    if (lg_cosets > rate_bits || ((size_t)coset_first + ((size_t)1 << lg_cosets)) > ((size_t)1 << rate_bits))
+        return fail(PCS_ERR_ARG, "coset range outside [0, 2^rate_bits)");
+    const unsigned lg_n = lg_d + lg_cosets;   // leaves of this (shard of the) tree
+    if (int rc = check_cap_height(cap_height, lg_n)) return rc;
+    cudaStream_t st = g_ctx.stream;
+    if (!(kind & BATCH_ROWS) && !ntt_plan_get(lg_d, rate_bits, false, 7 /* F::coset_shift(), types.rs:437 */, st))
+        return fail(PCS_ERR_ALLOC, "twiddle table allocation failed");
+    const size_t n = (size_t)1 << lg_n, n_cap = (size_t)1 << cap_height;
+    BatchOwner b(batch_new());
+    b->w = w; b->salt_w = salt_w; b->lg_d = lg_d; b->rate_bits = lg_cosets; b->cap_height = cap_height;
+    b->full_rate_bits = rate_bits; b->coset_first = coset_first; b->rows_only = kind & BATCH_ROWS;
+    b->n = n; b->n_digests = 2 * (n - n_cap);
+    if (!(kind & BATCH_UNTIMED))
+        for (auto& e : b->ev) PCS_CUDA(cudaEventCreate(&e));
+    PCS_CUDA(cudaMallocAsync((void**)&b->lde, (w + salt_w) * n * 8, st));
+    PCS_CUDA(cudaMallocAsync((void**)&b->digests, b->n_digests ? b->n_digests * 32 : 32, st));
+    PCS_CUDA(cudaMallocAsync((void**)&b->cap, n_cap * 32, st));
+    out = std::move(b);
+    return PCS_OK;
+}
+
+int batch_extend(pcs_batch* b, const uint64_t* src, const uint64_t* const* ptr_table, size_t first, size_t count) {
+    cudaStream_t st = g_ctx.stream;
+    NttPlan* plan = ntt_plan_get(b->lg_d, b->full_rate_bits, false, 7, st);
+    if (!plan) return fail(PCS_ERR_ALLOC, "twiddle table allocation failed");
+    PCS_CUDA(ntt_lde_cosets(plan, src, (size_t)1 << b->lg_d, b->lde + first * b->n, b->n, count, b->coset_first, b->rate_bits, st,
+                            ptr_table));
+    // streaming sponge: groups that arrive in order are hashed at once, up to a multiple of the sponge rate, while later
+    // groups are still in flight; the last group is absorbed by batch_finish together with the salt columns, and a batch
+    // that gets all its polynomials in one call keeps the single hash kernel
+    if (first == b->extended) b->extended += count;
+    const bool whole = first == 0 && count == b->w;
+    if (!whole && b->w + b->salt_w > 4 && b->extended < b->w) return absorb_columns(b, (b->extended / 8) * 8, false, st, true);
+    return PCS_OK;
+}
+
+int batch_finish(pcs_batch* b, uint64_t* cap_out) {
+    cudaStream_t st = g_ctx.stream;
+    PCS_CUDA(cudaEventRecord(b->ev[2], st));
+    // "transpose LDEs" (oracle.rs:83): fused away -- the hash kernel reads columns directly
+    PCS_CUDA(cudaEventRecord(b->ev[3], st));
+    // "build Merkle tree" (oracle.rs:85-89)
+    const size_t wt = b->w + b->salt_w;
+    const unsigned lg_n = b->lg_d + b->rate_bits;
+    int rc;
+    if (b->absorbed > 0) {
+        rc = absorb_columns(b, wt, true, st, false);     // the remaining columns (+ salts) and the digests
+        if (rc) return rc;
+        PCS_CUDA(cudaEventRecord(b->ev[4], st));
+        rc = node_levels_dev(b->n, lg_n - b->cap_height, b->digests, b->cap, st);
+    } else {
+        rc = build_tree_dev(b->lde, b->n, wt, lg_n, b->cap_height, b->digests, b->cap, st, b->ev[4]);
+    }
+    if (rc) return rc;
+    PCS_CUDA(cudaEventRecord(b->ev[5], st));
+    b->committed = true;
+    if (cap_out) {
+        PCS_CUDA(cudaMemcpyAsync(cap_out, b->cap, ((size_t)32) << b->cap_height, cudaMemcpyDeviceToHost, st));
+        PCS_CUDA(cudaStreamSynchronize(st));
     }
     return PCS_OK;
 }
@@ -274,7 +341,7 @@ void pcs_shutdown(void) {
 void* pcs_stream(void) { return g_ctx.init ? (void*)g_ctx.stream : nullptr; }
 
 int pcs_synchronize(void) {
-    PCS_NEED_INIT();
+    if (int rc = need_init()) return rc;
     PCS_CUDA(cudaStreamSynchronize(g_ctx.stream));
     return PCS_OK;
 }
@@ -283,7 +350,7 @@ int pcs_synchronize(void) {
 // primitives
 // ------------------------------------------------------------------------------------------------
 int pcs_field_op(int op, const uint64_t* a, const uint64_t* b, size_t n, uint64_t* out) {
-    PCS_NEED_INIT();
+    if (int rc = need_init()) return rc;
     if (n == 0) return PCS_OK;
     if (!a || !out) return fail(PCS_ERR_ARG, "NULL pointer");
     if (op < PCS_OP_ADD || op > PCS_OP_MUL_2EXP) return fail(PCS_ERR_ARG, "unknown field operation");
@@ -305,7 +372,7 @@ int pcs_field_op(int op, const uint64_t* a, const uint64_t* b, size_t n, uint64_
 }
 
 int pcs_poseidon_permute(uint64_t* states, size_t n) {
-    PCS_NEED_INIT();
+    if (int rc = need_init()) return rc;
     if (n == 0) return PCS_OK;
     if (!states) return fail(PCS_ERR_ARG, "states is NULL");
     cudaStream_t st = g_ctx.stream;
@@ -319,7 +386,7 @@ int pcs_poseidon_permute(uint64_t* states, size_t n) {
 }
 
 int pcs_pow_grind(const uint64_t* state, unsigned witness_pos, unsigned min_leading_zeros, uint64_t* witness) {
-    PCS_NEED_INIT();
+    if (int rc = need_init()) return rc;
     if (!state || !witness) return fail(PCS_ERR_ARG, "NULL pointer");
     if (witness_pos >= 12) return fail(PCS_ERR_ARG, "witness position outside the sponge state");
     if (min_leading_zeros > 40) return fail(PCS_ERR_ARG, "proof-of-work difficulty above 40 bits is not supported");
@@ -350,7 +417,7 @@ int pcs_pow_grind(const uint64_t* state, unsigned witness_pos, unsigned min_lead
 }
 
 int pcs_hash_or_noop(const uint64_t* rows, size_t n, size_t len, uint64_t* out) {
-    PCS_NEED_INIT();
+    if (int rc = need_init()) return rc;
     if (n == 0) return PCS_OK;
     if (!rows || !out) return fail(PCS_ERR_ARG, "NULL pointer");
     if (len == 0) {  // hash_or_noop of an empty slice: all-zero HashOut (config.rs:56-62)
@@ -371,7 +438,7 @@ int pcs_hash_or_noop(const uint64_t* rows, size_t n, size_t len, uint64_t* out) 
 }
 
 int pcs_two_to_one(const uint64_t* left, const uint64_t* right, size_t n, uint64_t* out) {
-    PCS_NEED_INIT();
+    if (int rc = need_init()) return rc;
     if (n == 0) return PCS_OK;
     if (!left || !right || !out) return fail(PCS_ERR_ARG, "NULL pointer");
     cudaStream_t st = g_ctx.stream;
@@ -387,23 +454,17 @@ int pcs_two_to_one(const uint64_t* left, const uint64_t* right, size_t n, uint64
     return PCS_OK;
 }
 
-int pcs_ntt(uint64_t* polys, size_t w, unsigned lg_n, int inverse) {
-    PCS_NEED_INIT();
-    if (w == 0) return PCS_OK;
-    if (!polys) return fail(PCS_ERR_ARG, "polys is NULL");
-    if (lg_n > 32) return fail(PCS_ERR_TWO_ADICITY, "n_log <= TWO_ADICITY violated");
-    cudaStream_t st = g_ctx.stream;
-    size_t n = (size_t)1 << lg_n;
-    NttPlan* plan = ntt_plan_get(lg_n, 0, inverse != 0, 1, st);
+}  // extern "C"
+
+// In place on the device, natural order in and out: w polynomials [w][2^lg_n], forward NTT or inverse NTT (scaled by 1/n)
+static int ntt_dev(uint64_t* polys, size_t w, unsigned lg_n, bool inverse, cudaStream_t st) {
+    const size_t n = (size_t)1 << lg_n;
+    NttPlan* plan = ntt_plan_get(lg_n, 0, inverse, 1, st);
     if (!plan) return fail(PCS_ERR_ALLOC, "twiddle table allocation failed");
-    DevBuf a, b;
-    PCS_CUDA(a.alloc(w * n * 8, st));
+    DevBuf b;
     PCS_CUDA(b.alloc(w * n * 8, st));
-    PCS_CUDA(cudaMemcpyAsync(a.p, polys, w * n * 8, cudaMemcpyHostToDevice, st));
-    PCS_CUDA(ntt_lde(plan, a.u64(), n, b.u64(), n, w, st));            // natural -> bit-reversed
-    PCS_CUDA(launch_bitrev_permute(b.u64(), n, a.u64(), n, w, lg_n, st, ntt_plan_scale(plan)));  // -> natural (+ 1/n)
-    PCS_CUDA(cudaMemcpyAsync(polys, a.p, w * n * 8, cudaMemcpyDeviceToHost, st));
-    PCS_CUDA(cudaStreamSynchronize(st));
+    PCS_CUDA(ntt_lde(plan, polys, n, b.u64(), n, w, st));                                          // -> bit-reversed
+    PCS_CUDA(launch_bitrev_permute(b.u64(), n, polys, n, w, lg_n, st, ntt_plan_scale(plan)));      // -> natural (* 1/n)
     return PCS_OK;
 }
 
@@ -417,60 +478,62 @@ static uint64_t host_inverse(uint64_t a) {  // a^(p-2) mod p
     return (uint64_t)acc;
 }
 
-int pcs_coset_intt(uint64_t* values, size_t w, unsigned lg_n, uint64_t shift) {
-    PCS_NEED_INIT();
-    if (w == 0) return PCS_OK;
-    if (!values) return fail(PCS_ERR_ARG, "values is NULL");
-    if (lg_n > 32) return fail(PCS_ERR_TWO_ADICITY, "n_log <= TWO_ADICITY violated");
-    if (shift % 0xFFFFFFFF00000001ULL == 0) return fail(PCS_ERR_ARG, "shift must be non-zero");
+// coset_ifft in place on the device: values on shift * <w_n>, natural order -> coefficients
+static int coset_intt_dev(uint64_t* values, size_t w, unsigned lg_n, uint64_t shift, cudaStream_t st) {
+    const size_t n = (size_t)1 << lg_n;
+    if (int rc = ntt_dev(values, w, lg_n, true, st)) return rc;
+    PCS_CUDA(launch_mul_powers(values, n, w, n, host_inverse(shift), st));   // c_i *= shift^-i  (mod.rs:68-72)
+    return PCS_OK;
+}
+
+// host data [w][2^lg_n] -> a device copy -> body(copy) -> back into data; synchronises
+template <class Body>
+static int through_device(uint64_t* data, size_t w, unsigned lg_n, Body body) {
     cudaStream_t st = g_ctx.stream;
-    size_t n = (size_t)1 << lg_n;
-    NttPlan* plan = ntt_plan_get(lg_n, 0, true, 1, st);
-    if (!plan) return fail(PCS_ERR_ALLOC, "twiddle table allocation failed");
-    DevBuf a, b;
-    PCS_CUDA(a.alloc(w * n * 8, st));
-    PCS_CUDA(b.alloc(w * n * 8, st));
-    PCS_CUDA(cudaMemcpyAsync(a.p, values, w * n * 8, cudaMemcpyHostToDevice, st));
-    PCS_CUDA(ntt_lde(plan, a.u64(), n, b.u64(), n, w, st));
-    PCS_CUDA(launch_bitrev_permute(b.u64(), n, a.u64(), n, w, lg_n, st, ntt_plan_scale(plan)));
-    PCS_CUDA(launch_mul_powers(a.u64(), n, w, n, host_inverse(shift), st));   // c_i *= shift^-i  (mod.rs:68-72)
-    PCS_CUDA(cudaMemcpyAsync(values, a.p, w * n * 8, cudaMemcpyDeviceToHost, st));
+    const size_t bytes = (w * 8) << lg_n;
+    DevBuf a;
+    PCS_CUDA(a.alloc(bytes, st));
+    PCS_CUDA(cudaMemcpyAsync(a.p, data, bytes, cudaMemcpyHostToDevice, st));
+    if (int rc = body(a.u64(), st)) return rc;
+    PCS_CUDA(cudaMemcpyAsync(data, a.p, bytes, cudaMemcpyDeviceToHost, st));
     PCS_CUDA(cudaStreamSynchronize(st));
     return PCS_OK;
 }
 
+extern "C" {
+
+int pcs_ntt(uint64_t* polys, size_t w, unsigned lg_n, int inverse) {
+    if (int rc = need_init()) return rc;
+    if (w == 0) return PCS_OK;
+    if (!polys) return fail(PCS_ERR_ARG, "polys is NULL");
+    if (int rc = check_two_adicity(lg_n)) return rc;
+    return through_device(polys, w, lg_n, [&](uint64_t* p, cudaStream_t st) { return ntt_dev(p, w, lg_n, inverse != 0, st); });
+}
+
+int pcs_coset_intt(uint64_t* values, size_t w, unsigned lg_n, uint64_t shift) {
+    if (int rc = need_init()) return rc;
+    if (w == 0) return PCS_OK;
+    if (!values) return fail(PCS_ERR_ARG, "values is NULL");
+    if (int rc = check_two_adicity(lg_n)) return rc;
+    if (int rc = check_shift(shift)) return rc;
+    return through_device(values, w, lg_n, [&](uint64_t* v, cudaStream_t st) { return coset_intt_dev(v, w, lg_n, shift, st); });
+}
+
 int pcs_coset_intt_dev(uint64_t* values_dev, size_t w, unsigned lg_n, uint64_t shift) {
-    PCS_NEED_INIT();
+    if (int rc = need_init()) return rc;
     if (w == 0) return PCS_OK;
     if (!values_dev) return fail(PCS_ERR_ARG, "values is NULL");
-    if (lg_n > 32) return fail(PCS_ERR_TWO_ADICITY, "n_log <= TWO_ADICITY violated");
-    if (shift % 0xFFFFFFFF00000001ULL == 0) return fail(PCS_ERR_ARG, "shift must be non-zero");
-    cudaStream_t st = g_ctx.stream;
-    size_t n = (size_t)1 << lg_n;
-    NttPlan* plan = ntt_plan_get(lg_n, 0, true, 1, st);
-    if (!plan) return fail(PCS_ERR_ALLOC, "twiddle table allocation failed");
-    DevBuf b;
-    PCS_CUDA(b.alloc(w * n * 8, st));
-    PCS_CUDA(ntt_lde(plan, values_dev, n, b.u64(), n, w, st));                                             // -> bit-reversed
-    PCS_CUDA(launch_bitrev_permute(b.u64(), n, values_dev, n, w, lg_n, st, ntt_plan_scale(plan)));         // -> natural, * 1/n
-    PCS_CUDA(launch_mul_powers(values_dev, n, w, n, host_inverse(shift), st));                             // c_i *= shift^-i
-    return PCS_OK;   // asynchronous on pcs_stream()
+    if (int rc = check_two_adicity(lg_n)) return rc;
+    if (int rc = check_shift(shift)) return rc;
+    return coset_intt_dev(values_dev, w, lg_n, shift, g_ctx.stream);   // asynchronous on pcs_stream()
 }
 
 int pcs_ntt_dev(uint64_t* polys_dev, size_t w, unsigned lg_n, int inverse) {
-    PCS_NEED_INIT();
+    if (int rc = need_init()) return rc;
     if (w == 0) return PCS_OK;
     if (!polys_dev) return fail(PCS_ERR_ARG, "polys is NULL");
-    if (lg_n > 32) return fail(PCS_ERR_TWO_ADICITY, "n_log <= TWO_ADICITY violated");
-    cudaStream_t st = g_ctx.stream;
-    size_t n = (size_t)1 << lg_n;
-    NttPlan* plan = ntt_plan_get(lg_n, 0, inverse != 0, 1, st);
-    if (!plan) return fail(PCS_ERR_ALLOC, "twiddle table allocation failed");
-    DevBuf b;
-    PCS_CUDA(b.alloc(w * n * 8, st));
-    PCS_CUDA(ntt_lde(plan, polys_dev, n, b.u64(), n, w, st));                                              // -> bit-reversed
-    PCS_CUDA(launch_bitrev_permute(b.u64(), n, polys_dev, n, w, lg_n, st, ntt_plan_scale(plan)));          // -> natural
-    return PCS_OK;   // asynchronous on pcs_stream()
+    if (int rc = check_two_adicity(lg_n)) return rc;
+    return ntt_dev(polys_dev, w, lg_n, inverse != 0, g_ctx.stream);   // asynchronous on pcs_stream()
 }
 
 }  // extern "C"
@@ -500,7 +563,7 @@ static int d2h_pageable(void* dst, const void* src_dev, size_t bytes, cudaStream
 constexpr size_t RING_SLOT_BYTES = 16u << 20;
 constexpr unsigned STAGE_THREADS = 4;
 
-static bool is_pageable_host(const void* p) {
+bool pcs::is_pageable_host(const void* p) {
     cudaPointerAttributes a;
     if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
         cudaGetLastError();
@@ -563,6 +626,38 @@ static int stage_polys(const uint64_t* const* polys, size_t w, size_t d, bool de
     return PCS_OK;
 }
 
+static bool contiguous(const uint64_t* const* polys, size_t count, size_t d) {
+    for (size_t j = 1; j < count; j++)
+        if (polys[j] != polys[0] + j * d) return false;
+    return true;
+}
+
+// Where ntt_lde_cosets reads `count` device polynomials of 2^lg_d coefficients from: the caller's matrix when they are
+// contiguous, else a device table of their pointers that the first NTT pass follows (they may live in PEER memory: no
+// staging copy), or, for lg_d == 0, which has no such pass, a staged contiguous copy.
+struct DevInput {
+    const uint64_t* src = nullptr;
+    const uint64_t* const* ptrs = nullptr;
+    DevBuf table, staged;
+};
+
+static int resolve_dev_input(const uint64_t* const* polys, size_t count, unsigned lg_d, cudaStream_t st, DevInput& in) {
+    const size_t d = (size_t)1 << lg_d;
+    for (size_t j = 0; j < count; j++)
+        if (!polys[j]) return fail(PCS_ERR_ARG, "NULL polynomial pointer");
+    in.src = polys[0];
+    if (contiguous(polys, count, d)) return PCS_OK;
+    if (lg_d >= 1) {
+        PCS_CUDA(in.table.alloc(count * sizeof(uint64_t*), st));
+        PCS_CUDA(cudaMemcpyAsync(in.table.p, polys, count * sizeof(uint64_t*), cudaMemcpyHostToDevice, st));
+        in.ptrs = (const uint64_t* const*)in.table.p;
+        return PCS_OK;
+    }
+    PCS_CUDA(in.staged.alloc(count * d * 8, st));
+    in.src = in.staged.u64();
+    return stage_polys(polys, count, d, true, in.staged.u64(), st);
+}
+
 static void host_copy_mt(char* dst, const char* src, size_t bytes) {
     const unsigned nt = bytes >= (4u << 20) ? STAGE_THREADS : 1;
     if (nt == 1) {
@@ -612,10 +707,10 @@ extern "C" {
 
 int pcs_coset_lde(const uint64_t* const* coeffs, size_t w, unsigned lg_d, unsigned rate_bits, uint64_t shift,
                   uint64_t* out, int layout) {
-    PCS_NEED_INIT();
+    if (int rc = need_init()) return rc;
     if (w == 0) return fail(PCS_ERR_ARG, "empty batch (oracle.rs:103 polynomials[0])");
     if (!coeffs || !out) return fail(PCS_ERR_ARG, "NULL pointer");
-    if (lg_d + rate_bits > 32) return fail(PCS_ERR_TWO_ADICITY, "n_log <= TWO_ADICITY violated");
+    if (int rc = check_two_adicity(lg_d + rate_bits)) return rc;
     cudaStream_t st = g_ctx.stream;
     size_t d = (size_t)1 << lg_d, n = d << rate_bits;
     NttPlan* plan = ntt_plan_get(lg_d, rate_bits, false, shift, st);
@@ -638,46 +733,26 @@ int pcs_coset_lde(const uint64_t* const* coeffs, size_t w, unsigned lg_d, unsign
 
 int pcs_coset_lde_dev(const uint64_t* const* coeffs_dev, size_t w, unsigned lg_d, unsigned rate_bits, uint64_t shift,
                       uint64_t* out_dev) {
-    PCS_NEED_INIT();
+    if (int rc = need_init()) return rc;
     if (w == 0) return fail(PCS_ERR_ARG, "empty batch (oracle.rs:103 polynomials[0])");
     if (!coeffs_dev || !out_dev) return fail(PCS_ERR_ARG, "NULL pointer");
-    if (lg_d + rate_bits > 32) return fail(PCS_ERR_TWO_ADICITY, "n_log <= TWO_ADICITY violated");
+    if (int rc = check_two_adicity(lg_d + rate_bits)) return rc;
     cudaStream_t st = g_ctx.stream;
     const size_t d = (size_t)1 << lg_d, n = d << rate_bits;
     NttPlan* plan = ntt_plan_get(lg_d, rate_bits, false, shift, st);
     if (!plan) return fail(PCS_ERR_ALLOC, "twiddle table allocation failed");
-    bool contiguous = true;
-    for (size_t j = 0; j < w; j++) {
-        if (!coeffs_dev[j]) return fail(PCS_ERR_ARG, "NULL polynomial pointer");
-        contiguous = contiguous && coeffs_dev[j] == coeffs_dev[0] + j * d;
-    }
-    DevBuf table, staged;
-    const uint64_t* src = coeffs_dev[0];
-    const uint64_t* const* ptrs = nullptr;
-    if (!contiguous) {
-        if (lg_d >= 1) {
-            PCS_CUDA(table.alloc(w * sizeof(uint64_t*), st));
-            PCS_CUDA(cudaMemcpyAsync(table.p, coeffs_dev, w * sizeof(uint64_t*), cudaMemcpyHostToDevice, st));
-            ptrs = (const uint64_t* const*)table.p;
-        } else {
-            PCS_CUDA(staged.alloc(w * d * 8, st));
-            int rc = stage_polys(coeffs_dev, w, d, true, staged.u64(), st);
-            if (rc) return rc;
-            src = staged.u64();
-        }
-    }
-    PCS_CUDA(ntt_lde_cosets(plan, src, d, out_dev, n, w, 0, rate_bits, st, ptrs));
+    DevInput in;
+    if (int rc = resolve_dev_input(coeffs_dev, w, lg_d, st, in)) return rc;
+    PCS_CUDA(ntt_lde_cosets(plan, in.src, d, out_dev, n, w, 0, rate_bits, st, in.ptrs));
     return PCS_OK;   // asynchronous on pcs_stream()
 }
 
 int pcs_merkle_build(const uint64_t* leaves, size_t n, size_t len, unsigned cap_height, uint64_t* digests,
                      uint64_t* cap) {
-    PCS_NEED_INIT();
+    if (int rc = need_init()) return rc;
     int lg_n = ilog2_strict(n);
     if (lg_n < 0) return fail(PCS_ERR_NOT_POW2, "Not a power of two: " + std::to_string(n));
-    if ((int)cap_height > lg_n)
-        return fail(PCS_ERR_CAP_HEIGHT, "cap_height=" + std::to_string(cap_height) +
-                                            " should be at most log2(leaves.len())=" + std::to_string(lg_n));
+    if (int rc = check_cap_height(cap_height, (unsigned)lg_n)) return rc;
     if (!leaves || !cap || len == 0) return fail(PCS_ERR_ARG, "NULL pointer or empty leaves");
     cudaStream_t st = g_ctx.stream;
     size_t n_cap = (size_t)1 << cap_height, n_dig = 2 * (n - n_cap);
@@ -726,6 +801,148 @@ void pcs_batch_free(pcs_batch* b) {
     delete b;
 }
 
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------
+// the steps of commit_common
+// ------------------------------------------------------------------------------------------------
+// On every exit taken once H2D copies were enqueued on the copy stream, wait for them before the batch's owner returns their
+// destination to the pool (and release the pinned ring slots).  Declared after the owner, so destroyed before it.
+struct CopyDrain {
+    bool armed = false;
+    ~CopyDrain() {
+        if (g_ctx.d2h_stream) cudaStreamSynchronize(g_ctx.d2h_stream);   // D2H copies out of a buffer the owner is about to free
+        if (!armed || !g_ctx.copy_stream) return;
+        cudaStreamSynchronize(g_ctx.copy_stream);
+        for (auto& busy : g_ctx.ring_busy) busy = false;
+    }
+};
+
+// Where the LDE reads a commitment's input (values or coefficients) from, and, for host inputs that arrive chunk by chunk
+// on the copy stream, the chunk bounds: chunk k = polynomials [cb[k], cb[k+1]).
+struct CommitInput {
+    DevInput dev;
+    std::vector<size_t> cb;   // empty: the whole input is in place once the main stream gets there
+    bool pageable = false;    // chunks go through the pinned ring, each staged right before its compute is enqueued
+};
+
+// Device coefficients that are neither kept nor transformed are read in place; every other input is copied into b->coeffs:
+// device inputs and small host polynomials at once, larger host polynomials chunk by chunk on the copy stream.
+static int stage_inputs(const uint64_t* const* polys, bool from_values, unsigned flags, pcs_batch* b, CommitInput& in,
+                        CopyDrain& drain) {
+    cudaStream_t st = g_ctx.stream;
+    const size_t w = b->w, d = (size_t)1 << b->lg_d;
+    const bool dev_ptrs = flags & PCS_DEVICE_PTRS;
+    if (dev_ptrs && !from_values && !(flags & PCS_KEEP_COEFFS)) return resolve_dev_input(polys, w, b->lg_d, st, in.dev);
+    PCS_CUDA(cudaMallocAsync((void**)&b->coeffs, w * d * 8, st));   // owned by the batch from here on
+    uint64_t* const staged = b->coeffs;
+    in.dev.src = staged;
+    if (dev_ptrs) {
+        if (!contiguous(polys, w, d)) return stage_polys(polys, w, d, true, staged, st);
+        PCS_CUDA(cudaMemcpyAsync(staged, polys[0], w * d * 8, cudaMemcpyDeviceToDevice, st));
+        return PCS_OK;
+    }
+    if (d * 8 <= SMALL_POLY_BYTES && w * d * 8 <= PIN_STAGING_MAX && pinned(g_ctx.pin_in, g_ctx.pin_in_bytes, w * d * 8)) {
+        // small host polynomials: one gather on the host, one H2D copy
+        for (size_t j = 0; j < w; j++) {
+            if (!polys[j]) return fail(PCS_ERR_ARG, "NULL polynomial pointer");
+            memcpy((char*)g_ctx.pin_in + j * d * 8, polys[j], d * 8);
+        }
+        PCS_CUDA(cudaMemcpyAsync(staged, g_ctx.pin_in, w * d * 8, cudaMemcpyHostToDevice, st));
+        return PCS_OK;
+    }
+    // host inputs: chunked H2D on the copy stream, one event per chunk
+    if (!g_ctx.copy_stream) PCS_CUDA(cudaStreamCreateWithFlags(&g_ctx.copy_stream, cudaStreamNonBlocking));
+    if (!g_ctx.ev_sync) PCS_CUDA(cudaEventCreateWithFlags(&g_ctx.ev_sync, cudaEventDisableTiming));
+    for (size_t j = 0; j < w; j++)
+        if (!polys[j]) return fail(PCS_ERR_ARG, "NULL polynomial pointer");
+    in.pageable = w * d * 8 >= (8u << 20) && is_pageable_host(polys[0]);   // below 8 MB the threads cost more than they save
+    // Chunk sizes: the first transfer is the only one nothing hides, so it is small (8 polynomials = one absorb of the
+    // sponge, or one 16 MB ring slot's worth for short polynomials); a chunk's compute (LDE + its share of the leaf
+    // hashing, ~0.9 ms per polynomial at 2^20) outlasts a transfer 5x its size, so the groups grow 5x and few sponge
+    // states have to be parked (each group boundary costs 192 B of HBM traffic per leaf).
+    std::vector<size_t>& cb = in.cb;
+    size_t first = 8;
+    if (first * d * 8 < RING_SLOT_BYTES) first = (RING_SLOT_BYTES / (d * 8) + 7) / 8 * 8;
+    cb.assign(1, 0);
+    for (size_t sz = first; cb.back() < w; sz *= 5) cb.push_back(cb.back() + sz < w ? cb.back() + sz : w);
+    if (cb.size() > 2 && w - cb[cb.size() - 2] < 8) cb.erase(cb.end() - 2);   // no tiny tail group
+    const size_t n_chunks = cb.size() - 1;
+    while (g_ctx.chunk_ev.size() < n_chunks) {
+        cudaEvent_t e;
+        PCS_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        g_ctx.chunk_ev.push_back(e);
+    }
+    PCS_CUDA(cudaEventRecord(g_ctx.ev_sync, st));               // `staged` exists from here on
+    PCS_CUDA(cudaStreamWaitEvent(g_ctx.copy_stream, g_ctx.ev_sync, 0));
+    drain.armed = true;
+    for (size_t k = 0; k < n_chunks && !in.pageable; k++) {
+        if (int rc = stage_polys(polys + cb[k], cb[k + 1] - cb[k], d, false, staged + cb[k] * d, g_ctx.copy_stream)) return rc;
+        PCS_CUDA(cudaEventRecord(g_ctx.chunk_ev[k], g_ctx.copy_stream));
+    }
+    return PCS_OK;
+}
+
+// How from_values returns the coefficients to coeffs_out
+enum class CoeffsOut {
+    none,
+    small_pinned,   // one D2H copy into pinned staging after the LDE, scattered to the caller's vectors after the final sync
+    big_pinned,     // every chunk's coefficients leave on the D2H stream into pinned staging while the LDE and the hashing go
+                    // on, and are scattered into the caller's (pageable, separately allocated) vectors by a few host threads
+    direct,         // one D2H copy per polynomial on the main stream
+};
+
+static CoeffsOut choose_coeffs_out(bool from_values, uint64_t* const* coeffs_out, size_t w, size_t d) {
+    if (!from_values || !coeffs_out) return CoeffsOut::none;
+    const size_t bytes = w * d * 8;
+    if (d * 8 <= SMALL_POLY_BYTES && bytes <= PIN_STAGING_MAX && pinned(g_ctx.pin_out, g_ctx.pin_out_bytes, bytes))
+        return CoeffsOut::small_pinned;
+    // larger outputs: the reference keeps `polynomials`, so a Rust caller always asks for them
+    if (bytes <= ((size_t)512 << 20) && pinned(g_ctx.pin_out, g_ctx.pin_out_bytes, bytes)) return CoeffsOut::big_pinned;
+    return CoeffsOut::direct;
+}
+
+// after the commit has been synchronised: the coefficients staged in pinned memory into the caller's vectors
+static int hand_back_coeffs(CoeffsOut mode, uint64_t* const* coeffs_out, size_t w, size_t d) {
+    const char* srcp = (const char*)g_ctx.pin_out;
+    if (mode == CoeffsOut::small_pinned)
+        for (size_t j = 0; j < w; j++)
+            if (coeffs_out[j]) memcpy(coeffs_out[j], srcp + j * d * 8, d * 8);
+    if (mode == CoeffsOut::big_pinned) {
+        PCS_CUDA(cudaStreamSynchronize(g_ctx.stream));
+        PCS_CUDA(cudaStreamSynchronize(g_ctx.d2h_stream));
+        const unsigned nt = STAGE_THREADS;
+        std::thread th[STAGE_THREADS];
+        for (unsigned t = 0; t < nt; t++)
+            th[t] = std::thread([=]() {
+                for (size_t j = t; j < w; j += nt)
+                    if (coeffs_out[j]) memcpy(coeffs_out[j], srcp + j * d * 8, d * 8);
+            });
+        for (unsigned t = 0; t < nt; t++) th[t].join();
+    }
+    return PCS_OK;
+}
+
+// Blinding (oracle.rs:119-123): the caller's salt column k is in natural LDE order like lde_values, the leaves are in
+// bit-reversed order (oracle.rs:84).  A shard's salt rows are its own leaf range, already in leaf order.
+static int write_salts(pcs_batch* b, const uint64_t* const* salts, bool dev_ptrs, bool shard, cudaStream_t st) {
+    const size_t n = b->n;
+    for (size_t k = 0; k < b->salt_w; k++) {
+        if (!salts[k]) return fail(PCS_ERR_ARG, "NULL salt pointer");
+        uint64_t* row = b->lde + (b->w + k) * n;
+        DevBuf tmp;
+        PCS_CUDA(tmp.alloc(n * 8, st));
+        PCS_CUDA(cudaMemcpyAsync(tmp.p, salts[k], n * 8, dev_ptrs ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
+        PCS_CUDA(launch_canonicalize(tmp.u64(), n, st));
+        if (shard)
+            PCS_CUDA(cudaMemcpyAsync(row, tmp.p, n * 8, cudaMemcpyDeviceToDevice, st));
+        else
+            PCS_CUDA(launch_bitrev_permute(tmp.u64(), n, row, n, 1, b->lg_d + b->rate_bits, st));
+    }
+    return PCS_OK;
+}
+
+// PolynomialBatch::from_coeffs / from_values (oracle.rs:43-125).
 // shard == true: only the cosets [coset_first, coset_first + 2^lg_cosets) (leaf order) are extended and the
 // tree is built over those d << lg_cosets leaves with `cap_height` (the caller's LOCAL cap height); salts are
 // then the shard's rows, already in leaf order.
@@ -733,141 +950,42 @@ static int commit_common(const uint64_t* const* polys, bool from_values, size_t 
                          unsigned cap_height, const uint64_t* const* salts, size_t salt_w, unsigned flags,
                          uint64_t* const* coeffs_out, uint64_t* cap_out, pcs_batch** out, bool shard = false,
                          unsigned coset_first = 0, unsigned lg_cosets = 0) {
-    PCS_NEED_INIT();
+    if (int rc = need_init()) return rc;
     if (!out) return fail(PCS_ERR_ARG, "out is NULL");
     *out = nullptr;
     if (w == 0 || !polys) return fail(PCS_ERR_ARG, "empty batch (oracle.rs:76 polynomials[0])");
     if (salt_w && !salts) return fail(PCS_ERR_ARG, "salts is NULL");
-    if (lg_d + rate_bits > 32) return fail(PCS_ERR_TWO_ADICITY, "n_log <= TWO_ADICITY violated");
     if (!shard) lg_cosets = rate_bits;
-    if (lg_cosets > rate_bits || ((size_t)coset_first + ((size_t)1 << lg_cosets)) > ((size_t)1 << rate_bits))
-        return fail(PCS_ERR_ARG, "coset range outside [0, 2^rate_bits)");
-    unsigned lg_n = lg_d + lg_cosets;   // leaves of this (shard of the) tree
-    if (cap_height > lg_n)
-        return fail(PCS_ERR_CAP_HEIGHT, "cap_height=" + std::to_string(cap_height) +
-                                            " should be at most log2(leaves.len())=" + std::to_string(lg_n));
+    BatchOwner b;
+    if (int rc = batch_begin(w, salt_w, lg_d, rate_bits, coset_first, lg_cosets, cap_height, BATCH_LDE, b)) return rc;
     cudaStream_t st = g_ctx.stream;
-    const bool dev_ptrs = flags & PCS_DEVICE_PTRS;
-    const size_t d = (size_t)1 << lg_d, n = d << lg_cosets, wt = w + salt_w;
-    const size_t n_cap = (size_t)1 << cap_height;
-
-    NttPlan* plan = ntt_plan_get(lg_d, rate_bits, false, 7 /* F::coset_shift(), types.rs:437 */, st);
     NttPlan* iplan = from_values ? ntt_plan_get(lg_d, 0, true, 1, st) : nullptr;
-    if (!plan || (from_values && !iplan)) return fail(PCS_ERR_ALLOC, "twiddle table allocation failed");
+    if (from_values && !iplan) return fail(PCS_ERR_ALLOC, "twiddle table allocation failed");
+    b->has_ifft = from_values;
+    CopyDrain drain;
+    const bool dev_ptrs = flags & PCS_DEVICE_PTRS;
+    const size_t d = (size_t)1 << lg_d, n = b->n, wt = w + salt_w;
 
-    pcs_batch* b = batch_new();
-    b->w = w; b->salt_w = salt_w; b->lg_d = lg_d; b->rate_bits = lg_cosets; b->cap_height = cap_height;
-    b->full_rate_bits = rate_bits; b->coset_first = coset_first;
-    b->n = n; b->n_digests = 2 * (n - n_cap); b->has_ifft = from_values;
-    struct Guard { pcs_batch* b; bool armed = true; ~Guard() { if (armed) pcs_batch_free(b); } } guard{b};
-    // Declared after `guard`, so destroyed before it: on every failure exit taken once H2D copies were enqueued on the copy
-    // stream, wait for them before the guard returns their destination to the pool (and release the pinned ring slots).
-    struct CopyDrain {
-        bool armed = false;
-        ~CopyDrain() {
-            if (g_ctx.d2h_stream) cudaStreamSynchronize(g_ctx.d2h_stream);   // D2H copies out of a buffer the guard is about to free
-            if (!armed || !g_ctx.copy_stream) return;
-            cudaStreamSynchronize(g_ctx.copy_stream);
-            for (auto& busy : g_ctx.ring_busy) busy = false;
-        }
-    } copy_drain;
-    for (auto& e : b->ev) PCS_CUDA(cudaEventCreate(&e));
-    PCS_CUDA(cudaMallocAsync((void**)&b->lde, wt * n * 8, st));
-    PCS_CUDA(cudaMallocAsync((void**)&b->digests, b->n_digests ? b->n_digests * 32 : 32, st));
-    PCS_CUDA(cudaMallocAsync((void**)&b->cap, n_cap * 32, st));
-
-    // ---- inputs -> one contiguous [w][d] device matrix ----
-    bool contiguous_dev = dev_ptrs;
-    if (dev_ptrs)
-        for (size_t j = 0; j < w; j++) contiguous_dev = contiguous_dev && polys[j] == polys[0] + j * d;
-    const uint64_t* src = nullptr;   // [w][d] device input (values or coefficients)
-    DevBuf ptr_table;                // or: device table of the caller's w polynomial pointers, read in place
-    uint64_t* staged = nullptr;
-    bool scatter_coeffs = false;
-    std::vector<size_t> cb;           // chunk k = polynomials [cb[k], cb[k+1]) of the host-input pipeline
-    size_t n_chunks = 0;              // > 0: host inputs arrive chunk by chunk on the copy stream
-    bool pageable = false;            // ... through the pinned ring, each chunk staged right before its compute is enqueued
-    if (contiguous_dev && !from_values && !(flags & PCS_KEEP_COEFFS)) {
-        src = polys[0];
-    } else if (dev_ptrs && !from_values && !(flags & PCS_KEEP_COEFFS) && lg_d >= 1) {
-        // separately allocated device polynomials (possibly in PEER memory): no staging copy, the first NTT pass
-        // follows the pointer table
-        for (size_t j = 0; j < w; j++)
-            if (!polys[j]) return fail(PCS_ERR_ARG, "NULL polynomial pointer");
-        PCS_CUDA(ptr_table.alloc(w * sizeof(uint64_t*), st));
-        PCS_CUDA(cudaMemcpyAsync(ptr_table.p, polys, w * sizeof(uint64_t*), cudaMemcpyHostToDevice, st));
-    } else {
-        PCS_CUDA(cudaMallocAsync((void**)&staged, w * d * 8, st));
-        b->coeffs = staged;  // owned by the batch from here on
-        if (contiguous_dev)
-            PCS_CUDA(cudaMemcpyAsync(staged, polys[0], w * d * 8, cudaMemcpyDeviceToDevice, st));
-        else if (dev_ptrs) {
-            int rc = stage_polys(polys, w, d, true, staged, st);
-            if (rc) return rc;
-        } else if (d * 8 <= SMALL_POLY_BYTES && w * d * 8 <= PIN_STAGING_MAX &&
-                   pinned(g_ctx.pin_in, g_ctx.pin_in_bytes, w * d * 8)) {
-            // small host polynomials: one gather on the host, one H2D copy
-            for (size_t j = 0; j < w; j++) {
-                if (!polys[j]) return fail(PCS_ERR_ARG, "NULL polynomial pointer");
-                memcpy((char*)g_ctx.pin_in + j * d * 8, polys[j], d * 8);
-            }
-            PCS_CUDA(cudaMemcpyAsync(staged, g_ctx.pin_in, w * d * 8, cudaMemcpyHostToDevice, st));
-        } else {
-            // host inputs: chunked H2D on the copy stream, one event per chunk
-            if (!g_ctx.copy_stream) PCS_CUDA(cudaStreamCreateWithFlags(&g_ctx.copy_stream, cudaStreamNonBlocking));
-            if (!g_ctx.ev_sync) PCS_CUDA(cudaEventCreateWithFlags(&g_ctx.ev_sync, cudaEventDisableTiming));
-            for (size_t j = 0; j < w; j++)
-                if (!polys[j]) return fail(PCS_ERR_ARG, "NULL polynomial pointer");
-            pageable = w * d * 8 >= (8u << 20) && is_pageable_host(polys[0]);   // below 8 MB the threads cost more than they save
-            // Chunk sizes: the first transfer is the only one nothing hides, so it is small (8 polynomials = one absorb of the
-            // sponge, or one 16 MB ring slot's worth for short polynomials); a chunk's compute (LDE + its share of the leaf
-            // hashing, ~0.9 ms per polynomial at 2^20) outlasts a transfer 5x its size, so the groups grow 5x and few sponge
-            // states have to be parked (each group boundary costs 192 B of HBM traffic per leaf).
-            size_t first = 8;
-            if (first * d * 8 < RING_SLOT_BYTES) first = (RING_SLOT_BYTES / (d * 8) + 7) / 8 * 8;
-            cb.assign(1, 0);
-            for (size_t sz = first; cb.back() < w; sz *= 5) cb.push_back(cb.back() + sz < w ? cb.back() + sz : w);
-            if (cb.size() > 2 && w - cb[cb.size() - 2] < 8) cb.erase(cb.end() - 2);   // no tiny tail group
-            n_chunks = cb.size() - 1;
-            while (g_ctx.chunk_ev.size() < n_chunks) {
-                cudaEvent_t e;
-                PCS_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-                g_ctx.chunk_ev.push_back(e);
-            }
-            PCS_CUDA(cudaEventRecord(g_ctx.ev_sync, st));               // `staged` exists from here on
-            PCS_CUDA(cudaStreamWaitEvent(g_ctx.copy_stream, g_ctx.ev_sync, 0));
-            copy_drain.armed = true;
-            for (size_t k = 0; k < n_chunks && !pageable; k++) {
-                size_t j0 = cb[k], j1 = cb[k + 1];
-                int rc = stage_polys(polys + j0, j1 - j0, d, false, staged + j0 * d, g_ctx.copy_stream);
-                if (rc) {
-                    cudaStreamSynchronize(g_ctx.copy_stream);   // `staged` is released by the guard
-                    return rc;
-                }
-                PCS_CUDA(cudaEventRecord(g_ctx.chunk_ev[k], g_ctx.copy_stream));
-            }
-        }
-        src = staged;
-    }
+    // ---- inputs ----
+    CommitInput in;
+    if (int rc = stage_inputs(polys, from_values, flags, b.get(), in, drain)) return rc;
+    const uint64_t* const src = in.dev.src;
+    const size_t n_chunks = in.cb.empty() ? 0 : in.cb.size() - 1;   // > 0: IFFT and LDE follow each chunk as it lands
     PCS_CUDA(cudaEventRecord(b->ev[0], st));
 
-    // ---- "IFFT" (oracle.rs:51-55) for polynomials [j0, j1): values (natural order) -> coefficients in `staged` ----
+    // ---- "IFFT" (oracle.rs:51-55) for polynomials [j0, j1): values (natural order) -> coefficients in b->coeffs ----
     // scratch for the bit-reversed intermediate = the TAIL of the LDE buffer (the last w*d elements): LDE rows already
     // written for earlier polynomials end at j0*n <= wt*n - w*d + j0*d, so chunk-by-chunk processing never clobbers them
     uint64_t* const ifft_scratch = b->lde + (wt * n - w * d);
-    const bool small_out = from_values && coeffs_out && d * 8 <= SMALL_POLY_BYTES && w * d * 8 <= PIN_STAGING_MAX &&
-                           pinned(g_ctx.pin_out, g_ctx.pin_out_bytes, w * d * 8);
-    // larger outputs (the reference keeps `polynomials`, so a Rust caller always asks for them): every chunk's coefficients
-    // leave on their own stream into pinned staging while the LDE and the hashing go on, and are scattered into the caller's
-    // (pageable, separately allocated) vectors by a few host threads after the commit
-    const bool big_out = from_values && coeffs_out && !small_out && w * d * 8 <= ((size_t)512 << 20) &&
-                         pinned(g_ctx.pin_out, g_ctx.pin_out_bytes, w * d * 8);
+    uint64_t* const coeffs = b->coeffs;
+    const CoeffsOut mode = choose_coeffs_out(from_values, coeffs_out, w, d);
+    if (mode == CoeffsOut::big_pinned && !g_ctx.d2h_stream)
+        PCS_CUDA(cudaStreamCreateWithFlags(&g_ctx.d2h_stream, cudaStreamNonBlocking));
     size_t n_d2h = 0;
-    if (big_out && !g_ctx.d2h_stream) PCS_CUDA(cudaStreamCreateWithFlags(&g_ctx.d2h_stream, cudaStreamNonBlocking));
     auto ifft_range = [&](size_t j0, size_t j1) -> int {
         PCS_CUDA(ntt_inverse_bitrev(iplan, src + j0 * d, d, ifft_scratch + j0 * d, d, j1 - j0, st));
-        PCS_CUDA(launch_bitrev_permute(ifft_scratch + j0 * d, d, staged + j0 * d, d, j1 - j0, lg_d, st, ntt_plan_scale(iplan)));
-        if (big_out) {
+        PCS_CUDA(launch_bitrev_permute(ifft_scratch + j0 * d, d, coeffs + j0 * d, d, j1 - j0, lg_d, st, ntt_plan_scale(iplan)));
+        if (mode == CoeffsOut::big_pinned) {
             if (g_ctx.d2h_ev.size() <= n_d2h) {
                 cudaEvent_t e;
                 PCS_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
@@ -876,118 +994,51 @@ static int commit_common(const uint64_t* const* polys, bool from_values, size_t 
             PCS_CUDA(cudaEventRecord(g_ctx.d2h_ev[n_d2h], st));
             PCS_CUDA(cudaStreamWaitEvent(g_ctx.d2h_stream, g_ctx.d2h_ev[n_d2h], 0));
             n_d2h++;
-            PCS_CUDA(cudaMemcpyAsync((char*)g_ctx.pin_out + j0 * d * 8, staged + j0 * d, (j1 - j0) * d * 8, cudaMemcpyDeviceToHost,
+            PCS_CUDA(cudaMemcpyAsync((char*)g_ctx.pin_out + j0 * d * 8, coeffs + j0 * d, (j1 - j0) * d * 8, cudaMemcpyDeviceToHost,
                                      g_ctx.d2h_stream));
-        } else if (coeffs_out && !small_out) {
+        } else if (mode == CoeffsOut::direct) {
             for (size_t j = j0; j < j1; j++)
                 if (coeffs_out[j])
-                    PCS_CUDA(cudaMemcpyAsync(coeffs_out[j], staged + j * d, d * 8, cudaMemcpyDeviceToHost, st));
+                    PCS_CUDA(cudaMemcpyAsync(coeffs_out[j], coeffs + j * d, d * 8, cudaMemcpyDeviceToHost, st));
         }
         return PCS_OK;
     };
-    const bool chunked = n_chunks > 0;   // host inputs arriving chunk by chunk: IFFT and LDE follow each chunk
-    if (from_values && !chunked) {
-        int rc = ifft_range(0, w);
-        if (rc) return rc;
-    }
+    if (from_values && !n_chunks)
+        if (int rc = ifft_range(0, w)) return rc;
     PCS_CUDA(cudaEventRecord(b->ev[1], st));
 
     // ---- "FFT + blinding" (oracle.rs:100-125), output already in leaf order ----
-    if (chunked) {
-        for (size_t k = 0; k < n_chunks; k++) {
-            size_t j0 = cb[k], j1 = cb[k + 1];
-            if (pageable) {
-                int rc = stage_pageable(polys + j0, j1 - j0, d, staged + j0 * d, g_ctx.copy_stream);
-                if (rc) {
-                    cudaStreamSynchronize(g_ctx.copy_stream);
-                    return rc;
-                }
-                PCS_CUDA(cudaEventRecord(g_ctx.chunk_ev[k], g_ctx.copy_stream));
-            }
-            PCS_CUDA(cudaStreamWaitEvent(st, g_ctx.chunk_ev[k], 0));
-            if (from_values) {
-                int rc = ifft_range(j0, j1);
-                if (rc) return rc;
-            }
-            PCS_CUDA(ntt_lde_cosets(plan, src + j0 * d, d, b->lde + j0 * n, n, j1 - j0, coset_first, lg_cosets, st));
-            // streaming sponge: hash what has landed while the next chunks are still crossing PCIe (the last group is absorbed
-            // by "build Merkle tree" below, together with the salt columns)
-            b->extended = j1;
-            if (wt > 4 && j1 < w) {
-                int rc = absorb_columns(b, (j1 / 8) * 8, false, st, true);
-                if (rc) return rc;
-            }
+    for (size_t k = 0; k < n_chunks; k++) {
+        const size_t j0 = in.cb[k], j1 = in.cb[k + 1];
+        if (in.pageable) {
+            if (int rc = stage_pageable(polys + j0, j1 - j0, d, coeffs + j0 * d, g_ctx.copy_stream)) return rc;
+            PCS_CUDA(cudaEventRecord(g_ctx.chunk_ev[k], g_ctx.copy_stream));
         }
-    } else {
-        PCS_CUDA(ntt_lde_cosets(plan, src, d, b->lde, n, w, coset_first, lg_cosets, st,
-                                (const uint64_t* const*)ptr_table.p));
+        PCS_CUDA(cudaStreamWaitEvent(st, g_ctx.chunk_ev[k], 0));
+        if (from_values)
+            if (int rc = ifft_range(j0, j1)) return rc;
+        if (int rc = batch_extend(b.get(), src + j0 * d, nullptr, j0, j1 - j0)) return rc;
     }
-    if (small_out) {
-        PCS_CUDA(cudaMemcpyAsync(g_ctx.pin_out, staged, w * d * 8, cudaMemcpyDeviceToHost, st));
-        scatter_coeffs = true;   // scattered to the caller's vectors after the final synchronisation
-    }
-    for (size_t k = 0; k < salt_w; k++) {
-        if (!salts[k]) return fail(PCS_ERR_ARG, "NULL salt pointer");
-        // the caller's salt column k is in natural LDE order like lde_values (oracle.rs:119-123);
-        // leaf order = bit-reversed rows (oracle.rs:84)
-        DevBuf tmp;
-        PCS_CUDA(tmp.alloc(n * 8, st));
-        PCS_CUDA(cudaMemcpyAsync(tmp.p, salts[k], n * 8, dev_ptrs ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
-        PCS_CUDA(launch_canonicalize(tmp.u64(), n, st));
-        if (shard)   // already in leaf order
-            PCS_CUDA(cudaMemcpyAsync(b->lde + (w + k) * n, tmp.p, n * 8, cudaMemcpyDeviceToDevice, st));
-        else
-            PCS_CUDA(launch_bitrev_permute(tmp.u64(), n, b->lde + (w + k) * n, n, 1, lg_n, st));
-    }
-    PCS_CUDA(cudaEventRecord(b->ev[2], st));
-    // "transpose LDEs" (oracle.rs:83): fused away -- the hash kernel reads columns directly
-    PCS_CUDA(cudaEventRecord(b->ev[3], st));
+    if (!n_chunks)
+        if (int rc = batch_extend(b.get(), src, in.dev.ptrs, 0, w)) return rc;
+    if (mode == CoeffsOut::small_pinned) PCS_CUDA(cudaMemcpyAsync(g_ctx.pin_out, coeffs, w * d * 8, cudaMemcpyDeviceToHost, st));
+    if (int rc = write_salts(b.get(), salts, dev_ptrs, shard, st)) return rc;
 
-    // ---- "build Merkle tree" (oracle.rs:85-89) ----
-    int rc;
-    if (b->absorbed > 0) {
-        rc = absorb_columns(b, wt, true, st, false);     // the remaining columns (+ salts) and the digests
-        if (rc) return rc;
-        PCS_CUDA(cudaEventRecord(b->ev[4], st));
-        rc = node_levels_dev(n, lg_n - cap_height, b->digests, b->cap, st);
-    } else {
-        rc = build_tree_dev(b->lde, n, wt, lg_n, cap_height, b->digests, b->cap, st, b->ev[4]);
-    }
-    if (rc) return rc;
-    PCS_CUDA(cudaEventRecord(b->ev[5], st));
-
+    // ---- "transpose LDEs" (fused away), "build Merkle tree" (oracle.rs:83-89) ----
+    if (int rc = batch_finish(b.get(), cap_out)) return rc;
     if (b->coeffs && !from_values && !(flags & PCS_KEEP_COEFFS)) {
         cudaFreeAsync(b->coeffs, st);
         b->coeffs = nullptr;
     }
-    if (cap_out) {
-        PCS_CUDA(cudaMemcpyAsync(cap_out, b->cap, n_cap * 32, cudaMemcpyDeviceToHost, st));
-        PCS_CUDA(cudaStreamSynchronize(st));
-    } else if (!dev_ptrs || scatter_coeffs) {
+    if (!cap_out && (!dev_ptrs || mode == CoeffsOut::small_pinned))
         PCS_CUDA(cudaStreamSynchronize(st));  // host inputs must not be reused before the copies finish
-    }
-    if (scatter_coeffs)
-        for (size_t j = 0; j < w; j++)
-            if (coeffs_out[j]) memcpy(coeffs_out[j], (char*)g_ctx.pin_out + j * d * 8, d * 8);
-    if (big_out) {
-        PCS_CUDA(cudaStreamSynchronize(st));
-        PCS_CUDA(cudaStreamSynchronize(g_ctx.d2h_stream));
-        const unsigned nt = STAGE_THREADS;
-        std::thread th[STAGE_THREADS];
-        const char* srcp = (const char*)g_ctx.pin_out;
-        for (unsigned t = 0; t < nt; t++)
-            th[t] = std::thread([=]() {
-                for (size_t j = t; j < w; j += nt)
-                    if (coeffs_out[j]) memcpy(coeffs_out[j], srcp + j * d * 8, d * 8);
-            });
-        for (unsigned t = 0; t < nt; t++) th[t].join();
-    }
-    guard.armed = false;
-    copy_drain.armed = false;   // the main stream waited on every chunk event and has been synchronised (host inputs)
-    b->committed = true;
-    *out = b;
+    if (int rc = hand_back_coeffs(mode, coeffs_out, w, d)) return rc;
+    drain.armed = false;   // the main stream waited on every chunk event and has been synchronised (host inputs)
+    *out = b.release();
     return PCS_OK;
 }
+
+extern "C" {
 
 int pcs_commit_from_coeffs(const uint64_t* const* polys, size_t w, unsigned lg_d, unsigned rate_bits,
                            unsigned cap_height, const uint64_t* const* salts, size_t salt_w, unsigned flags,
@@ -1004,67 +1055,37 @@ int pcs_commit_shard_from_coeffs(const uint64_t* const* polys, size_t w, unsigne
 }
 
 // ---- streaming shard commit: the polynomials arrive in groups (e.g. chunks of an all-gather still in flight) ----
+// The input and IFFT phases of such a shard are empty.
+static int shard_open(BatchOwner& b, pcs_batch** out) {
+    PCS_CUDA(cudaEventRecord(b->ev[0], g_ctx.stream));
+    PCS_CUDA(cudaEventRecord(b->ev[1], g_ctx.stream));
+    *out = b.release();
+    return PCS_OK;
+}
+
 int pcs_shard_begin(size_t w, size_t salt_w, unsigned lg_d, unsigned rate_bits, unsigned coset_first, unsigned lg_cosets,
                     unsigned local_cap_height, pcs_batch** out) {
-    PCS_NEED_INIT();
+    if (int rc = need_init()) return rc;
     if (!out) return fail(PCS_ERR_ARG, "out is NULL");
     *out = nullptr;
     if (w == 0) return fail(PCS_ERR_ARG, "empty batch (oracle.rs:76 polynomials[0])");
-    if (lg_d + rate_bits > 32) return fail(PCS_ERR_TWO_ADICITY, "n_log <= TWO_ADICITY violated");
-    if (lg_cosets > rate_bits || ((size_t)coset_first + ((size_t)1 << lg_cosets)) > ((size_t)1 << rate_bits))
-        return fail(PCS_ERR_ARG, "coset range outside [0, 2^rate_bits)");
-    unsigned lg_n = lg_d + lg_cosets;
-    if (local_cap_height > lg_n)
-        return fail(PCS_ERR_CAP_HEIGHT, "cap_height=" + std::to_string(local_cap_height) +
-                                            " should be at most log2(leaves.len())=" + std::to_string(lg_n));
-    cudaStream_t st = g_ctx.stream;
-    if (!ntt_plan_get(lg_d, rate_bits, false, 7, st)) return fail(PCS_ERR_ALLOC, "twiddle table allocation failed");
-    const size_t n = (size_t)1 << lg_n, n_cap = (size_t)1 << local_cap_height;
-    pcs_batch* b = batch_new();
-    b->w = w; b->salt_w = salt_w; b->lg_d = lg_d; b->rate_bits = lg_cosets; b->cap_height = local_cap_height;
-    b->full_rate_bits = rate_bits; b->coset_first = coset_first;
-    b->n = n; b->n_digests = 2 * (n - n_cap);
-    struct Guard { pcs_batch* b; bool armed = true; ~Guard() { if (armed) pcs_batch_free(b); } } guard{b};
-    for (auto& e : b->ev) PCS_CUDA(cudaEventCreate(&e));
-    PCS_CUDA(cudaMallocAsync((void**)&b->lde, (w + salt_w) * n * 8, st));
-    PCS_CUDA(cudaMallocAsync((void**)&b->digests, b->n_digests ? b->n_digests * 32 : 32, st));
-    PCS_CUDA(cudaMallocAsync((void**)&b->cap, n_cap * 32, st));
-    PCS_CUDA(cudaEventRecord(b->ev[0], st));
-    PCS_CUDA(cudaEventRecord(b->ev[1], st));
-    guard.armed = false;
-    *out = b;
-    return PCS_OK;
+    BatchOwner b;
+    if (int rc = batch_begin(w, salt_w, lg_d, rate_bits, coset_first, lg_cosets, local_cap_height, BATCH_LDE, b)) return rc;
+    return shard_open(b, out);
 }
 
 // A tree shard whose LDE rows are computed elsewhere (another GPU's LDE arriving over NVLink: the north-star's
 // polynomial-partitioned LDE + all-to-all): `width` rows of 2^lg_n leaves each, filled through pcs_shard_set_rows or written
 // in place at pcs_batch_lde_dev() + row * 2^lg_n, then pcs_shard_finish.
 int pcs_shard_begin_rows(size_t width, size_t salt_w, unsigned lg_n, unsigned local_cap_height, pcs_batch** out) {
-    PCS_NEED_INIT();
+    if (int rc = need_init()) return rc;
     if (!out) return fail(PCS_ERR_ARG, "out is NULL");
     *out = nullptr;
     if (width == 0) return fail(PCS_ERR_ARG, "empty batch (oracle.rs:76 polynomials[0])");
     if (salt_w > width) return fail(PCS_ERR_ARG, "more salt columns than columns");
-    if (lg_n > 32) return fail(PCS_ERR_TWO_ADICITY, "n_log <= TWO_ADICITY violated");
-    if (local_cap_height > lg_n)
-        return fail(PCS_ERR_CAP_HEIGHT, "cap_height=" + std::to_string(local_cap_height) +
-                                            " should be at most log2(leaves.len())=" + std::to_string(lg_n));
-    cudaStream_t st = g_ctx.stream;
-    const size_t n = (size_t)1 << lg_n, n_cap = (size_t)1 << local_cap_height;
-    pcs_batch* b = batch_new();
-    b->w = width - salt_w; b->salt_w = salt_w; b->lg_d = lg_n; b->rate_bits = 0; b->cap_height = local_cap_height;
-    b->full_rate_bits = 0; b->coset_first = 0; b->rows_only = true;
-    b->n = n; b->n_digests = 2 * (n - n_cap);
-    struct Guard { pcs_batch* b; bool armed = true; ~Guard() { if (armed) pcs_batch_free(b); } } guard{b};
-    for (auto& e : b->ev) PCS_CUDA(cudaEventCreate(&e));
-    PCS_CUDA(cudaMallocAsync((void**)&b->lde, width * n * 8, st));
-    PCS_CUDA(cudaMallocAsync((void**)&b->digests, b->n_digests ? b->n_digests * 32 : 32, st));
-    PCS_CUDA(cudaMallocAsync((void**)&b->cap, n_cap * 32, st));
-    PCS_CUDA(cudaEventRecord(b->ev[0], st));
-    PCS_CUDA(cudaEventRecord(b->ev[1], st));
-    guard.armed = false;
-    *out = b;
-    return PCS_OK;
+    BatchOwner b;
+    if (int rc = batch_begin(width - salt_w, salt_w, lg_n, 0, 0, 0, local_cap_height, BATCH_ROWS, b)) return rc;
+    return shard_open(b, out);
 }
 
 int pcs_shard_set_rows(pcs_batch* b, size_t row_first, size_t count, const uint64_t* const* rows_dev, int canonical) {
@@ -1091,66 +1112,16 @@ int pcs_shard_extend(pcs_batch* b, size_t poly_first, size_t count, const uint64
     if (b->rows_only) return fail(PCS_ERR_ARG, "this shard takes LDE rows (pcs_shard_set_rows), not polynomials");
     if (poly_first > b->w || count > b->w - poly_first) return fail(PCS_ERR_ARG, "polynomial range out of bounds");
     if (count == 0) return PCS_OK;
-    cudaStream_t st = g_ctx.stream;
-    const size_t d = (size_t)1 << b->lg_d;
-    NttPlan* plan = ntt_plan_get(b->lg_d, b->full_rate_bits, false, 7, st);
-    if (!plan) return fail(PCS_ERR_ALLOC, "twiddle table allocation failed");
-    bool contiguous = true;
-    for (size_t j = 0; j < count; j++) {
-        if (!polys[j]) return fail(PCS_ERR_ARG, "NULL polynomial pointer");
-        contiguous = contiguous && polys[j] == polys[0] + j * d;
-    }
-    DevBuf table, staged;
-    const uint64_t* src = polys[0];
-    const uint64_t* const* ptrs = nullptr;
-    if (!contiguous) {
-        if (b->lg_d >= 1) {
-            PCS_CUDA(table.alloc(count * sizeof(uint64_t*), st));
-            PCS_CUDA(cudaMemcpyAsync(table.p, polys, count * sizeof(uint64_t*), cudaMemcpyHostToDevice, st));
-            ptrs = (const uint64_t* const*)table.p;
-        } else {
-            PCS_CUDA(staged.alloc(count * d * 8, st));
-            int rc = stage_polys(polys, count, d, true, staged.u64(), st);
-            if (rc) return rc;
-            src = staged.u64();
-        }
-    }
-    PCS_CUDA(ntt_lde_cosets(plan, src, d, b->lde + poly_first * b->n, b->n, count, b->coset_first, b->rate_bits, st, ptrs));
-    // streaming sponge: groups that arrive in order are hashed at once (while the next group's coefficients are still in
-    // flight); a shard that gets all its polynomials in one call keeps the single hash kernel of pcs_shard_finish
-    if (poly_first == b->extended) b->extended += count;
-    const bool whole = poly_first == 0 && count == b->w;
-    if (!whole && b->w + b->salt_w > 4 && b->extended < b->w) {
-        int rc = absorb_columns(b, (b->extended / 8) * 8, false, st, true);
-        if (rc) return rc;
-    }
-    return PCS_OK;   // asynchronous on pcs_stream()
+    DevInput in;
+    if (int rc = resolve_dev_input(polys, count, b->lg_d, g_ctx.stream, in)) return rc;
+    return batch_extend(b, in.src, in.ptrs, poly_first, count);   // asynchronous on pcs_stream()
 }
 
 int pcs_shard_finish(pcs_batch* b, uint64_t* cap_out) {
     BatchScope scope(b);
     if (!b) return fail(PCS_ERR_ARG, "NULL pointer");
     if (b->committed) return fail(PCS_ERR_ARG, "batch already finished");
-    cudaStream_t st = g_ctx.stream;
-    PCS_CUDA(cudaEventRecord(b->ev[2], st));
-    PCS_CUDA(cudaEventRecord(b->ev[3], st));
-    int rc;
-    if (b->absorbed > 0) {
-        rc = absorb_columns(b, b->w + b->salt_w, true, st, false);
-        if (rc) return rc;
-        PCS_CUDA(cudaEventRecord(b->ev[4], st));
-        rc = node_levels_dev(b->n, b->lg_d + b->rate_bits - b->cap_height, b->digests, b->cap, st);
-    } else {
-        rc = build_tree_dev(b->lde, b->n, b->w + b->salt_w, b->lg_d + b->rate_bits, b->cap_height, b->digests, b->cap, st, b->ev[4]);
-    }
-    if (rc) return rc;
-    PCS_CUDA(cudaEventRecord(b->ev[5], st));
-    b->committed = true;
-    if (cap_out) {
-        PCS_CUDA(cudaMemcpyAsync(cap_out, b->cap, ((size_t)32) << b->cap_height, cudaMemcpyDeviceToHost, st));
-        PCS_CUDA(cudaStreamSynchronize(st));
-    }
-    return PCS_OK;
+    return batch_finish(b, cap_out);
 }
 
 int pcs_commit_from_values(const uint64_t* const* values, size_t w, unsigned lg_d, unsigned rate_bits,
@@ -1318,18 +1289,11 @@ int pcs_batch_timings(const pcs_batch* b, float ms[5]) {
     BatchScope scope(b);
     if (!b || !ms) return fail(PCS_ERR_ARG, "NULL pointer");
     PCS_CUDA(cudaStreamSynchronize(g_ctx.stream));
-    for (int i = 0; i < 5; i++) PCS_CUDA(cudaEventElapsedTime(&ms[i], b->ev[i], b->ev[i + 1]));
-    for (size_t k = 0; k + 1 < b->absorb_ev.size(); k += 2) {   // streamed leaf hashing ran inside the LDE phase
-        float t = 0;
-        PCS_CUDA(cudaEventElapsedTime(&t, b->absorb_ev[k], b->absorb_ev[k + 1]));
-        ms[1] -= t;
-        ms[3] += t;
-    }
-    return PCS_OK;
+    return phase_times(b, ms);
 }
 
 int pcs_timing_totals(float ms[5], unsigned* n_commits, int reset) {
-    PCS_NEED_INIT();
+    if (int rc = need_init()) return rc;
     PCS_CUDA(cudaStreamSynchronize(g_ctx.stream));
     drain_pending();
     if (ms)

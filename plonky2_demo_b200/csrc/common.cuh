@@ -4,6 +4,7 @@
 #include <stddef.h>
 #include <stdint.h>
 
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -48,10 +49,48 @@ void set_error(const std::string& msg);
 
 
 int fail(int code, const std::string& msg);   // set_error + return code
+// Initialise the engine on first use, else re-select the current context's device (the caller -- torch ... -- may have
+// switched this thread's device).  Every entry point that works on the current context starts with it (api.cu).
+int need_init();
+// argument checks shared by the entry points: PCS_OK, or the reference's panic message and its code
+static inline int check_two_adicity(unsigned lg_n) {
+    return lg_n > 32 ? fail(PCS_ERR_TWO_ADICITY, "n_log <= TWO_ADICITY violated") : PCS_OK;
+}
+static inline int check_cap_height(unsigned cap_height, unsigned lg_n) {
+    if (cap_height <= lg_n) return PCS_OK;
+    return fail(PCS_ERR_CAP_HEIGHT, "cap_height=" + std::to_string(cap_height) +
+                                        " should be at most log2(leaves.len())=" + std::to_string(lg_n));
+}
+static inline int check_shift(uint64_t shift) {   // a coset shift must be a unit
+    return shift % 0xFFFFFFFF00000001ULL == 0 ? fail(PCS_ERR_ARG, "shift must be non-zero") : PCS_OK;
+}
 // host polynomials (pageable memory) -> contiguous device block through the current context's pinned ring (api.cu)
 int stage_pageable(const uint64_t* const* polys, size_t count, size_t d, uint64_t* dst, cudaStream_t copy_st);
+bool is_pageable_host(const void* p);         // not page-locked or registered: plain copies stage through the driver (api.cu)
 void multi_shutdown_locked();                 // multi.cu: release the multi-GPU state (called by pcs_shutdown)
 pcs_batch* batch_new();                       // a batch bound to the calling thread's current context (api.cu)
+struct BatchFree {
+    void operator()(pcs_batch* b) const { pcs_batch_free(b); }
+};
+using BatchOwner = std::unique_ptr<pcs_batch, BatchFree>;   // frees the batch on every exit until it is released
+
+// One commitment's lifecycle (api.cu), shared by the single-GPU commit, the shard commits and every device of pcs_multi_*.
+//   batch_begin:  checks the shape and allocates the batch (LDE rows, digests, cap) of the cosets [coset_first,
+//                 coset_first + 2^lg_cosets) of a rate-2^rate_bits LDE of w polynomials of degree 2^lg_d plus salt_w salt
+//                 rows, with a Merkle tree of cap height cap_height over its d << lg_cosets leaves.
+//   batch_extend: the LDE rows of polynomials [first, first + count), read from src + j * d or from a device table of
+//                 pointers; polynomials that arrive in order are leaf-hashed at once (streaming sponge).
+//   batch_finish: records phase events 2-5, hashes the remaining columns (or all of them), builds the node levels and marks
+//                 the batch committed; with cap_out, copies the cap out and synchronises.
+enum BatchKind : unsigned {
+    BATCH_LDE = 0,        // polynomials are extended by batch_extend (its twiddle tables are made here)
+    BATCH_ROWS = 1,       // the caller writes the LDE rows itself
+    BATCH_UNTIMED = 2,    // no phase events
+};
+int batch_begin(size_t w, size_t salt_w, unsigned lg_d, unsigned rate_bits, unsigned coset_first, unsigned lg_cosets,
+                unsigned cap_height, unsigned kind, BatchOwner& out);
+int batch_extend(pcs_batch* b, const uint64_t* src, const uint64_t* const* ptr_table, size_t first, size_t count);
+int batch_finish(pcs_batch* b, uint64_t* cap_out);
 // Run on the context (device + stream) that owns `b`, whatever the calling thread's current one is; the caller's
 // context is restored on destruction (api.cu).
 struct BatchScope {

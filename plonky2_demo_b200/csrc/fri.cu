@@ -469,8 +469,6 @@ __global__ void k_fri_leaf_columns(const uint64_t* __restrict__ lde /*[2][n]*/, 
 
 inline unsigned blocks_for(size_t n, unsigned threads) { return (unsigned)((n + threads - 1) / threads); }
 
-int need_init() { return pcs_init(-1, nullptr); }   // no-op once the engine is up
-
 // E = suffix scan of c (both [2][stride] component-major, n elements) at point z; e may alias c
 int ext_suffix_scan(const uint64_t* c, size_t c_stride, size_t n, glh::ext2 z, uint64_t* e, size_t e_stride,
                     cudaStream_t st) {
@@ -557,7 +555,7 @@ int pcs_eval_ext_dev(const uint64_t* const* polys_dev, size_t w, unsigned lg_d, 
     if (int rc = need_init()) return rc;
     if (w == 0) return PCS_OK;
     if (!polys_dev || !point || !out) return fail(PCS_ERR_ARG, "NULL pointer");
-    if (lg_d > 32) return fail(PCS_ERR_TWO_ADICITY, "n_log <= TWO_ADICITY violated");
+    if (int rc = check_two_adicity(lg_d)) return rc;
     return eval_ext_common(nullptr, polys_dev, w, lg_d, point, out);
 }
 
@@ -716,7 +714,7 @@ int pcs_fri_final_poly_dev(const uint64_t* const* polys_dev, unsigned lg_d, size
     if (!out) return fail(PCS_ERR_ARG, "out is NULL");
     *out = nullptr;
     if (!polys_dev || !n_batches || !points || !batch_len || !alpha) return fail(PCS_ERR_ARG, "NULL pointer or empty instance");
-    if (lg_d > 32) return fail(PCS_ERR_TWO_ADICITY, "n_log <= TWO_ADICITY violated");
+    if (int rc = check_two_adicity(lg_d)) return rc;
     size_t total = 0;
     for (size_t i = 0; i < n_batches; i++) {
         if (batch_len[i] == 0) return fail(PCS_ERR_ARG, "empty FRI batch");
@@ -734,8 +732,8 @@ static int ext_lde(const pcs_ext_poly* p, unsigned rate_bits, uint64_t shift, ui
                    cudaStream_t st) {
     int lg_d = ilog2_strict(p->len);
     if (lg_d < 0) return fail(PCS_ERR_NOT_POW2, "Not a power of two: " + std::to_string(p->len));
-    if ((unsigned)lg_d + rate_bits > 32) return fail(PCS_ERR_TWO_ADICITY, "n_log <= TWO_ADICITY violated");
-    if (shift % glh::P == 0) return fail(PCS_ERR_ARG, "shift must be non-zero");
+    if (int rc = check_two_adicity((unsigned)lg_d + rate_bits)) return rc;
+    if (int rc = check_shift(shift)) return rc;
     NttPlan* plan = ntt_plan_get((unsigned)lg_d, rate_bits, false, shift % glh::P, st);
     if (!plan) return fail(PCS_ERR_ALLOC, "twiddle table allocation failed");
     const size_t n = p->len << rate_bits;
@@ -777,18 +775,10 @@ int pcs_fri_commit_layer(const pcs_ext_poly* p, unsigned rate_bits, uint64_t shi
     const unsigned lg_n = (unsigned)lg_d + rate_bits;
     if (arity_bits > lg_n) return fail(PCS_ERR_ARG, "arity larger than the LDE");
     const unsigned lg_leaves = lg_n - arity_bits;
-    if (cap_height > lg_leaves)
-        return fail(PCS_ERR_CAP_HEIGHT, "cap_height=" + std::to_string(cap_height) +
-                                            " should be at most log2(leaves.len())=" + std::to_string(lg_leaves));
     const size_t n = (size_t)1 << lg_n, n_leaves = (size_t)1 << lg_leaves, width = (size_t)2 << arity_bits;
     const size_t n_cap = (size_t)1 << cap_height;
-    pcs_batch* b = batch_new();
-    b->w = width; b->lg_d = lg_leaves; b->rate_bits = 0; b->full_rate_bits = 0; b->cap_height = cap_height;
-    b->n = n_leaves; b->n_digests = 2 * (n_leaves - n_cap);
-    struct Guard { pcs_batch* b; bool armed = true; ~Guard() { if (armed) pcs_batch_free(b); } } guard{b};
-    PCS_CUDA(cudaMallocAsync((void**)&b->lde, width * n_leaves * 8, st));
-    PCS_CUDA(cudaMallocAsync((void**)&b->digests, b->n_digests ? b->n_digests * 32 : 32, st));
-    PCS_CUDA(cudaMallocAsync((void**)&b->cap, n_cap * 32, st));
+    BatchOwner b;   // a tree over rows written here, without phase events
+    if (int rc = batch_begin(width, 0, lg_leaves, 0, 0, 0, cap_height, BATCH_ROWS | BATCH_UNTIMED, b)) return rc;
     DevBuf lde;
     PCS_CUDA(lde.alloc(2 * n * 8, st));
     unsigned lg_n2 = 0;
@@ -802,8 +792,7 @@ int pcs_fri_commit_layer(const pcs_ext_poly* p, unsigned rate_bits, uint64_t shi
         PCS_CUDA(cudaMemcpyAsync(cap_out, b->cap, n_cap * 32, cudaMemcpyDeviceToHost, st));
         PCS_CUDA(cudaStreamSynchronize(st));
     }
-    guard.armed = false;
-    *tree = b;
+    *tree = b.release();
     return PCS_OK;
 }
 

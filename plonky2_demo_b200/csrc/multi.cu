@@ -140,6 +140,24 @@ struct Plan {
     }
 };
 
+// The levels of two_to_one above the devices' local caps (merkle_tree.rs:69-96): `level` (digests in device order) becomes the
+// level `levels` above.  With `siblings`, the sibling of node `idx` is collected at every level on the way, bottom-up.
+int combine_top_levels(std::vector<uint64_t>& level, unsigned levels, size_t idx, uint64_t* siblings) {
+    for (unsigned t = 0; t < levels; t++, idx >>= 1) {
+        if (siblings) memcpy(siblings + (size_t)t * 4, level.data() + (idx ^ 1) * 4, 32);
+        const size_t m = level.size() / 8;
+        std::vector<uint64_t> l(m * 4), r(m * 4), o(m * 4);
+        for (size_t i = 0; i < m; i++)
+            for (int k = 0; k < 4; k++) {
+                l[4 * i + k] = level[8 * i + k];
+                r[4 * i + k] = level[8 * i + 4 + k];
+            }
+        if (int rc = pcs_two_to_one(l.data(), r.data(), m, o.data())) return rc;
+        level.swap(o);
+    }
+    return PCS_OK;
+}
+
 }  // namespace
 
 void multi_shutdown_locked() {
@@ -265,10 +283,8 @@ static int multi_commit(const uint64_t* const* polys, bool from_values, size_t w
     if (!g_multi.init) return fail(PCS_ERR_NOT_INIT, "pcs_multi_init has not been called");
     if (w == 0 || !polys) return fail(PCS_ERR_ARG, "empty batch (oracle.rs:76 polynomials[0])");
     if (salt_w && !salts) return fail(PCS_ERR_ARG, "salts is NULL");
-    if (lg_d + rate_bits > 32) return fail(PCS_ERR_TWO_ADICITY, "n_log <= TWO_ADICITY violated");
-    if (cap_height > lg_d + rate_bits)
-        return fail(PCS_ERR_CAP_HEIGHT, "cap_height=" + std::to_string(cap_height) +
-                                            " should be at most log2(leaves.len())=" + std::to_string(lg_d + rate_bits));
+    if (int rc = check_two_adicity(lg_d + rate_bits)) return rc;
+    if (int rc = check_cap_height(cap_height, lg_d + rate_bits)) return rc;
     for (size_t j = 0; j < w; j++)
         if (!polys[j]) return fail(PCS_ERR_ARG, "NULL polynomial pointer");
     std::lock_guard<std::recursive_mutex> lock(g_multi_mutex);
@@ -453,10 +469,7 @@ static int multi_commit(const uint64_t* const* polys, bool from_values, size_t w
                                 for (size_t j = a; j < b; j++)
                                     PCS_CUDA(cudaMemcpyAsync(dst + (j - a) * d, polys[j], d * 8, cudaMemcpyDefault, cst));
                             } else {
-                                cudaPointerAttributes at;
-                                bool pageable = cudaPointerGetAttributes(&at, polys[a]) != cudaSuccess || at.type == cudaMemoryTypeUnregistered;
-                                cudaGetLastError();
-                                if (pageable && (b - a) * d * 8 >= (1u << 20)) {
+                                if (is_pageable_host(polys[a]) && (b - a) * d * 8 >= (1u << 20)) {
                                     rc = stage_pageable(polys + a, b - a, d, dst, cst);
                                     if (rc) return rc;
                                 } else {
@@ -567,20 +580,8 @@ static int multi_commit(const uint64_t* const* polys, bool from_values, size_t w
     if (staged && !keep) mb->poly_ptr.clear();   // the blocks go back to the pool: PolynomialBatch.polynomials was not asked for
 
     // ---- cap: local caps in device order; above them log2(G) - cap_height levels of two_to_one (merkle_tree.rs:69-96) ----
-    std::vector<uint64_t> level = mb->local_caps;
-    for (unsigned t = 0; t < plan.top_levels; t++) {
-        const size_t m = level.size() / 8;
-        std::vector<uint64_t> l(m * 4), r(m * 4), o(m * 4);
-        for (size_t i = 0; i < m; i++)
-            for (int k = 0; k < 4; k++) {
-                l[4 * i + k] = level[8 * i + k];
-                r[4 * i + k] = level[8 * i + 4 + k];
-            }
-        int rc = pcs_two_to_one(l.data(), r.data(), m, o.data());
-        if (rc) return rc;
-        level.swap(o);
-    }
-    mb->cap = level;
+    mb->cap = mb->local_caps;
+    if (int rc = combine_top_levels(mb->cap, plan.top_levels, 0, nullptr)) return rc;
     if (cap_out) memcpy(cap_out, mb->cap.data(), mb->cap.size() * 8);
     guard.armed = false;
     *out = mb;
@@ -661,22 +662,7 @@ int pcs_multi_batch_prove(const pcs_multi_batch* mb, size_t leaf_index, uint64_t
     if (rc) return rc;
     // above the device's root (n_dev > 2^cap_height): siblings from the other devices' roots, combined level by level
     std::vector<uint64_t> level = mb->local_caps;   // local_cap_height == 0 here: one root per device
-    size_t idx = (size_t)g;
-    for (unsigned t = 0; t < mb->top_levels; t++) {
-        memcpy(siblings + (size_t)(n_local + t) * 4, level.data() + (idx ^ 1) * 4, 32);
-        const size_t m = level.size() / 8;
-        std::vector<uint64_t> l(m * 4), r(m * 4), o(m * 4);
-        for (size_t i = 0; i < m; i++)
-            for (int k = 0; k < 4; k++) {
-                l[4 * i + k] = level[8 * i + k];
-                r[4 * i + k] = level[8 * i + 4 + k];
-            }
-        rc = pcs_two_to_one(l.data(), r.data(), m, o.data());
-        if (rc) return rc;
-        level.swap(o);
-        idx >>= 1;
-    }
-    return PCS_OK;
+    return combine_top_levels(level, mb->top_levels, (size_t)g, siblings + (size_t)n_local * 4);
 }
 
 int pcs_multi_batch_timings(const pcs_multi_batch* mb, float ms[5]) {
