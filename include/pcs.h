@@ -57,7 +57,15 @@ typedef enum {
 enum {
     PCS_DEVICE_PTRS = 1u << 0,   /* input polynomial pointers are device pointers (no H2D copy)         */
     PCS_KEEP_COEFFS = 1u << 1,   /* keep the coefficient vectors on the device (PolynomialBatch.polynomials) */
-    PCS_MULTI_CE_GATHER = 1u << 2    /* pcs_multi_*: exchange by copy-engine gathers instead of peer loads inside the first NTT pass (slower; kept for A/B) */
+    PCS_MULTI_CE_GATHER = 1u << 2,   /* pcs_multi_*: exchange by copy-engine gathers instead of peer loads inside the first NTT pass (slower; kept for A/B) */
+    PCS_LDE_ON_DEMAND = 1u << 3      /* pcs_commit_from_coeffs / _from_values: keep no LDE rows in HBM.  The LDE is extended and
+                                      * hashed a few columns at a time through a reused scratch buffer; the batch keeps the
+                                      * coefficients (implies PCS_KEEP_COEFFS: device inputs are copied), salts, digests and
+                                      * cap, about 1 / (2^rate_bits + 1) of a resident batch's HBM plus the salt rows.  The
+                                      * commitment is bit-identical.  pcs_batch_get_rows, pcs_batch_leaves and
+                                      * pcs_batch_lde_natural recompute the rows they return (few rows: evaluated from the
+                                      * coefficients; many: the LDE regenerated group by group); pcs_batch_lde_dev returns NULL.
+                                      * Refused (PCS_ERR_ARG) by the shard and pcs_multi_* commits. */
 };
 
 /* ---- lifetime ------------------------------------------------------------------------------- */
@@ -210,7 +218,8 @@ PCS_API int pcs_batch_prove_many(const pcs_batch* b, const uint64_t* leaf_indice
 PCS_API int pcs_batch_coeffs(const pcs_batch* b, size_t poly, uint64_t* coeffs /*[d]*/);
 /* All of `polynomials` at once as one [w][d] matrix.                                                  */
 PCS_API int pcs_batch_all_coeffs(const pcs_batch* b, uint64_t* coeffs /*[w][d]*/);
-/* Device views (valid until pcs_batch_free): LDE is [leaf_len][N] poly-major in leaf order.        */
+/* Device views (valid until pcs_batch_free): LDE is [leaf_len][N] poly-major in leaf order, NULL for a batch committed
+ * with PCS_LDE_ON_DEMAND (it keeps no LDE rows).                                                    */
 PCS_API const uint64_t* pcs_batch_lde_dev(const pcs_batch* b);
 PCS_API const uint64_t* pcs_batch_coeffs_dev(const pcs_batch* b);   /* [w][d], or NULL when the coefficients were not kept */
 PCS_API const uint64_t* pcs_batch_digests_dev(const pcs_batch* b);

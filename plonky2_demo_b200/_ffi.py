@@ -15,6 +15,7 @@ sz = C.c_size_t
 PCS_DEVICE_PTRS = 1
 PCS_KEEP_COEFFS = 2
 PCS_MULTI_CE_GATHER = 4
+PCS_LDE_ON_DEMAND = 8
 
 # every symbol include/pcs.h declares: name -> (restype, argtypes)
 SIGNATURES = {

@@ -144,8 +144,9 @@ int build_tree_dev(const uint64_t* cols, size_t n, size_t width, unsigned lg_n, 
 }
 
 // Streaming sponge: absorb the LDE columns [b->absorbed, upto) of every leaf (upto a multiple of the rate, or all columns
-// with last = true, which also emits the digests).  timed: bracket the launch with an event pair (absorbs that run inside the
-// "FFT + blinding" phase are booked as leaf hashing by the timing queries).
+// with last = true, which also emits the digests); an on-demand batch holds them at the start of its group scratch.
+// timed: bracket the launch with an event pair (absorbs that run inside the "FFT + blinding" phase are booked as leaf hashing
+// by the timing queries).
 static int absorb_columns(pcs_batch* b, size_t upto, bool last, cudaStream_t st, bool timed) {
     if (upto < b->absorbed) return fail(PCS_ERR_ARG, "internal: sponge cannot go backwards");
     if (upto == b->absorbed && !last) return PCS_OK;
@@ -160,7 +161,8 @@ static int absorb_columns(pcs_batch* b, size_t upto, bool last, cudaStream_t st,
         b->absorb_ev.push_back(e1);
         PCS_CUDA(cudaEventRecord(e0, st));
     }
-    PCS_CUDA(launch_leaf_hash_group(b->lde + b->absorbed * b->n, b->n, (uint32_t)(upto - b->absorbed), b->n, first, last, b->sponge,
+    const uint64_t* cols = b->on_demand ? b->scratch : b->lde + b->absorbed * b->n;
+    PCS_CUDA(launch_leaf_hash_group(cols, b->n, (uint32_t)(upto - b->absorbed), b->n, first, last, b->sponge,
                                     lg_sub, b->digests, b->cap, st));
     if (timed) PCS_CUDA(cudaEventRecord(e1, st));
     b->absorbed = upto;
@@ -185,10 +187,14 @@ int batch_begin(size_t w, size_t salt_w, unsigned lg_d, unsigned rate_bits, unsi
     BatchOwner b(batch_new());
     b->w = w; b->salt_w = salt_w; b->lg_d = lg_d; b->rate_bits = lg_cosets; b->cap_height = cap_height;
     b->full_rate_bits = rate_bits; b->coset_first = coset_first; b->rows_only = kind & BATCH_ROWS;
+    b->on_demand = kind & BATCH_ON_DEMAND;
     b->n = n; b->n_digests = 2 * (n - n_cap);
     if (!(kind & BATCH_UNTIMED))
         for (auto& e : b->ev) PCS_CUDA(cudaEventCreate(&e));
-    PCS_CUDA(cudaMallocAsync((void**)&b->lde, (w + salt_w) * n * 8, st));
+    if (b->on_demand)
+        PCS_CUDA(cudaMallocAsync((void**)&b->salts, salt_w * n * 8, st));
+    else
+        PCS_CUDA(cudaMallocAsync((void**)&b->lde, (w + salt_w) * n * 8, st));
     PCS_CUDA(cudaMallocAsync((void**)&b->digests, b->n_digests ? b->n_digests * 32 : 32, st));
     PCS_CUDA(cudaMallocAsync((void**)&b->cap, n_cap * 32, st));
     out = std::move(b);
@@ -199,14 +205,20 @@ int batch_extend(pcs_batch* b, const uint64_t* src, const uint64_t* const* ptr_t
     cudaStream_t st = g_ctx.stream;
     NttPlan* plan = ntt_plan_get(b->lg_d, b->full_rate_bits, false, 7, st);
     if (!plan) return fail(PCS_ERR_ALLOC, "twiddle table allocation failed");
-    PCS_CUDA(ntt_lde_cosets(plan, src, (size_t)1 << b->lg_d, b->lde + first * b->n, b->n, count, b->coset_first, b->rate_bits, st,
-                            ptr_table));
+    // an on-demand batch gets its polynomials in order, one group of <= LDE_GROUP at a time: each overwrites the scratch
+    // once the previous one has been absorbed (stream order)
+    uint64_t* const dst = b->on_demand ? b->scratch : b->lde + first * b->n;
+    PCS_CUDA(ntt_lde_cosets(plan, src, (size_t)1 << b->lg_d, dst, b->n, count, b->coset_first, b->rate_bits, st, ptr_table));
     // streaming sponge: groups that arrive in order are hashed at once, up to a multiple of the sponge rate, while later
     // groups are still in flight; the last group is absorbed by batch_finish together with the salt columns, and a batch
     // that gets all its polynomials in one call keeps the single hash kernel
+    if (b->on_demand && first != b->absorbed) return fail(PCS_ERR_ARG, "internal: on-demand groups must arrive in order");
     if (first == b->extended) b->extended += count;
     const bool whole = first == 0 && count == b->w;
     if (!whole && b->w + b->salt_w > 4 && b->extended < b->w) return absorb_columns(b, (b->extended / 8) * 8, false, st, true);
+    // the last group and the salt rows are absorbed together by batch_finish: one sponge chunk may cover both
+    if (b->on_demand && b->salt_w && b->extended == b->w)
+        PCS_CUDA(cudaMemcpyAsync(b->scratch + count * b->n, b->salts, b->salt_w * b->n * 8, cudaMemcpyDeviceToDevice, st));
     return PCS_OK;
 }
 
@@ -225,7 +237,7 @@ int batch_finish(pcs_batch* b, uint64_t* cap_out) {
         PCS_CUDA(cudaEventRecord(b->ev[4], st));
         rc = node_levels_dev(b->n, lg_n - b->cap_height, b->digests, b->cap, st);
     } else {
-        rc = build_tree_dev(b->lde, b->n, wt, lg_n, b->cap_height, b->digests, b->cap, st, b->ev[4]);
+        rc = build_tree_dev(b->on_demand ? b->scratch : b->lde, b->n, wt, lg_n, b->cap_height, b->digests, b->cap, st, b->ev[4]);
     }
     if (rc) return rc;
     PCS_CUDA(cudaEventRecord(b->ev[5], st));
@@ -703,6 +715,30 @@ static int d2h_pageable(void* dst, const void* src_dev, size_t bytes, cudaStream
     return PCS_OK;
 }
 
+// Row accessors of an on-demand batch: the leaf columns [0, width) on the cosets [c0, c1), recomputed group by group.
+// body(cols, stride, j0, j1) reads leaf c0 * d + l of column j0 + k at cols[k * stride + l]: polynomial columns are
+// regenerated from the kept coefficients into scratch ([LDE_GROUP][(c1 - c0) * d]); salt columns (width > w) are read where
+// the batch keeps them.
+template <class Body>
+static int for_each_group(const pcs_batch* b, size_t width, size_t c0, size_t c1, uint64_t* scratch, cudaStream_t st,
+                          Body body) {
+    const size_t d = (size_t)1 << b->lg_d, stride = (c1 - c0) * d;
+    NttPlan* plan = ntt_plan_get(b->lg_d, b->rate_bits, false, 7, st);
+    if (!plan) return fail(PCS_ERR_ALLOC, "twiddle table allocation failed");
+    for (size_t g0 = 0; g0 < b->w; g0 += LDE_GROUP) {
+        const size_t g1 = b->w - g0 < LDE_GROUP ? b->w : g0 + LDE_GROUP;
+        const uint64_t* src = b->coeffs + g0 * d;
+        if (c1 - c0 == ((size_t)1 << b->rate_bits))
+            PCS_CUDA(ntt_lde_cosets(plan, src, d, scratch, stride, g1 - g0, 0, b->rate_bits, st));
+        else
+            for (size_t c = c0; c < c1; c++)
+                PCS_CUDA(ntt_lde_cosets(plan, src, d, scratch + (c - c0) * d, stride, g1 - g0, (unsigned)c, 0, st));
+        if (int rc = body((const uint64_t*)scratch, stride, g0, g1)) return rc;
+    }
+    if (width > b->w) return body((const uint64_t*)b->salts + c0 * d, b->n, b->w, width);
+    return PCS_OK;
+}
+
 extern "C" {
 
 int pcs_coset_lde(const uint64_t* const* coeffs, size_t w, unsigned lg_d, unsigned rate_bits, uint64_t shift,
@@ -781,6 +817,7 @@ void pcs_batch_free(pcs_batch* b) {
     cudaStream_t st = g_ctx.stream;
     if (b->coeffs) cudaFreeAsync(b->coeffs, st);
     if (b->lde) cudaFreeAsync(b->lde, st);
+    if (b->salts) cudaFreeAsync(b->salts, st);
     if (b->digests) cudaFreeAsync(b->digests, st);
     if (b->cap) cudaFreeAsync(b->cap, st);
     if (b->sponge) cudaFreeAsync(b->sponge, st);
@@ -929,7 +966,7 @@ static int write_salts(pcs_batch* b, const uint64_t* const* salts, bool dev_ptrs
     const size_t n = b->n;
     for (size_t k = 0; k < b->salt_w; k++) {
         if (!salts[k]) return fail(PCS_ERR_ARG, "NULL salt pointer");
-        uint64_t* row = b->lde + (b->w + k) * n;
+        uint64_t* row = b->on_demand ? b->salts + k * n : b->lde + (b->w + k) * n;
         DevBuf tmp;
         PCS_CUDA(tmp.alloc(n * 8, st));
         PCS_CUDA(cudaMemcpyAsync(tmp.p, salts[k], n * 8, dev_ptrs ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
@@ -956,8 +993,13 @@ static int commit_common(const uint64_t* const* polys, bool from_values, size_t 
     if (w == 0 || !polys) return fail(PCS_ERR_ARG, "empty batch (oracle.rs:76 polynomials[0])");
     if (salt_w && !salts) return fail(PCS_ERR_ARG, "salts is NULL");
     if (!shard) lg_cosets = rate_bits;
+    const bool on_demand = flags & PCS_LDE_ON_DEMAND;
+    if (on_demand && shard) return fail(PCS_ERR_ARG, "PCS_LDE_ON_DEMAND is not supported by shard commits");
+    if (on_demand) flags |= PCS_KEEP_COEFFS;   // the rows are recomputed from the coefficients: copy device inputs
     BatchOwner b;
-    if (int rc = batch_begin(w, salt_w, lg_d, rate_bits, coset_first, lg_cosets, cap_height, BATCH_LDE, b)) return rc;
+    if (int rc = batch_begin(w, salt_w, lg_d, rate_bits, coset_first, lg_cosets, cap_height,
+                             on_demand ? BATCH_ON_DEMAND : BATCH_LDE, b))
+        return rc;
     cudaStream_t st = g_ctx.stream;
     NttPlan* iplan = from_values ? ntt_plan_get(lg_d, 0, true, 1, st) : nullptr;
     if (from_values && !iplan) return fail(PCS_ERR_ALLOC, "twiddle table allocation failed");
@@ -975,16 +1017,21 @@ static int commit_common(const uint64_t* const* polys, bool from_values, size_t 
 
     // ---- "IFFT" (oracle.rs:51-55) for polynomials [j0, j1): values (natural order) -> coefficients in b->coeffs ----
     // scratch for the bit-reversed intermediate = the TAIL of the LDE buffer (the last w*d elements): LDE rows already
-    // written for earlier polynomials end at j0*n <= wt*n - w*d + j0*d, so chunk-by-chunk processing never clobbers them
-    uint64_t* const ifft_scratch = b->lde + (wt * n - w * d);
+    // written for earlier polynomials end at j0*n <= wt*n - w*d + j0*d, so chunk-by-chunk processing never clobbers them.
+    // An on-demand batch has no LDE buffer: it transforms group by group through the group scratch (chunked inputs), or all
+    // at once through a [w][d] buffer released before the group scratch is allocated.
+    DevBuf ifft_buf, group_scratch;
+    if (on_demand && from_values && in.cb.empty()) PCS_CUDA(ifft_buf.alloc(w * d * 8, st));
+    uint64_t* const ifft_scratch = on_demand ? ifft_buf.u64() : b->lde + (wt * n - w * d);
     uint64_t* const coeffs = b->coeffs;
     const CoeffsOut mode = choose_coeffs_out(from_values, coeffs_out, w, d);
     if (mode == CoeffsOut::big_pinned && !g_ctx.d2h_stream)
         PCS_CUDA(cudaStreamCreateWithFlags(&g_ctx.d2h_stream, cudaStreamNonBlocking));
     size_t n_d2h = 0;
     auto ifft_range = [&](size_t j0, size_t j1) -> int {
-        PCS_CUDA(ntt_inverse_bitrev(iplan, src + j0 * d, d, ifft_scratch + j0 * d, d, j1 - j0, st));
-        PCS_CUDA(launch_bitrev_permute(ifft_scratch + j0 * d, d, coeffs + j0 * d, d, j1 - j0, lg_d, st, ntt_plan_scale(iplan)));
+        uint64_t* const scr = on_demand && !ifft_buf.p ? b->scratch : ifft_scratch + j0 * d;
+        PCS_CUDA(ntt_inverse_bitrev(iplan, src + j0 * d, d, scr, d, j1 - j0, st));
+        PCS_CUDA(launch_bitrev_permute(scr, d, coeffs + j0 * d, d, j1 - j0, lg_d, st, ntt_plan_scale(iplan)));
         if (mode == CoeffsOut::big_pinned) {
             if (g_ctx.d2h_ev.size() <= n_d2h) {
                 cudaEvent_t e;
@@ -1008,6 +1055,28 @@ static int commit_common(const uint64_t* const* polys, bool from_values, size_t 
     PCS_CUDA(cudaEventRecord(b->ev[1], st));
 
     // ---- "FFT + blinding" (oracle.rs:100-125), output already in leaf order ----
+    // On demand: polynomials [j0, j1) are extended and absorbed in groups of <= LDE_GROUP through one scratch of LDE_GROUP
+    // columns plus the salt rows, which follow the last group's columns (written first: they cannot be recomputed).
+    auto extend = [&](size_t j0, size_t j1, bool ifft) -> int {
+        if (!on_demand) {
+            if (ifft)
+                if (int rc = ifft_range(j0, j1)) return rc;
+            return batch_extend(b.get(), src + j0 * d, j0 == 0 && j1 == w ? in.dev.ptrs : nullptr, j0, j1 - j0);
+        }
+        for (size_t g0 = j0; g0 < j1; g0 += LDE_GROUP) {
+            const size_t g1 = j1 - g0 < LDE_GROUP ? j1 : g0 + LDE_GROUP;
+            if (ifft)
+                if (int rc = ifft_range(g0, g1)) return rc;
+            if (int rc = batch_extend(b.get(), src + g0 * d, nullptr, g0, g1 - g0)) return rc;
+        }
+        return PCS_OK;
+    };
+    if (on_demand) {
+        ifft_buf.release();
+        PCS_CUDA(group_scratch.alloc((LDE_GROUP + salt_w) * n * 8, st));
+        b->scratch = group_scratch.u64();
+        if (int rc = write_salts(b.get(), salts, dev_ptrs, shard, st)) return rc;
+    }
     for (size_t k = 0; k < n_chunks; k++) {
         const size_t j0 = in.cb[k], j1 = in.cb[k + 1];
         if (in.pageable) {
@@ -1015,17 +1084,17 @@ static int commit_common(const uint64_t* const* polys, bool from_values, size_t 
             PCS_CUDA(cudaEventRecord(g_ctx.chunk_ev[k], g_ctx.copy_stream));
         }
         PCS_CUDA(cudaStreamWaitEvent(st, g_ctx.chunk_ev[k], 0));
-        if (from_values)
-            if (int rc = ifft_range(j0, j1)) return rc;
-        if (int rc = batch_extend(b.get(), src + j0 * d, nullptr, j0, j1 - j0)) return rc;
+        if (int rc = extend(j0, j1, from_values)) return rc;
     }
     if (!n_chunks)
-        if (int rc = batch_extend(b.get(), src, in.dev.ptrs, 0, w)) return rc;
+        if (int rc = extend(0, w, false)) return rc;
     if (mode == CoeffsOut::small_pinned) PCS_CUDA(cudaMemcpyAsync(g_ctx.pin_out, coeffs, w * d * 8, cudaMemcpyDeviceToHost, st));
-    if (int rc = write_salts(b.get(), salts, dev_ptrs, shard, st)) return rc;
+    if (!on_demand)
+        if (int rc = write_salts(b.get(), salts, dev_ptrs, shard, st)) return rc;
 
     // ---- "transpose LDEs" (fused away), "build Merkle tree" (oracle.rs:83-89) ----
     if (int rc = batch_finish(b.get(), cap_out)) return rc;
+    b->scratch = nullptr;   // group_scratch goes back to the pool, in stream order, on return
     if (b->coeffs && !from_values && !(flags & PCS_KEEP_COEFFS)) {
         cudaFreeAsync(b->coeffs, st);
         b->coeffs = nullptr;
@@ -1167,12 +1236,29 @@ int pcs_batch_leaves(const pcs_batch* b, size_t first, size_t count, uint64_t* r
     cudaStream_t st = g_ctx.stream;
     size_t wt = b->w + b->salt_w;
     // transpose in slabs so that the staging buffer stays small
-    const size_t slab = (size_t)1 << 18;
-    DevBuf tmp;
+    size_t slab = (size_t)1 << 18;
+    const size_t d = (size_t)1 << b->lg_d;
+    // on demand, every slab regenerates the cosets it touches: slabs of up to a coset (and 1 GB) waste less of that work
+    while (b->on_demand && slab < d && 2 * slab * wt * 8 <= ((size_t)1 << 30)) slab *= 2;
+    DevBuf tmp, scratch;
     PCS_CUDA(tmp.alloc((count < slab ? count : slab) * wt * 8, st));
+    if (b->on_demand) {
+        size_t span = (slab + d - 1) / d + 1;   // cosets one slab can touch
+        if (span > ((size_t)1 << b->rate_bits)) span = (size_t)1 << b->rate_bits;
+        PCS_CUDA(scratch.alloc(LDE_GROUP * span * d * 8, st));
+    }
     for (size_t off = 0; off < count; off += slab) {
         size_t c = count - off < slab ? count - off : slab;
-        PCS_CUDA(launch_transpose(b->lde + first + off, b->n, tmp.u64(), wt, wt, c, st));
+        if (b->on_demand) {
+            const size_t f = first + off, c0 = f / d, c1 = (f + c - 1) / d + 1;
+            int rc = for_each_group(b, wt, c0, c1, scratch.u64(), st, [&](const uint64_t* cols, size_t stride, size_t j0, size_t j1) {
+                PCS_CUDA(launch_transpose(cols + (f - c0 * d), stride, tmp.u64() + j0, wt, j1 - j0, c, st));
+                return PCS_OK;
+            });
+            if (rc) return rc;
+        } else {
+            PCS_CUDA(launch_transpose(b->lde + first + off, b->n, tmp.u64(), wt, wt, c, st));
+        }
         int rc = d2h_pageable(rows + off * wt, tmp.p, c * wt * 8, st);
         if (rc) return rc;
     }
@@ -1190,8 +1276,35 @@ int pcs_batch_get_rows(const pcs_batch* b, const uint64_t* leaf_indices, size_t 
     DevBuf idx, o;
     PCS_CUDA(idx.alloc(n * 8, st));
     PCS_CUDA(o.alloc(n * wt * 8, st));
-    PCS_CUDA(cudaMemcpyAsync(idx.p, leaf_indices, n * 8, cudaMemcpyHostToDevice, st));
-    PCS_CUDA(launch_gather_rows(b->lde, b->n, (uint32_t)wt, idx.u64(), n, o.u64(), st));
+    std::vector<uint64_t> rel;   // on demand, many rows: leaf indices relative to the first coset regenerated
+    if (b->on_demand && n <= ROWS_EVAL_MAX) {
+        PCS_CUDA(cudaMemcpyAsync(idx.p, leaf_indices, n * 8, cudaMemcpyHostToDevice, st));
+        if (int rc = rows_eval(b, idx.u64(), n, o.u64(), st)) return rc;
+    } else if (b->on_demand) {
+        // regenerate the cosets [c0, c1) the leaves fall in, group by group, and gather from each group
+        const size_t d = (size_t)1 << b->lg_d;
+        size_t lo = leaf_indices[0], hi = leaf_indices[0];
+        for (size_t k = 1; k < n; k++) {
+            lo = leaf_indices[k] < lo ? leaf_indices[k] : lo;
+            hi = leaf_indices[k] > hi ? leaf_indices[k] : hi;
+        }
+        const size_t c0 = lo / d, c1 = hi / d + 1;
+        rel.assign(leaf_indices, leaf_indices + n);
+        for (auto& i : rel) i -= c0 * d;
+        PCS_CUDA(cudaMemcpyAsync(idx.p, rel.data(), n * 8, cudaMemcpyHostToDevice, st));
+        DevBuf scratch, g;
+        PCS_CUDA(scratch.alloc(LDE_GROUP * (c1 - c0) * d * 8, st));
+        PCS_CUDA(g.alloc(n * (LDE_GROUP > b->salt_w ? LDE_GROUP : b->salt_w) * 8, st));
+        int rc = for_each_group(b, wt, c0, c1, scratch.u64(), st, [&](const uint64_t* cols, size_t stride, size_t j0, size_t j1) {
+            PCS_CUDA(launch_gather_rows(cols, stride, (uint32_t)(j1 - j0), idx.u64(), n, g.u64(), st));
+            PCS_CUDA(cudaMemcpy2DAsync(o.u64() + j0, wt * 8, g.p, (j1 - j0) * 8, (j1 - j0) * 8, n, cudaMemcpyDeviceToDevice, st));
+            return PCS_OK;
+        });
+        if (rc) return rc;
+    } else {
+        PCS_CUDA(cudaMemcpyAsync(idx.p, leaf_indices, n * 8, cudaMemcpyHostToDevice, st));
+        PCS_CUDA(launch_gather_rows(b->lde, b->n, (uint32_t)wt, idx.u64(), n, o.u64(), st));
+    }
     PCS_CUDA(cudaMemcpyAsync(rows, o.p, n * wt * 8, cudaMemcpyDeviceToHost, st));
     PCS_CUDA(cudaStreamSynchronize(st));
     return PCS_OK;
@@ -1207,16 +1320,34 @@ int pcs_batch_lde_natural(const pcs_batch* b, size_t index_start, size_t step, s
     cudaStream_t st = g_ctx.stream;
     const size_t w = b->w;                       // salt columns are dropped (oracle.rs:131-132)
     const unsigned lg_n = b->lg_d + b->rate_bits;
-    // slabs of <= 256 MB: gather on the device, then stream to the caller's (usually pageable) rows
-    const size_t SLAB = (size_t)256 << 20;
+    // slabs of <= 256 MB: gather on the device, then stream to the caller's (usually pageable) rows.  On demand every slab
+    // regenerates the LDE, so slabs are 1 GB.
+    const size_t SLAB = (size_t)(b->on_demand ? 1024 : 256) << 20;
     size_t ch = SLAB / (w * 8);
     if (ch < 1) ch = 1;
     if (ch > count) ch = count;
-    DevBuf tmp;
+    DevBuf tmp, scratch, g;
     PCS_CUDA(tmp.alloc(ch * w * 8, st));
+    // natural points that are multiples of step = 2^s lie on the cosets [0, 2^(rate_bits - s)) of the leaf order
+    unsigned s = 0;
+    while (((size_t)1 << s) < step) s++;
+    const size_t d = (size_t)1 << b->lg_d, c1 = (size_t)1 << (s < b->rate_bits ? b->rate_bits - s : 0);
+    if (b->on_demand) {
+        PCS_CUDA(scratch.alloc(LDE_GROUP * c1 * d * 8, st));
+        PCS_CUDA(g.alloc(ch * LDE_GROUP * 8, st));
+    }
     for (size_t off = 0; off < count; off += ch) {
         const size_t c = count - off < ch ? count - off : ch;
-        PCS_CUDA(launch_lde_natural(b->lde, b->n, (uint32_t)w, lg_n, index_start + off, step, c, tmp.u64(), st));
+        if (b->on_demand) {
+            int rc = for_each_group(b, w, 0, c1, scratch.u64(), st, [&](const uint64_t* cols, size_t stride, size_t j0, size_t j1) {
+                PCS_CUDA(launch_lde_natural(cols, stride, (uint32_t)(j1 - j0), lg_n, index_start + off, step, c, g.u64(), st));
+                PCS_CUDA(cudaMemcpy2DAsync(tmp.u64() + j0, w * 8, g.p, (j1 - j0) * 8, (j1 - j0) * 8, c, cudaMemcpyDeviceToDevice, st));
+                return PCS_OK;
+            });
+            if (rc) return rc;
+        } else {
+            PCS_CUDA(launch_lde_natural(b->lde, b->n, (uint32_t)w, lg_n, index_start + off, step, c, tmp.u64(), st));
+        }
         int rc = d2h_pageable(rows + off * w, tmp.p, c * w * 8, st);
         if (rc) return rc;
     }
@@ -1280,7 +1411,7 @@ int pcs_batch_all_coeffs(const pcs_batch* b, uint64_t* coeffs) {
     return PCS_OK;
 }
 
-const uint64_t* pcs_batch_lde_dev(const pcs_batch* b) { return b ? b->lde : nullptr; }
+const uint64_t* pcs_batch_lde_dev(const pcs_batch* b) { return b ? b->lde : nullptr; }   // NULL for an on-demand batch
 const uint64_t* pcs_batch_coeffs_dev(const pcs_batch* b) { return b ? b->coeffs : nullptr; }
 const uint64_t* pcs_batch_digests_dev(const pcs_batch* b) { return b ? b->digests : nullptr; }
 const uint64_t* pcs_batch_cap_dev(const pcs_batch* b) { return b ? b->cap : nullptr; }

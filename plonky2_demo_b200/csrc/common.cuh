@@ -18,13 +18,16 @@ struct pcs_batch {
     size_t n = 0;          // N = d << rate_bits
     size_t n_digests = 0;  // 2 (N - 2^cap)
     uint64_t* coeffs = nullptr;   // [w][d] or null
-    uint64_t* lde = nullptr;      // [w + salt_w][N], leaf order
+    uint64_t* lde = nullptr;      // [w + salt_w][N], leaf order; null for an on-demand batch
+    uint64_t* salts = nullptr;    // on-demand batch: [salt_w][N], leaf order (blinding cannot be recomputed)
     uint64_t* digests = nullptr;  // [n_digests][4]
     uint64_t* cap = nullptr;      // [2^cap][4]
     cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     bool has_ifft = false;
     bool committed = false;  // all six events recorded
     bool rows_only = false;  // pcs_shard_begin_rows: LDE rows are supplied, not computed here
+    bool on_demand = false;  // PCS_LDE_ON_DEMAND: no LDE rows in HBM; accessors recompute them from `coeffs`
+    uint64_t* scratch = nullptr;     // on-demand commit in flight: [LDE_GROUP + salt_w][N] columns of the current group
     // streaming sponge (leaf hashing group by group while later groups are still in flight)
     uint64_t* sponge = nullptr;      // [12][n] parked states, allocated at the first partial absorb
     size_t absorbed = 0;             // columns [0, absorbed) are in the sponge states
@@ -86,7 +89,23 @@ enum BatchKind : unsigned {
     BATCH_LDE = 0,        // polynomials are extended by batch_extend (its twiddle tables are made here)
     BATCH_ROWS = 1,       // the caller writes the LDE rows itself
     BATCH_UNTIMED = 2,    // no phase events
+    BATCH_ON_DEMAND = 4,  // no LDE rows: salt rows only; batch_extend writes each group to b->scratch (PCS_LDE_ON_DEMAND)
 };
+// Columns per group of an on-demand batch: the commit extends and absorbs at most this many polynomials at a time, and the
+// row accessors recompute them group by group.  A multiple of the sponge rate (8).  16: the widest group that keeps the
+// 135 x 2^20 rate-3 commit under 4 GB of HBM (3.55 GB, 121.3 ms; 32: 4.62 GB, 120.9 ms; profiles/r03_lde_on_demand.md).
+#ifndef PCS_LDE_GROUP
+#define PCS_LDE_GROUP 16
+#endif
+constexpr size_t LDE_GROUP = PCS_LDE_GROUP;
+static_assert(LDE_GROUP % 8 == 0, "a group must end on the sponge rate");
+// pcs_batch_get_rows of an on-demand batch: up to this many rows are evaluated from the coefficients (rows_eval.cu), more are
+// gathered from the regenerated LDE.  At 135 x 2^20, rate 3: 128 rows take 19.5 ms evaluated and 21.1 ms regenerated, 512
+// rows 77.8 ms and 21.1 ms (profiles/r03_lde_on_demand.md)
+#ifndef PCS_ROWS_EVAL_MAX
+#define PCS_ROWS_EVAL_MAX 128
+#endif
+constexpr size_t ROWS_EVAL_MAX = PCS_ROWS_EVAL_MAX;
 int batch_begin(size_t w, size_t salt_w, unsigned lg_d, unsigned rate_bits, unsigned coset_first, unsigned lg_cosets,
                 unsigned cap_height, unsigned kind, BatchOwner& out);
 int batch_extend(pcs_batch* b, const uint64_t* src, const uint64_t* const* ptr_table, size_t first, size_t count);
@@ -105,6 +124,10 @@ struct CtxScope {
     explicit CtxScope(void* ctx);
     ~CtxScope();
 };
+
+// rows_eval.cu: rows [n][w + salt_w] of an on-demand batch at the leaves idx_dev[0 .. n) (device), evaluated from its kept
+// coefficients (salt columns gathered from its salt rows), into out_dev; asynchronous on st
+int rows_eval(const pcs_batch* b, const uint64_t* idx_dev, size_t n, uint64_t* out_dev, cudaStream_t st);
 
 // stream-ordered temporary buffer
 struct DevBuf {

@@ -280,6 +280,7 @@ static int multi_commit(const uint64_t* const* polys, bool from_values, size_t w
                         uint64_t* const* coeffs_out, uint64_t* cap_out, pcs_multi_batch** out) {
     if (!out) return fail(PCS_ERR_ARG, "out is NULL");
     *out = nullptr;
+    if (flags & PCS_LDE_ON_DEMAND) return fail(PCS_ERR_ARG, "PCS_LDE_ON_DEMAND is not supported by pcs_multi_* commits");
     if (!g_multi.init) return fail(PCS_ERR_NOT_INIT, "pcs_multi_init has not been called");
     if (w == 0 || !polys) return fail(PCS_ERR_ARG, "empty batch (oracle.rs:76 polynomials[0])");
     if (salt_w && !salts) return fail(PCS_ERR_ARG, "salts is NULL");

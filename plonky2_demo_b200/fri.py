@@ -180,19 +180,22 @@ class PolynomialBatch:
 
     # ---- constructors -------------------------------------------------------------------------
     @classmethod
-    def from_values(cls, values, rate_bits, blinding, cap_height, timing=None, fft_root_table=None, salts=None):
+    def from_values(cls, values, rate_bits, blinding, cap_height, timing=None, fft_root_table=None, salts=None,
+                    lde_on_demand=False):
         """oracle.rs:43-65.  `values`: list of PolynomialValues / arrays, or a [w][d] matrix.
         `timing` (a dict or None) receives the reference's TimingTree scope names with device times
-        in ms; `fft_root_table` is accepted and ignored (the engine owns its twiddles)."""
-        return cls._commit(values, True, rate_bits, blinding, cap_height, timing, salts)
+        in ms; `fft_root_table` is accepted and ignored (the engine owns its twiddles).
+        lde_on_demand: keep no LDE rows on the device (PCS_LDE_ON_DEMAND); the same commitment, and every accessor
+        recomputes the rows it returns from the kept coefficients."""
+        return cls._commit(values, True, rate_bits, blinding, cap_height, timing, salts, lde_on_demand=lde_on_demand)
 
     @classmethod
     def from_coeffs(cls, polynomials, rate_bits, blinding, cap_height, timing=None, fft_root_table=None, salts=None,
-                    keep_coeffs=False):
+                    keep_coeffs=False, lde_on_demand=False):
         """oracle.rs:68-98.  keep_coeffs: also keep `polynomials` on the device (PCS_KEEP_COEFFS), which the opening
         proof (fri_prover.prove_openings, eval_commitment) reads; the host copy the caller passed stays referenced
-        either way."""
-        return cls._commit(polynomials, False, rate_bits, blinding, cap_height, timing, salts, keep_coeffs)
+        either way.  lde_on_demand: as in from_values (implies keep_coeffs)."""
+        return cls._commit(polynomials, False, rate_bits, blinding, cap_height, timing, salts, keep_coeffs, lde_on_demand)
 
     @classmethod
     def _rows(cls, polys):
@@ -206,7 +209,7 @@ class PolynomialBatch:
         return rows
 
     @classmethod
-    def _commit(cls, polys, is_values, rate_bits, blinding, cap_height, timing, salts, keep_coeffs=False):
+    def _commit(cls, polys, is_values, rate_bits, blinding, cap_height, timing, salts, keep_coeffs=False, lde_on_demand=False):
         rows = cls._rows(polys)
         if len(rows) == 0:
             raise IndexError("index out of bounds: the len is 0 but the index is 0")  # oracle.rs:76 polynomials[0]
@@ -233,15 +236,16 @@ class PolynomialBatch:
         pp = _ffi.ptr_array(rows)
         sp = _ffi.ptr_array(salt_rows) if salt_rows else None
         L = _ffi.lib()
+        on_demand = _ffi.PCS_LDE_ON_DEMAND if lde_on_demand else 0
         if is_values:
             # the coefficients stay on the device with the batch (PCS_KEEP_COEFFS) and are fetched when
             # `polynomials` is first read, like the leaves
             rc = L.pcs_commit_from_values(pp, len(rows), lg_d, rate_bits, cap_height, sp, len(salt_rows),
-                                          _ffi.PCS_KEEP_COEFFS, None, _ffi.ptr(cap), C.byref(h))
+                                          _ffi.PCS_KEEP_COEFFS | on_demand, None, _ffi.ptr(cap), C.byref(h))
             self._coeffs_host = None
         else:
             rc = L.pcs_commit_from_coeffs(pp, len(rows), lg_d, rate_bits, cap_height, sp, len(salt_rows),
-                                          _ffi.PCS_KEEP_COEFFS if keep_coeffs else 0, _ffi.ptr(cap), C.byref(h))
+                                          (_ffi.PCS_KEEP_COEFFS if keep_coeffs else 0) | on_demand, _ffi.ptr(cap), C.byref(h))
             self._coeffs_host = rows
         if rc == _ffi_cap_height_code():
             raise ValueError(L.pcs_last_error().decode())  # merkle_tree.rs:136-142 message
