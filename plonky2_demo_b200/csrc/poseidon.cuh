@@ -19,10 +19,10 @@
 //    and verified independently in tests/golden/make_golden.py:mds_network_check.
 //    The next round's constant is folded into the network's additions (3-input IADD3), so
 //    constant_layer costs nothing; one 96-bit fold per lane brings the result back to 64 bits.
-//  * partial rounds use the dense network too, with the constants pushed through the linear layer
-//    (FAST_PARTIAL_FIRST_ROUND_CONSTANT once, then the scalar FAST_PARTIAL_ROUND_CONSTANTS[r] times
-//    the first MDS column); the sparse "fast" matrices of poseidon.rs:584-596 would need 23 full
-//    64x64 multiplies per round on the scarce pipe.
+//  * partial rounds use the same network's middle stage alone, with the state kept in its transform
+//    domain (crt_mid_half) and the scalar FAST_PARTIAL_ROUND_CONSTANTS[r] added to lane 0 after
+//    its S-box; the sparse "fast" matrices of poseidon.rs:584-596 would need 23 full 64x64
+//    multiplies per round on the scarce pipe.
 #pragma once
 #include "gl64.cuh"
 #include "poseidon_constants.cuh"
@@ -184,27 +184,32 @@ __device__ __forceinline__ void mds_layer_fp64(uint64_t (&s)[12], const uint64_t
 }
 
 // ------------------------------------------------------------------------------------------------
-// Partial rounds with lanes 1..11 RESIDENT in the FP64 network's domain.
+// Partial rounds in the FP64 network's TRANSFORM domain.
 //
-// In the 22 partial rounds only lane 0 passes the S-box, so only lane 0 has to exist as a 64-bit integer.
-// Lanes 1..11 stay as pairs of exact doubles (lo, hi), value = lo + hi * 2^32 (mod p), and go from one
-// round's network output straight into the next round's network input: no 96-bit fold, no int<->double
-// re-biasing for 11 of the 12 lanes.  Magnitudes grow by the MDS row sum (264 < 2^8.05) per round, and the
-// network's widest intermediate is bounded by 2^8.5 x its inputs (L1 norms checked symbolically in
-// tests/test_mds_network_bounds.py), so TWO rounds fit the 53-bit significand:
-//     normalised inputs < 2^33.01 -> round A outputs < 2^41.1 -> round B intermediates < 2^49.7, outputs < 2^49.2.
-// After round B the lanes are renormalised in 8 FP64 operations each (floor by the 2^52 trick with
-// round-down FMAs, 2^64 = 2^32 - 1 folded back, plus one multiple of p so that both halves stay positive):
-//     lo'' = lo - (l1-1) 2^32 - (h1-1)                 in [2^32 - 2^18, 2^33]
-//     hi'' = hi - (h1-1)(2^32 - 1) + (l1-1)            in [2^32 - 2, 2^33 + 2^19),      l1 = lo >> 32, h1 = hi >> 32
-//     lo'' + hi'' 2^32 = lo + hi 2^32 + p - h1 (2^64 - 2^32 + 1)  ==  lo + hi 2^32   (mod p).
-// The scalar round constant is added to lane 0 right after its S-box (poseidon.rs:584-596 does the same in
-// the "fast" form), so the network carries no per-lane constants in these rounds.
+// The network factors circ through the CRT of x^12 - 1 in three stages.  Per 32-bit half, the forward stage F maps
+// the 12 lanes to three groups of (A, B, P, Q):
+//     A_j = s_j + s_j+3 + s_j+6 + s_j+9,  B_j = s_j - s_j+3 + s_j+6 - s_j+9,  P_j = s_j - s_j+6,  Q_j = s_j+3 - s_j+9,
+// the middle stage G is the three twisted 3-point products (Ya, Yb, re/im) and the inverse stage H gives the lanes back,
+// with  F(circ s) = S G(F s),  S = diag(4, 4, 2, 2) on the (A, B, P, Q) blocks.  In the 22 partial rounds only lane 0
+// passes an S-box, so the state stays in this domain as U = F(circ part of the state), the diagonal term 8 x_prev
+// (MDS_MATRIX_DIAG[0] = 8) is kept aside, and a round is S G alone -- F and H drop out of the loop:
+//     ext = (A_0 + B_0 + 2 P_0) / 4           lane 0 of the circulant part (read off G's outputs before S: no division)
+//     s_0 = ext + 8 x_prev                    x_prev: previous round's S-box output + constant, 0 on entry
+//     x   = sbox(s_0) + PARTIAL_RC[r]
+//     U  <- S G(U + (x - ext) tau)            tau: + to A_0, B_0 and P_0
+// The 22nd round runs G and then the network's inverse stage H instead of S, which yields the lanes (+ 8 x e_0) directly.
+// The injected value is formed as (x - s_0) + 8 x_prev from the FOLDED s_0 (halves < 2^32), so it stays below 2^36 in
+// magnitude however large ext's double representation is.
+// The values are signed integers held exactly in doubles.  Per round A grows by the L1 row norm 256 of S G, B by 44,
+// P/Q by 50, so all 12 (lo, hi) pairs are renormalised every two rounds (renorm_d, valid for either sign), and lane 0
+// is folded with a positive multiple of p added (fold_signed_d).  tests/test_partial_crt.py proves every intermediate
+// an integer below 2^53 over the full signed input ranges and replays the whole permutation on integers.
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ double u32_as_double(uint32_t x) { return __hiloint2double(0x43300000, (int)x) - TWO52; }
+__device__ __forceinline__ double u32_biased(uint32_t x) { return __hiloint2double(0x43300000, (int)x); }   // 2^52 + x
 
-// y = circ-correlation(s) + 8*s0*e0 on exact doubles (no constants).  ZERO0: lane 0 is taken as 0 (its
-// contribution is added afterwards, see partial_round_d).
+// y = circ-correlation(s) + 8*s0*e0 on exact doubles (no constants), the whole network in the lane domain, as the pipe
+// benchmarks in tools/ run it.  ZERO0: lane 0 is taken as 0.
 template <bool ZERO0>
 __device__ __forceinline__ void mds_net_d(const double (&s)[12], double (&y)[12]) {
     double A[3], B[3], P[3], Q[3];
@@ -240,57 +245,104 @@ __device__ __forceinline__ void mds_net_d(const double (&s)[12], double (&y)[12]
     if (!ZERO0) y[0] = fma(s[0], 8.0, y[0]);  // MDS_MATRIX_DIAG[0] = 8
 }
 
-// (lo, hi) < 2^52, positive  ->  equivalent pair with both halves in [2^32 - 2^18, 2^33 + 2^19)
+// u = F(s) for one 32-bit half of the 12 lanes; u = (A_0..2, B_0..2, P_0..2, Q_0..2)
+__device__ __forceinline__ void crt_forward_d(const uint32_t (&s)[12], double (&u)[12]) {
+#pragma unroll
+    for (int j = 0; j < 3; j++) {
+        double v0 = u32_biased(s[j]), v3 = u32_biased(s[j + 3]), v6 = u32_biased(s[j + 6]), v9 = u32_biased(s[j + 9]);
+        double P = v0 - v6, Q = v3 - v9;
+        double a = fma(v6 - TWO52, 2.0, P);   // s_j + s_j+6
+        double b = fma(v9 - TWO52, 2.0, Q);   // s_j+3 + s_j+9
+        u[j] = a + b;
+        u[j + 3] = a - b;
+        u[j + 6] = P;
+        u[j + 9] = Q;
+    }
+}
+
+// G on one half: w = G(u + g tau) = (4 Ya, Yb, re, im), the A block already carrying its factor 4 of S (it folds into
+// the FMAs); the other blocks get theirs in crt_scale_half, or go through H unscaled in the last round (crt_lanes_half).
+__device__ __forceinline__ void crt_mid_half(const double (&u)[12], double g, double (&w)[12]) {
+    const double A0 = u[0] + g, A1 = u[1], A2 = u[2];
+    const double B0 = u[3] + g, B1 = u[4], B2 = u[5];
+    const double P0 = u[6] + g, P1 = u[7], P2 = u[8];
+    const double Q0 = u[9], Q1 = u[10], Q2 = u[11];
+    const double T = ((A1 + A2) + A0) * 64.0;              // 4 * 16 * (A_0 + A_1 + A_2)
+    w[0] = fma(A2, 64.0, T);
+    w[1] = fma(A0, 64.0, T);
+    w[2] = fma(A1, 64.0, T);
+    w[3] = fma(B1, -2.0, fma(B2, 8.0, -B0));
+    w[4] = fma(B2, -2.0, fma(B0, -8.0, -B1));
+    w[5] = fma(B1, -8.0, fma(B0, 2.0, -B2));
+    w[6] = fma(Q2, 4.0, fma(Q1, -16.0, fma(P0, 2.0, -Q0) + P1) + P2);
+    w[7] = fma(Q2, -16.0, fma(P1, 2.0, fma(P0, -4.0, Q0) - Q1) + P2);
+    w[8] = fma(P2, 2.0, fma(P1, -4.0, fma(P0, 16.0, Q0) + Q1) - Q2);
+    w[9] = fma(P2, -4.0, fma(P1, 16.0, fma(Q0, 2.0, P0) + Q1) + Q2);
+    w[10] = fma(P2, 16.0, fma(Q1, 2.0, fma(Q0, -4.0, -P0) + P1) + Q2);
+    w[11] = fma(Q2, 2.0, fma(Q1, -4.0, fma(Q0, 16.0, -P0) - P1) + P2);
+}
+
+// u <- S G = the rest of S applied to w.  Returns ext = (A_0 + B_0 + 2 P_0) / 4 of the new u, formed before the scaling.
+__device__ __forceinline__ double crt_scale_half(const double (&w)[12], double (&u)[12]) {
+#pragma unroll
+    for (int j = 0; j < 3; j++) {
+        u[j] = w[j];
+        u[j + 3] = w[j + 3] * 4.0;
+        u[j + 6] = w[j + 6] * 2.0;
+        u[j + 9] = w[j + 9] * 2.0;
+    }
+    return fma(w[0], 0.25, w[3] + w[6]);
+}
+
+// The last round's lanes: y = H w (the network's own inverse stage: circ part of the state) + bias + rcd, with rcd the
+// biased constants 2^52 + half of the next full round (stride 2).
+__device__ __forceinline__ void crt_lanes_half(const double (&w)[12], double bias, const double* __restrict__ rcd,
+                                               double (&y)[12]) {
+#pragma unroll
+    for (int j = 0; j < 3; j++) {
+        double e1 = fma(w[j], 0.25, w[j + 3] + bias), e2 = fma(w[j], 0.25, bias - w[j + 3]);   // Ya +- Yb
+        y[j] = (e1 + w[j + 6]) + rcd[2 * j];
+        y[j + 6] = (e1 - w[j + 6]) + rcd[2 * (j + 6)];
+        y[j + 3] = (e2 + w[j + 9]) + rcd[2 * (j + 3)];
+        y[j + 9] = (e2 - w[j + 9]) + rcd[2 * (j + 9)];
+    }
+}
+
+// (lo, hi), |lo|, |hi| < 2^51  ->  equivalent pair with both halves in [-2^20, 2^32 + 2^20]:
+//   l1 = floor(lo / 2^32), h1 = floor(hi / 2^32) (round-down FMA onto 1.5 * 2^52, where doubles are spaced 1 apart for
+//   either sign of the quotient),  lo' = lo - l1 2^32 - h1,  hi' = hi - h1 (2^32 - 1) + l1,  lo' + hi' 2^32 = lo + hi 2^32 - h1 p.
 __device__ __forceinline__ void renorm_d(double& lo, double& hi) {
-    const double M1 = TWO52 + 1.0, INV32 = 1.0 / 4294967296.0;
-    double l1m = __fma_rd(lo, INV32, TWO52) - M1;   // (lo >> 32) - 1
-    double h1m = __fma_rd(hi, INV32, TWO52) - M1;   // (hi >> 32) - 1
-    double lo2 = fma(l1m, -4294967296.0, lo) - h1m;
-    double hi2 = fma(h1m, -4294967295.0, hi) + l1m;
+    const double C = 6755399441055744.0, INV32 = 1.0 / 4294967296.0;
+    double l1 = __fma_rd(lo, INV32, C) - C;
+    double h1 = __fma_rd(hi, INV32, C) - C;
+    double lo2 = fma(l1, -4294967296.0, lo) - h1;
+    double hi2 = fma(h1, -4294967295.0, hi) + l1;
     lo = lo2;
     hi = hi2;
 }
 
-// lane value (lo + hi 2^32, both < 2^52 and >= 0) as a loose u64
-__device__ __forceinline__ uint64_t fold_d(double lo, double hi) {
-    double bl = lo + TWO52, bh = hi + TWO52;
+// (BIAS_LO, BIAS_HI) = 2^19 p as lo + hi 2^32: added to a signed pair with |lo|, |hi| < 2^51 - 2^20 it makes both halves
+// non-negative and below 2^52, the range fold_halves_biased reads from the bit pattern of 2^52 + half.
+constexpr double BIAS_LO = 2251799813685248.0 + 524288.0;    // 2^51 + 2^19
+constexpr double BIAS_HI = 2251799813685248.0 - 1048576.0;   // 2^51 - 2^20
+
+// signed lane value lo + hi 2^32 as a loose u64
+__device__ __forceinline__ uint64_t fold_signed_d(double lo, double hi) {
+    double bl = lo + (TWO52 + BIAS_LO), bh = hi + (TWO52 + BIAS_HI);
     return gl::fold_halves_biased((uint32_t)__double2loint(bl), (uint32_t)__double2hiint(bl),
                                   (uint32_t)__double2loint(bh), (uint32_t)__double2hiint(bh));
 }
 
-// One partial round: lane 0 = x0 (integer), lanes 1..11 = (dl, dh); (dl, dh) receive M * state.
-// M s = M (0, s1..s11) + x0' * M[:,0]: the bulk network does not depend on this round's S-box, so the FP64
-// work of lanes 1..11 and the (serial, latency-bound) integer S-box chain of lane 0 are independent
-// instruction streams that the scheduler interleaves; lane 0 then enters through 12 FMAs per half.
-#ifndef PCS_PARTIAL_SPLIT
-#define PCS_PARTIAL_SPLIT 0   // measured: 203.6 vs 199.2 clk per permutation with the split (the extra 24 FMAs cost more than the ILP gains)
-#endif
-__device__ __forceinline__ void partial_round_d(uint64_t& x0, double (&dl)[12], double (&dh)[12], uint64_t rc) {
-    double yl[12], yh[12];
-#if PCS_PARTIAL_SPLIT
-    mds_net_d<true>(dl, yl);
-    mds_net_d<true>(dh, yh);
-    x0 = gl::add_lc_p(sbox7(x0), rc);
-    const double al = u32_as_double((uint32_t)x0), ah = u32_as_double((uint32_t)(x0 >> 32));
-    // M[i][0] = MDS_MATRIX_CIRC[(12 - i) % 12] (+ MDS_MATRIX_DIAG[0] for i = 0)   poseidon_goldilocks.rs:24-25
-    constexpr double COL0[12] = {25.0, 20.0, 34.0, 18.0, 39.0, 13.0, 13.0, 28.0, 2.0, 16.0, 41.0, 15.0};
-#pragma unroll
-    for (int i = 0; i < 12; i++) {
-        dl[i] = fma(al, COL0[i], yl[i]);
-        dh[i] = fma(ah, COL0[i], yh[i]);
-    }
-#else
-    x0 = gl::add_lc_p(sbox7(x0), rc);
-    dl[0] = u32_as_double((uint32_t)x0);
-    dh[0] = u32_as_double((uint32_t)(x0 >> 32));
-    mds_net_d<false>(dl, yl);
-    mds_net_d<false>(dh, yh);
-#pragma unroll
-    for (int i = 0; i < 12; i++) {
-        dl[i] = yl[i];
-        dh[i] = yh[i];
-    }
-#endif
+// Lane 0 of one partial round: s_0 = ext + 8 x_prev through its S-box; (gl, gh) = x - ext as halves, to be injected;
+// (el, eh): ext of the current U, (xl, xh): x_prev, becomes x; rc = PARTIAL_RC[r].
+__device__ __forceinline__ void lane0_crt(double el, double eh, double& xl, double& xh, uint64_t rc, double& gl, double& gh) {
+    const uint64_t s0 = fold_signed_d(fma(xl, 8.0, el), fma(xh, 8.0, eh));
+    const uint64_t x = gl::add_lc_p(sbox7(s0), rc);
+    // x - ext = (x - s_0) + 8 x_prev
+    gl = fma(xl, 8.0, u32_biased((uint32_t)x) - u32_biased((uint32_t)s0));
+    gh = fma(xh, 8.0, u32_biased((uint32_t)(x >> 32)) - u32_biased((uint32_t)(s0 >> 32)));
+    xl = u32_as_double((uint32_t)x);
+    xh = u32_as_double((uint32_t)(x >> 32));
 }
 
 #ifndef PCS_PARTIAL_FP64
@@ -338,36 +390,55 @@ __device__ __forceinline__ void poseidon12(uint64_t (&s)[12]) {
 #pragma unroll
     for (int i = 0; i < 12; i++) s[i] = gl::add_lc_p(s[i], RC[i]);
 #if PCS_PARTIAL_FP64 && PCS_MDS_FP64
-    // rounds 0..3 (full), 4..25 (partial, FP64-resident lanes), 26..29 (full): the two full-round groups share
+    // rounds 0..3 (full), 4..25 (partial, FP64 transform domain), 26..29 (full): the two full-round groups share
     // ONE loop body (phase 0 and phase 1) so that the code stays small enough for the instruction cache
 #pragma unroll 1
     for (int phase = 0; phase < 2; phase++) {
 #pragma unroll 1
         for (int r = 0; r < 4; r++) full_round(s, 26 * phase + r);
         if (phase == 0) {
-            uint64_t x0 = s[0];
-            double dl[12], dh[12];
+            // rounds 4..25 in the transform domain (see crt_mid_half); entry: U = F(s), ext = s_0, x_prev = 0
+            double ul[12], uh[12];
+            {
+                uint32_t lo[12], hi[12];
 #pragma unroll
-            for (int i = 1; i < 12; i++) {
-                dl[i] = u32_as_double((uint32_t)s[i]);
-                dh[i] = u32_as_double((uint32_t)(s[i] >> 32));
+                for (int i = 0; i < 12; i++) {
+                    lo[i] = (uint32_t)s[i];
+                    hi[i] = (uint32_t)(s[i] >> 32);
+                }
+                crt_forward_d(lo, ul);
+                crt_forward_d(hi, uh);
             }
+            double el = u32_as_double((uint32_t)s[0]), eh = u32_as_double((uint32_t)(s[0] >> 32));
+            double xl = 0.0, xh = 0.0;
+            // the 22nd round runs G then H (the lanes, + RC[26] as 2^52 + halves of ROUND_ADD[25]) instead of S G
+            const double* rcd = reinterpret_cast<const double*>(&ROUND_ADD_D[24 * 25]);
 #pragma unroll 1
             for (int k = 0; k < 11; k++) {
-                partial_round_d(x0, dl, dh, PARTIAL_RC[2 * k]);        // inputs normalised
-                x0 = fold_d(dl[0], dh[0]);
-                partial_round_d(x0, dl, dh, PARTIAL_RC[2 * k + 1]);    // inputs up to 2^41
+                double gl, gh, wl[12], wh[12];
+                lane0_crt(el, eh, xl, xh, PARTIAL_RC[2 * k], gl, gh);
+                crt_mid_half(ul, gl, wl);
+                crt_mid_half(uh, gh, wh);
+                el = crt_scale_half(wl, ul);
+                eh = crt_scale_half(wh, uh);
+                lane0_crt(el, eh, xl, xh, PARTIAL_RC[2 * k + 1], gl, gh);
+                crt_mid_half(ul, gl, wl);
+                crt_mid_half(uh, gh, wh);
                 if (k < 10) {
-                    x0 = fold_d(dl[0], dh[0]);
+                    el = crt_scale_half(wl, ul);
+                    eh = crt_scale_half(wh, uh);
 #pragma unroll
-                    for (int i = 1; i < 12; i++) renorm_d(dl[i], dh[i]);
+                    for (int i = 0; i < 12; i++) renorm_d(ul[i], uh[i]);
+                } else {
+                    crt_lanes_half(wl, BIAS_LO, rcd, ul);
+                    crt_lanes_half(wh, BIAS_HI, rcd + 1, uh);
+                    ul[0] = fma(xl, 8.0, ul[0]);               // + 8 x_last (MDS_MATRIX_DIAG[0])
+                    uh[0] = fma(xh, 8.0, uh[0]);
                 }
             }
-            // leave the FP64 domain: + RC[26] (the next full round's constants), all lanes back to integers
-            const double* rcd = reinterpret_cast<const double*>(&ROUND_ADD_D[24 * 25]);  // 2^52 + halves of RC[26..]
 #pragma unroll
             for (int i = 0; i < 12; i++) {
-                double bl = dl[i] + rcd[2 * i], bh = dh[i] + rcd[2 * i + 1];
+                const double bl = ul[i], bh = uh[i];
                 s[i] = gl::fold_halves_biased((uint32_t)__double2loint(bl), (uint32_t)__double2hiint(bl),
                                               (uint32_t)__double2loint(bh), (uint32_t)__double2hiint(bh));
             }
