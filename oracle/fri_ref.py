@@ -168,7 +168,11 @@ def final_poly(oracle_coeffs, batches, alpha):
     d = oracle_coeffs[0].shape[1]
     fin = np.zeros((d, 2), dtype=np.uint64)
     for point, polys in batches:
-        rows = np.stack([oracle_coeffs[o][j] for o, j in polys])
+        o0, j0 = polys[0]
+        if all(o == o0 and j == j0 + k for k, (o, j) in enumerate(polys)):
+            rows = oracle_coeffs[o0][j0:j0 + len(polys)]     # a run of one oracle: a view, not a copy (18 GB at 135 x 2^24)
+        else:
+            rows = np.stack([oracle_coeffs[o][j] for o, j in polys])
         comp = reduce_polys_base(rows, alpha)
         quotient = ext_divide_by_linear(comp, point)
         fin = ext_scale_add(fin, ext_pow(alpha, len(polys)), quotient)
@@ -287,7 +291,9 @@ def fri_proof_of_work(challenger, proof_of_work_bits, limit=1 << 24):
 def prove_openings(oracles, batches, challenger, rate_bits, cap_height, reduction_arity_bits, proof_of_work_bits,
                    num_query_rounds):
     """oracle.rs:162-219 + prover.rs:20-67.  oracles: list of dicts (coeffs [w][d], leaves [N][w+s], digests, cap,
-    cap_height) as the commit oracle returns them.  Returns the FriProof as a dict."""
+    cap_height) as the commit oracle returns them.  An oracle whose leaves are too large to hold may give callables
+    instead: rows(i) -> leaf i, path(i) -> its Merkle path ([depth][4]); its leaves / digests are then not read.
+    Returns the FriProof as a dict."""
     alpha = challenger.get_extension_challenge()
     fin = final_poly([o["coeffs"] for o in oracles], batches, alpha)
     d = fin.shape[0]
@@ -306,6 +312,9 @@ def prove_openings(oracles, batches, challenger, rate_bits, cap_height, reductio
         indices.append(x_index)
         initial = []
         for o in oracles:
+            if "rows" in o:
+                initial.append((np.asarray(o["rows"](x_index), dtype=np.uint64), np.asarray(o["path"](x_index))))
+                continue
             lv = np.asarray(o["leaves"])
             initial.append((lv[x_index].copy(), merkle_prove(o["digests"], lv.shape[0], o["cap_height"], x_index)))
         steps = []

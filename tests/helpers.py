@@ -42,3 +42,36 @@ def brev(i, bits):
 def canon(a):
     a = np.asarray(a, dtype=np.uint64)
     return np.where(a >= np.uint64(P), a - np.uint64(P), a)
+
+
+def assert_same_proof(got, want):
+    """A device FriProof against fri_ref.prove_openings' dict, field by field."""
+    assert len(got.commit_phase_merkle_caps) == len(want["commit_phase_merkle_caps"])
+    for c, wc in zip(got.commit_phase_merkle_caps, want["commit_phase_merkle_caps"]):
+        assert np.array_equal(c.hashes, wc)
+    assert np.array_equal(got.final_poly, want["final_poly"])
+    assert got.pow_witness == want["pow_witness"]
+    assert got.fri_query_indices == want["_indices"]
+    assert len(got.query_round_proofs) == len(want["query_round_proofs"])
+    for r, wr in zip(got.query_round_proofs, want["query_round_proofs"]):
+        for (ev, mp), (wev, wmp) in zip(r.initial_trees_proof.evals_proofs, wr["initial_trees_proof"]):
+            assert np.array_equal(ev, wev)
+            assert np.array_equal(np.asarray(mp.siblings).reshape(-1, 4), wmp)
+        assert len(r.steps) == len(wr["steps"])
+        for s, ws in zip(r.steps, wr["steps"]):
+            assert np.array_equal(s.evals, ws["evals"])
+            assert np.array_equal(np.asarray(s.merkle_proof.siblings).reshape(-1, 4), ws["merkle_proof"])
+
+
+def as_oracle_proof(proof):
+    """A device FriProof in the dict form fri_ref.verify_fri_proof reads."""
+    return {
+        "commit_phase_merkle_caps": [c.hashes for c in proof.commit_phase_merkle_caps],
+        "final_poly": proof.final_poly,
+        "pow_witness": proof.pow_witness,
+        "query_round_proofs": [
+            {"initial_trees_proof": [(ev, np.asarray(mp.siblings).reshape(-1, 4)) for ev, mp in r.initial_trees_proof.evals_proofs],
+             "steps": [{"evals": s.evals, "merkle_proof": np.asarray(s.merkle_proof.siblings).reshape(-1, 4)} for s in r.steps]}
+            for r in proof.query_round_proofs
+        ],
+    }

@@ -338,3 +338,29 @@ def test_fri_roundtrip_random_shapes_and_more_tampering():
     bad["pow_witness"] = proof["pow_witness"] + 1
     with pytest.raises(AssertionError):
         fr.verify_fri_proof(batches, openings, ch.clone(), [o["cap"] for o in oracles], bad, *args)
+
+
+def test_prove_openings_with_row_and_path_callables():
+    """An oracle entry may give rows(i) / path(i) instead of leaves / digests (the benchmark-size tests hold no leaves):
+    rows by direct evaluation at 7 w_N^brev(i), paths from the digests, give the same proof as the leaves."""
+    lg_d, rate_bits, cap_height, arities, widths = 6, 3, 2, [2, 2], [3, 5, 4, 2]
+    oracles, batches = make_instance(lg_d, rate_bits, cap_height, widths, seed=7)
+    openings = openings_of(oracles, batches)
+    ch = seeded_challenger(oracles, openings)
+    want = fr.prove_openings(oracles, batches, ch.clone(), rate_bits, cap_height, arities, 4, 5)
+    lg_n = lg_d + rate_bits
+    w_n = fr.primitive_root_of_unity(lg_n)
+
+    def lean(o):
+        def rows(i):
+            x = fr.COSET_SHIFT * pow(w_n, fr.reverse_bits(i, lg_n), P) % P
+            return fr.eval_base_polys_ext(o["coeffs"], (x, 0))[:, 0]
+
+        return {"coeffs": o["coeffs"], "cap_height": cap_height, "rows": rows,
+                "path": lambda i: oracle.merkle_prove(o["digests"], 1 << lg_n, cap_height, i)}
+
+    got = fr.prove_openings([lean(o) for o in oracles], batches, ch.clone(), rate_bits, cap_height, arities, 4, 5)
+    assert got["_indices"] == want["_indices"]
+    for r, wr in zip(got["query_round_proofs"], want["query_round_proofs"]):
+        for (ev, mp), (wev, wmp) in zip(r["initial_trees_proof"], wr["initial_trees_proof"]):
+            assert np.array_equal(ev, wev) and np.array_equal(mp, wmp)

@@ -9,7 +9,7 @@ import pytest
 
 import oracle
 from oracle import fri_ref as fr
-from helpers import P, seeded_polys, splitmix64_stream
+from helpers import P, as_oracle_proof, assert_same_proof, seeded_polys, splitmix64_stream
 
 pytestmark = pytest.mark.gpu
 
@@ -41,7 +41,8 @@ def with_noncanonical(a, rng):
 # ---------------------------------------------------------------------------------------------
 # eval_commitment (proof.rs:316-322)
 # ---------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("w,lg_d", [(1, 0), (3, 1), (5, 7), (4, 12), (7, 13), (135, 15), (2, 17)])
+@pytest.mark.parametrize("w,lg_d", [(1, 0), (3, 1), (5, 7), (4, 12), (7, 13), (135, 15), (2, 17),
+                                    (3, 20), (1, 24)])   # 64 and 1024 chunks per polynomial (bench.py: 2^20; configs[4]: 2^24)
 def test_eval_commitment(pcs, w, lg_d):
     from plonky2_demo_b200.fri_prover import eval_commitment
 
@@ -74,7 +75,10 @@ def test_eval_commitment_needs_coefficients(pcs):
 # ---------------------------------------------------------------------------------------------
 # extension polynomials: round trip, LDE, fold
 # ---------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("lg_d,rate_bits", [(0, 0), (0, 3), (1, 1), (5, 3), (10, 2), (11, 3), (15, 3), (16, 1)])
+@pytest.mark.parametrize("lg_d,rate_bits", [(0, 0), (0, 3), (1, 1), (5, 3), (10, 2), (11, 3), (15, 3), (16, 1),
+                                            # the benchmark proof's final-poly LDE (plan [10, 10] at rate 3), then 2^24 outputs
+                                            # at rate 1 and 0 (3-pass plans)
+                                            (20, 3), (23, 1), (24, 0)])
 def test_ext_poly_lde(pcs, lg_d, rate_bits):
     from plonky2_demo_b200.fri_prover import ExtensionPolynomial
 
@@ -89,7 +93,8 @@ def test_ext_poly_lde(pcs, lg_d, rate_bits):
     p.free()
 
 
-@pytest.mark.parametrize("lg_d,arity_bits", [(4, 4), (4, 1), (8, 3), (12, 4), (15, 4), (13, 0)])
+@pytest.mark.parametrize("lg_d,arity_bits", [(4, 4), (4, 1), (8, 3), (12, 4), (15, 4), (13, 0),
+                                             (16, 4), (20, 4), (24, 4)])   # outputs past 2^15: the benchmark's folds
 def test_fri_fold(pcs, lg_d, arity_bits):
     from plonky2_demo_b200.fri_prover import ExtensionPolynomial
 
@@ -124,6 +129,7 @@ def test_fold_rejects_ragged_length(pcs):
 @pytest.mark.parametrize("lg_d,rate_bits,arity_bits,cap_height,shift", [
     (4, 3, 4, 0, 7), (4, 3, 4, 3, 7), (6, 1, 2, 1, 49), (10, 3, 4, 4, 7), (12, 3, 4, 4, pow(7, 16, P)), (3, 2, 1, 4, 7),
     (15, 3, 4, 4, 7),
+    (20, 3, 4, 4, 7), (16, 3, 4, 4, pow(7, 16, P)),    # the benchmark proof's first two trees: 2^19 and 2^15 leaves of 32
 ])
 def test_fri_commit_layer(pcs, lg_d, rate_bits, arity_bits, cap_height, shift):
     from plonky2_demo_b200.fri_prover import ExtensionPolynomial
@@ -212,6 +218,43 @@ def test_fri_final_poly(pcs, lg_d, widths):
         b.free()
 
 
+@pytest.mark.parametrize("lg_d", range(25))
+def test_fri_final_poly_single_polynomial(pcs, lg_d):
+    """One polynomial opened at two points, through pcs_fri_final_poly_dev on a torch tensor (no commit), for every degree
+    up to configs[4]'s 2^24: every recursion depth of the divide_by_linear suffix scan (segments of 16), including a level
+    of exactly 16 coefficients and levels of one or two segments.  Coefficients include 2^64 - 1, p and p + 1."""
+    import ctypes as C
+
+    import torch
+
+    from plonky2_demo_b200 import _ffi
+    from plonky2_demo_b200.fri_prover import ExtensionPolynomial, _ext_arg, _poly_ptr_array
+
+    d = 1 << lg_d
+    c = splitmix64_stream(0xF1A1 + lg_d, d)
+    edge = np.array([(1 << 64) - 1, P, P + 1], dtype=np.uint64)
+    c[: min(3, d)] = edge[: min(3, d)]
+    c[-min(3, d):] = edge[::-1][-min(3, d):]
+    c[d // 2::5] = edge[np.arange(c[d // 2::5].size) % 3]
+    rng = random.Random(lg_d)
+    batches = [(rand_ext(rng), [(0, 0)]), (rand_ext(rng), [(0, 0)])]
+    alpha = rand_ext(rng)
+    want = fr.final_poly([(c % np.uint64(P))[None, :]], batches, alpha)
+    t = torch.from_numpy(c.view(np.int64)).cuda()
+    torch.cuda.synchronize()
+    pts =np.array([pt for pt, _ in batches], dtype=np.uint64)
+    h = C.c_void_p()
+    _ffi.check(_ffi.lib().pcs_fri_final_poly_dev(_poly_ptr_array([t.data_ptr()] * 2), lg_d, 2, _ffi.ptr(pts),
+                                                 (C.c_size_t * 2)(1, 1), _ext_arg(alpha), C.byref(h)))
+    p = ExtensionPolynomial(h)
+    try:
+        got = p.coeffs
+    finally:
+        p.free()
+    bad = np.flatnonzero((got != want).any(axis=1))
+    assert bad.size == 0, f"{bad.size} of {d} coefficients differ, the first at {bad[:8].tolist()}"
+
+
 def test_fri_final_poly_errors(pcs):
     from plonky2_demo_b200.fri_prover import FriBatchInfo, FriInstanceInfo, FriOracleInfo, FriPolynomialInfo, final_poly
 
@@ -231,36 +274,6 @@ def test_fri_final_poly_errors(pcs):
         final_poly(FriInstanceInfo(info, [FriBatchInfo((1, 1), [])]), [a], (3, 4))
     for x in (a, b, nokeep):
         x.free()
-
-
-def _assert_same_proof(got, want):
-    assert len(got.commit_phase_merkle_caps) == len(want["commit_phase_merkle_caps"])
-    for c, wc in zip(got.commit_phase_merkle_caps, want["commit_phase_merkle_caps"]):
-        assert np.array_equal(c.hashes, wc)
-    assert np.array_equal(got.final_poly, want["final_poly"])
-    assert got.pow_witness == want["pow_witness"]
-    assert got.fri_query_indices == want["_indices"]
-    for r, wr in zip(got.query_round_proofs, want["query_round_proofs"]):
-        for (ev, mp), (wev, wmp) in zip(r.initial_trees_proof.evals_proofs, wr["initial_trees_proof"]):
-            assert np.array_equal(ev, wev)
-            assert np.array_equal(np.asarray(mp.siblings).reshape(-1, 4), wmp)
-        assert len(r.steps) == len(wr["steps"])
-        for s, ws in zip(r.steps, wr["steps"]):
-            assert np.array_equal(s.evals, ws["evals"])
-            assert np.array_equal(np.asarray(s.merkle_proof.siblings).reshape(-1, 4), ws["merkle_proof"])
-
-
-def _as_oracle_proof(proof):
-    return {
-        "commit_phase_merkle_caps": [c.hashes for c in proof.commit_phase_merkle_caps],
-        "final_poly": proof.final_poly,
-        "pow_witness": proof.pow_witness,
-        "query_round_proofs": [
-            {"initial_trees_proof": [(ev, np.asarray(mp.siblings).reshape(-1, 4)) for ev, mp in r.initial_trees_proof.evals_proofs],
-             "steps": [{"evals": s.evals, "merkle_proof": np.asarray(s.merkle_proof.siblings).reshape(-1, 4)} for s in r.steps]}
-            for r in proof.query_round_proofs
-        ],
-    }
 
 
 @pytest.mark.parametrize("lg_d,rate_bits,cap_height,arities,widths,pow_bits,n_queries,from_values", [
@@ -293,11 +306,11 @@ def test_prove_openings_matches_oracle_and_verifies(pcs, lg_d, rate_bits, cap_he
     verifier_ch = och.clone()
     got = prove_openings(inst, gpu, ch, params)
     want = fr.prove_openings(cpu, batches, och, rate_bits, cap_height, arities, pow_bits, n_queries)
-    _assert_same_proof(got, want)
+    assert_same_proof(got, want)
     # both transcripts end in the same state
     assert ch.get_challenge() == och.get_challenge()
     # and the restated verifier accepts the GPU proof
-    assert fr.verify_fri_proof(batches, openings, verifier_ch, [o["cap"] for o in cpu], _as_oracle_proof(got), rate_bits,
+    assert fr.verify_fri_proof(batches, openings, verifier_ch, [o["cap"] for o in cpu], as_oracle_proof(got), rate_bits,
                                cap_height, arities, pow_bits, n_queries, lg_d)
     for b in gpu:
         b.free()
@@ -329,8 +342,8 @@ def test_prove_openings_m64_demo_shape(pcs):
     got = prove_openings(inst, gpu, ch, params)
     want = fr.prove_openings(cpu, batches, och, cfg.rate_bits, cfg.cap_height, params.reduction_arity_bits,
                              cfg.proof_of_work_bits, cfg.num_query_rounds)
-    _assert_same_proof(got, want)
-    assert fr.verify_fri_proof(batches, openings, verifier_ch, [o["cap"] for o in cpu], _as_oracle_proof(got),
+    assert_same_proof(got, want)
+    assert fr.verify_fri_proof(batches, openings, verifier_ch, [o["cap"] for o in cpu], as_oracle_proof(got),
                                cfg.rate_bits, cfg.cap_height, params.reduction_arity_bits, cfg.proof_of_work_bits,
                                cfg.num_query_rounds, lg_d)
     for b in gpu:
@@ -403,7 +416,7 @@ def test_opening_set_and_plonk_instance(pcs):
     och.sponge_state = [int(x) for x in ch.sponge_state.state]
     och.input_buffer, och.output_buffer = list(ch.input_buffer), list(ch.output_buffer)
     proof = prove_openings(inst, gpu, ch, params)
-    assert fr.verify_fri_proof(batches, openings, och, [b.merkle_tree.cap.hashes for b in gpu], _as_oracle_proof(proof),
+    assert fr.verify_fri_proof(batches, openings, och, [b.merkle_tree.cap.hashes for b in gpu], as_oracle_proof(proof),
                                cfg.rate_bits, cfg.cap_height, params.reduction_arity_bits, cfg.proof_of_work_bits,
                                cfg.num_query_rounds, lg_d)
     for b in gpu:
@@ -447,10 +460,10 @@ def test_prove_openings_random_instances(pcs):
         want = fr.prove_openings(cpu, batches, och, rate_bits, cap_height, arities, pow_bits, n_q)
         ctx = (case, lg_d, rate_bits, cap_height, arities, widths)
         try:
-            _assert_same_proof(got, want)
+            assert_same_proof(got, want)
         except AssertionError as e:
             raise AssertionError(f"case {ctx}: {e}")
-        assert fr.verify_fri_proof(batches, openings, vch, [o["cap"] for o in cpu], _as_oracle_proof(got), rate_bits,
+        assert fr.verify_fri_proof(batches, openings, vch, [o["cap"] for o in cpu], as_oracle_proof(got), rate_bits,
                                    cap_height, arities, pow_bits, n_q, lg_d), ctx
         for b in gpu:
             b.free()
@@ -506,35 +519,3 @@ def test_device_pointer_entry_points_alignment_and_errors(pcs):
     with pytest.raises(pcs.PcsError, match="TWO_ADICITY"):
         _ffi.check(L.pcs_eval_ext_dev(_poly_ptr_array(addrs), w, 33, _ext_arg(z), _ffi.ptr(out)))
 
-
-def test_full_size_opening_properties(pcs):
-    """BASELINE's headline shape (135 x 2^20, rate 3): the oracle cannot redo the whole opening proof in seconds, so the
-    device results are checked through size-independent identities -- sampled polynomials against the CPU Horner
-    evaluation, and the quotient identity  final(x) * (x - z) == F(x) - F(z)  with F = sum_j alpha^j f_j, at a random x,
-    where F(x), F(z) come from device openings and final(x) from a CPU evaluation of the device's final polynomial."""
-    from plonky2_demo_b200.fri_prover import FriBatchInfo, FriInstanceInfo, FriOracleInfo, FriPolynomialInfo, eval_commitment, final_poly
-
-    w, lg_d = 135, 20
-    rng = np.random.default_rng(2026)
-    coeffs = rng.integers(0, 1 << 64, size=(w, 1 << lg_d), dtype=np.uint64)        # any u64: non-canonical inputs included
-    b = pcs.PolynomialBatch.from_coeffs(coeffs, 3, False, 4, keep_coeffs=True)
-    prng = random.Random(7)
-    z, x, alpha = rand_ext(prng), rand_ext(prng), rand_ext(prng)
-    at_z, at_x = eval_commitment(z, b), eval_commitment(x, b)
-    for j in (0, 67, 134):
-        assert tuple(int(v) for v in at_z[j]) == tuple(int(v) for v in fr.eval_base_polys_ext(coeffs[j:j + 1], z)[0])
-    inst = FriInstanceInfo([FriOracleInfo(w, False)], [FriBatchInfo(z, FriPolynomialInfo.from_range(0, range(w)))])
-    fin = final_poly(inst, [b], alpha)
-    fc = fin.coeffs
-    assert fc.shape == (1 << lg_d, 2) and (int(fc[-1, 0]), int(fc[-1, 1])) == (0, 0)   # quotient padded with one zero
-
-    def combine(vals):
-        acc = (0, 0)
-        for v in reversed(vals):
-            acc = fr.ext_add(fr.ext_mul(acc, alpha), (int(v[0]), int(v[1])))
-        return acc
-
-    lhs = fr.ext_mul(fr.ext_poly_eval(fc, x), fr.ext_sub(x, z))
-    assert lhs == fr.ext_sub(combine(at_x), combine(at_z))
-    fin.free()
-    b.free()

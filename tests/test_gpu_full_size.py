@@ -12,14 +12,19 @@ Every checked commit follows a decoy: other data of the same shape, committed th
 kernel over the whole leaf, or the streaming sponge over groups of columns), freed in stream order, with no host sync before
 the checked commit is enqueued, as in bench.py's timed loop.  Whatever the checked commit fails to write then holds the
 decoy's values.  The decoy takes the other form because a write skipped by one path is skipped by a decoy on that path too,
-and the memory can still hold the right values from an earlier case that committed the same data another way."""
+and the memory can still hold the right values from an earlier case that committed the same data another way.
+
+The opening proof bench.py times (eval_commitment, final_poly, prove_openings over the headline batch) is checked the same
+way: every opening, the 2^20-coefficient final polynomial, its 2^23-point LDE and the whole proof against fri_ref, on a
+resident and on an on-demand batch, each after a decoy proof over other data with non-canonical coefficients."""
 import ctypes as C
 
 import numpy as np
 import pytest
 
 import oracle
-from helpers import P, brev, seeded_polys
+from helpers import P, as_oracle_proof, assert_same_proof, brev, seeded_polys
+from oracle import fri_ref as fr
 
 pytestmark = pytest.mark.gpu
 
@@ -341,3 +346,155 @@ def test_deep_pageable_host(L, deep):
         _check(L, h, deep.digests, deep.cap, deep.idx, deep.rows, cap_out)
     finally:
         L.pcs_batch_free(h)
+
+
+# ---------------------------------------------------------------------------------------------
+# the opening proof bench.py times (kernels.fri_opening)
+# ---------------------------------------------------------------------------------------------
+ZETA = (0x0123456789ABCDEF % P, 0x0FEDCBA987654321 % P)   # bench.py's opening point
+N_NEXT = 20                                             # polynomials also opened at g * zeta
+FRI_ARITIES, POW_BITS, N_QUERIES = [4, 4, 4, 4], 16, 28  # standard_recursion_config at degree 2^20
+DECOY_ZETA, DECOY_ALPHA = (0x1DEC0, 0x2DEC0), (P - 5, 0xDEC0DEC0)
+
+
+def _opening_batches(zeta, w, lg_d):
+    zeta_next = fr.ext_mul((fr.primitive_root_of_unity(lg_d), 0), zeta)
+    return [(zeta, [(0, j) for j in range(w)]), (zeta_next, [(0, j) for j in range(min(N_NEXT, w))])]
+
+
+def _openings(coeffs, batches):
+    return [[tuple(int(x) for x in v) for v in fr.eval_base_polys_ext(coeffs[:len(polys)], pt)] for pt, polys in batches]
+
+
+class OpeningReference:
+    """fri_ref's opening proof over the headline batch, with bench.py's instance and transcript (the cap, then every
+    opening), and the decoy's openings and final polynomial.  The oracle holds no leaves: query rows are evaluated at
+    7 w_N^brev(i) and paths come from the digests.  The decoy's coefficients are non-canonical: every 7th is
+    presented as value + p (value < 2^31), and each polynomial starts with 2^64 - 1, p, p + 1."""
+
+    def __init__(self, ref):
+        self.batches = _opening_batches(ZETA, ref.w, ref.lg_d)
+        self.openings = _openings(ref.coeffs, self.batches)
+        och = fr.Challenger()
+        och.observe_cap(ref.cap)
+        for vals in self.openings:
+            och.observe_extension_elements(vals)
+        self.challenger = och.clone()
+        lg_n, w_n = ref.lg_d + ref.r, fr.primitive_root_of_unity(ref.lg_d + ref.r)
+
+        def rows(i):
+            x = fr.COSET_SHIFT * pow(w_n, brev(i, lg_n), P) % P
+            return fr.eval_base_polys_ext(ref.coeffs, (x, 0))[:, 0]
+
+        entry = {"coeffs": ref.coeffs, "cap_height": ref.cap_h, "rows": rows,
+                 "path": lambda i: oracle.merkle_prove(ref.digests, ref.n, ref.cap_h, i)}
+        self.proof = fr.prove_openings([entry], self.batches, och, ref.r, ref.cap_h, FRI_ARITIES, POW_BITS, N_QUERIES)
+        self.next_challenge = och.get_challenge()
+        nc = ref.decoy.copy()
+        flat = nc.reshape(-1)
+        flat[3::7] = (flat[3::7] & np.uint64((1 << 31) - 1)) + np.uint64(P)
+        nc[:, :3] = np.array([(1 << 64) - 1, P, P + 1], dtype=np.uint64)
+        self.decoy_nc = nc
+        canon = nc % np.uint64(P)
+        self.decoy_batches = _opening_batches(DECOY_ZETA, ref.w, ref.lg_d)
+        self.decoy_openings = _openings(canon, self.decoy_batches)
+        self.decoy_final = fr.final_poly([canon], self.decoy_batches, DECOY_ALPHA)
+
+
+@pytest.fixture(scope="module")
+def headline_opening(headline):
+    return OpeningReference(headline)
+
+
+def _commit_batch(L, pcs, dev, ref, flags):
+    """A PolynomialBatch over a commit of device coefficients with the coefficients kept, built as bench.py builds it."""
+    from plonky2_demo_b200 import _ffi
+    from plonky2_demo_b200.fri import _DeviceMerkleTree
+
+    h = C.c_void_p()
+    _ffi.check(L.pcs_commit_from_coeffs(_dev_ptrs(dev, 0, ref.w, ref.d), ref.w, ref.lg_d, ref.r, ref.cap_h, None, 0,
+                                        _ffi.PCS_DEVICE_PTRS | _ffi.PCS_KEEP_COEFFS | flags, None, C.byref(h)))
+    b = pcs.PolynomialBatch()
+    b._h, b._coeffs_host = h, []
+    b.degree_log, b.rate_bits, b.blinding, b.cap_height = ref.lg_d, ref.r, False, ref.cap_h
+    b.n_polys, b.salt_w, b.n_leaves = ref.w, 0, ref.n
+    b.n_digests = 2 * (ref.n - (1 << ref.cap_h))
+    b._cap = np.empty((1 << ref.cap_h, 4), dtype=np.uint64)
+    _ffi.check(L.pcs_batch_cap(h, _ffi.ptr(b._cap)))
+    b.merkle_tree = _DeviceMerkleTree(b)
+    return b
+
+
+def _instance(batches, w):
+    from plonky2_demo_b200.fri_prover import FriBatchInfo, FriInstanceInfo, FriOracleInfo, FriPolynomialInfo
+
+    return FriInstanceInfo([FriOracleInfo(w, False)],
+                           [FriBatchInfo(pt, [FriPolynomialInfo(o, j) for o, j in polys]) for pt, polys in batches])
+
+
+def _device_openings(b, batches):
+    from plonky2_demo_b200.fri_prover import eval_commitment
+
+    return [[tuple(int(x) for x in v) for v in eval_commitment(pt, b)[:len(polys)]] for pt, polys in batches]
+
+
+@pytest.mark.parametrize("on_demand", [False, True], ids=["resident", "on_demand"])
+def test_headline_opening_proof(L, headline, headline_opening, on_demand):
+    """bench.py's opening proof, exact: 155 openings, the final polynomial (2^20 coefficients) and its LDE (2^23 values),
+    and the proof field by field (4 commit-phase caps, final polynomial, PoW witness, 28 indices, initial rows and paths,
+    every step's evals and path); both transcripts end in the same state and the restated verifier accepts.
+
+    First a decoy: an on-demand batch over the decoy's non-canonical coefficients, whose openings and final polynomial are
+    checked, and a proof over it with other challenges, freed in stream order; whatever the checked proof fails to write
+    then holds the decoy's values, not the other arm's."""
+    import plonky2_demo_b200 as pcs
+    from plonky2_demo_b200 import _ffi
+    from plonky2_demo_b200.fri_prover import Challenger, final_poly, prove_openings
+
+    ref, want = headline, headline_opening
+    cfg = pcs.CircuitConfig.standard_recursion_config().fri_config
+    cfg = pcs.FriConfig(ref.r, ref.cap_h, cfg.proof_of_work_bits, cfg.reduction_strategy, cfg.num_query_rounds)
+    params = cfg.fri_params(ref.lg_d, False)
+    assert (params.reduction_arity_bits, cfg.proof_of_work_bits, cfg.num_query_rounds) == (FRI_ARITIES, POW_BITS, N_QUERIES)
+
+    dev_decoy = _to_device(want.decoy_nc)
+    db = _commit_batch(L, pcs, dev_decoy, ref, _ffi.PCS_LDE_ON_DEMAND)
+    del dev_decoy
+    try:
+        assert _device_openings(db, want.decoy_batches) == want.decoy_openings
+        fin = final_poly(_instance(want.decoy_batches, ref.w), [db], DECOY_ALPHA)
+        try:
+            _assert_rows_equal(fin.coeffs, want.decoy_final, "decoy final polynomial")
+        finally:
+            fin.free()
+        ch = Challenger()
+        ch.observe_cap(db.merkle_tree.cap)
+        prove_openings(_instance(want.decoy_batches, ref.w), [db], ch, params)
+    finally:
+        db.free()
+
+    dev = _to_device(ref.coeffs)
+    b = _commit_batch(L, pcs, dev, ref, _ffi.PCS_LDE_ON_DEMAND if on_demand else 0)
+    del dev
+    try:
+        _assert_rows_equal(b.merkle_tree.cap.hashes, ref.cap, "cap")
+        openings = _device_openings(b, want.batches)
+        assert openings == want.openings
+        inst = _instance(want.batches, ref.w)
+        ch = Challenger()
+        ch.observe_cap(b.merkle_tree.cap)
+        for vals in openings:
+            ch.observe_extension_elements(vals)
+        got = prove_openings(inst, [b], ch, params)
+        assert_same_proof(got, want.proof)
+        assert ch.get_challenge() == want.next_challenge
+        assert fr.verify_fri_proof(want.batches, openings, want.challenger.clone(), [ref.cap], as_oracle_proof(got), ref.r,
+                                   ref.cap_h, FRI_ARITIES, POW_BITS, N_QUERIES, ref.lg_d)
+        fin = final_poly(inst, [b], want.proof["_alpha"])
+        try:
+            _assert_rows_equal(fin.coeffs, want.proof["_final_poly_full"], "final polynomial")
+            _assert_rows_equal(fin.lde_coset_fft(ref.r), want.proof["_lde_values"], "final polynomial LDE")
+        finally:
+            fin.free()
+    finally:
+        b.free()

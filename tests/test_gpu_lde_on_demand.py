@@ -13,7 +13,7 @@ import numpy as np
 import pytest
 
 import oracle
-from helpers import P, brev, seeded_polys, splitmix64_stream
+from helpers import P, as_oracle_proof, assert_same_proof, brev, seeded_polys, splitmix64_stream
 from oracle import fri_ref as fr
 
 pytestmark = pytest.mark.gpu
@@ -246,37 +246,6 @@ def test_on_demand_refusals(L):
 # ---------------------------------------------------------------------------------------------
 # opening proofs over on-demand oracles (prove_openings reads rows through get_rows)
 # ---------------------------------------------------------------------------------------------
-def _assert_same_proof(got, want):
-    assert len(got.commit_phase_merkle_caps) == len(want["commit_phase_merkle_caps"])
-    for c, wc in zip(got.commit_phase_merkle_caps, want["commit_phase_merkle_caps"]):
-        assert np.array_equal(c.hashes, wc)
-    assert np.array_equal(got.final_poly, want["final_poly"])
-    assert got.pow_witness == want["pow_witness"]
-    assert got.fri_query_indices == want["_indices"]
-    assert len(got.query_round_proofs) == len(want["query_round_proofs"])
-    for r, wr in zip(got.query_round_proofs, want["query_round_proofs"]):
-        for (ev, mp), (wev, wmp) in zip(r.initial_trees_proof.evals_proofs, wr["initial_trees_proof"]):
-            assert np.array_equal(ev, wev)
-            assert np.array_equal(np.asarray(mp.siblings).reshape(-1, 4), wmp)
-        assert len(r.steps) == len(wr["steps"])
-        for s, ws in zip(r.steps, wr["steps"]):
-            assert np.array_equal(s.evals, ws["evals"])
-            assert np.array_equal(np.asarray(s.merkle_proof.siblings).reshape(-1, 4), ws["merkle_proof"])
-
-
-def _as_oracle_proof(proof):
-    return {
-        "commit_phase_merkle_caps": [c.hashes for c in proof.commit_phase_merkle_caps],
-        "final_poly": proof.final_poly,
-        "pow_witness": proof.pow_witness,
-        "query_round_proofs": [
-            {"initial_trees_proof": [(ev, np.asarray(mp.siblings).reshape(-1, 4)) for ev, mp in r.initial_trees_proof.evals_proofs],
-             "steps": [{"evals": s.evals, "merkle_proof": np.asarray(s.merkle_proof.siblings).reshape(-1, 4)} for s in r.steps]}
-            for r in proof.query_round_proofs
-        ],
-    }
-
-
 @pytest.mark.parametrize("lg_d,rate_bits,cap_height,arities,widths,n_queries", [
     (7, 3, 4, [4], [6, 9, 3, 2], 28),           # few query rows: evaluated from the coefficients
     (9, 2, 2, [2, 2], [17, 5, 24, 3], 300),     # more than ROWS_EVAL_MAX: the LDE is regenerated
@@ -315,8 +284,8 @@ def test_prove_openings_over_on_demand_oracles(L, lg_d, rate_bits, cap_height, a
         verifier_ch = och.clone()
         got = prove_openings(inst, gpu, ch, params)
         want = fr.prove_openings(cpu, batches, och, rate_bits, cap_height, arities, pow_bits, n_queries)
-        _assert_same_proof(got, want)
-        assert fr.verify_fri_proof(batches, openings, verifier_ch, [o["cap"] for o in cpu], _as_oracle_proof(got), rate_bits,
+        assert_same_proof(got, want)
+        assert fr.verify_fri_proof(batches, openings, verifier_ch, [o["cap"] for o in cpu], as_oracle_proof(got), rate_bits,
                                    cap_height, arities, pow_bits, n_queries, lg_d)
         for b in gpu:
             b.free()
@@ -398,26 +367,53 @@ def test_headline_shape_matches_resident_commit(L):
         L.pcs_batch_free(hr)
 
 
+def _mem_available_bytes():
+    try:
+        with open("/proc/meminfo") as f:
+            for line in f:
+                if line.startswith("MemAvailable:"):
+                    return int(line.split()[1]) * 1024
+    except OSError:
+        pass
+    return 0
+
+
 def test_large_commit_on_one_gpu(L):
-    """135 x 2^24 at rate 3: 145 GB of LDE rows as a resident batch, which does not fit one B200."""
+    """135 x 2^24 at rate 3: 145 GB of LDE rows as a resident batch, which does not fit one B200.  Rows equal direct
+    evaluation and Merkle paths verify against the cap.  Then configs[4]'s opening proof over it (bench.py's instance at
+    degree 2^24: all at zeta, the first 20 at g * zeta, arities [4] x 5, 28 queries, 16 PoW bits) against fri_ref: the CPU
+    cannot build this commitment's tree, so the transcript observes the device's cap, initial-tree rows come from direct
+    evaluation and initial-tree paths from pcs_batch_prove_many (the verifier checks them against the cap); everything else
+    must be equal: openings, the 2^24-coefficient final polynomial and its 2^27-point LDE, 5 commit-phase caps, the final
+    polynomial, the PoW witness and every query step."""
     import torch
 
+    import plonky2_demo_b200 as pcs
     from plonky2_demo_b200 import _ffi
+    from plonky2_demo_b200.fri import _DeviceMerkleTree
+    from plonky2_demo_b200.fri_prover import (Challenger, FriBatchInfo, FriInstanceInfo, FriOracleInfo, FriPolynomialInfo,
+                                              eval_commitment, final_poly, prove_openings)
 
     w, lg_d, r, cap_h = 135, 24, 3, 4
     d, n = 1 << lg_d, 1 << (lg_d + r)
-    free = torch.cuda.mem_get_info()[0]
+    free, host_mem = torch.cuda.mem_get_info()[0], _mem_available_bytes()
     if free < (80 << 30):
         pytest.skip(f"135 x 2^24 on demand needs 80 GiB of free HBM ({free >> 30} GiB free)")
+    if host_mem < (40 << 30):
+        pytest.skip(f"the 135 x 2^24 CPU reference needs 40 GiB of host memory ({host_mem >> 30} GiB available)")
     gen = torch.Generator(device="cuda").manual_seed(0x24)
     x = torch.randint(0, 1 << 62, (w, d), dtype=torch.int64, device="cuda", generator=gen)
     cap = np.empty((1 << cap_h, 4), dtype=np.uint64)
     h = C.c_void_p()
     _ffi.check(L.pcs_commit_from_coeffs(_ffi.dev_ptr_array(x.data_ptr(), w, d), w, lg_d, r, cap_h, None, 0,
                                         _ffi.PCS_DEVICE_PTRS | _ffi.PCS_LDE_ON_DEMAND, _ffi.ptr(cap), C.byref(h)))
+    b = pcs.PolynomialBatch()
+    b._h, b._coeffs_host, b._cap = h, [], cap
+    b.degree_log, b.rate_bits, b.blinding, b.cap_height = lg_d, r, False, cap_h
+    b.n_polys, b.salt_w, b.n_leaves, b.n_digests = w, 0, n, 2 * (n - (1 << cap_h))
+    b.merkle_tree = _DeviceMerkleTree(b)
     try:
-        polys = [0, 1, 67, 134]
-        host = {j: x[j].cpu().numpy().view(np.uint64) for j in polys}
+        coeffs = x.cpu().numpy().view(np.uint64)                 # 18 GB: the CPU reference's input
         del x
         torch.cuda.empty_cache()
         rng = np.random.default_rng(24)
@@ -426,12 +422,51 @@ def test_large_commit_on_one_gpu(L):
         g = oracle.primitive_root_of_unity(lg_d + r)
         for k, leaf in enumerate(idx):
             xk = oracle.gl_mul(7, oracle.gl_pow(g, brev(int(leaf), lg_d + r)))
-            for j in polys:
-                assert int(rows[k, j]) == oracle.poly_eval(host[j], xk), (int(leaf), j)
+            for j in [0, 1, 67, 134]:
+                assert int(rows[k, j]) == oracle.poly_eval(coeffs[j], xk), (int(leaf), j)
         idx = rng.integers(0, n, size=64).astype(np.uint64)
         rows = _get_rows(L, h, idx, w)
         sib = _prove_many(L, h, idx, lg_d + r - cap_h)
         for k, leaf in enumerate(idx):
             assert oracle.merkle_verify(rows[k], int(leaf), cap, sib[k])
+
+        # configs[4]'s opening proof
+        zeta = (0x0123456789ABCDEF % P, 0x0FEDCBA987654321 % P)
+        batches = [(zeta, [(0, j) for j in range(w)]),
+                   (fr.ext_mul((fr.primitive_root_of_unity(lg_d), 0), zeta), [(0, j) for j in range(20)])]
+        inst = FriInstanceInfo([FriOracleInfo(w, False)],
+                               [FriBatchInfo(pt, [FriPolynomialInfo(o, j) for o, j in ps]) for pt, ps in batches])
+        openings = [[tuple(int(v) for v in row) for row in eval_commitment(pt, b)[:len(ps)]] for pt, ps in batches]
+        for (pt, ps), vals in zip(batches, openings):
+            assert vals == [tuple(int(v) for v in row) for row in fr.eval_base_polys_ext(coeffs[:len(ps)], pt)], pt
+        cfg = pcs.CircuitConfig.standard_recursion_config().fri_config
+        params = cfg.fri_params(lg_d, False)
+        assert (cfg.rate_bits, cfg.cap_height, params.reduction_arity_bits) == (r, cap_h, [4] * 5)
+        ch, och = Challenger(), fr.Challenger()
+        for c in (ch, och):
+            c.observe_cap(cap)
+            for vals in openings:
+                c.observe_extension_elements(vals)
+        verifier_ch = och.clone()
+        got = prove_openings(inst, [b], ch, params)
+
+        def eval_row(i):
+            xi = fr.COSET_SHIFT * pow(g, brev(i, lg_d + r), P) % P
+            return fr.eval_base_polys_ext(coeffs, (xi, 0))[:, 0]
+
+        entry = {"coeffs": coeffs, "cap_height": cap_h, "rows": eval_row,
+                 "path": lambda i: np.asarray(b.prove_many([i])[0].siblings).reshape(-1, 4)}
+        want = fr.prove_openings([entry], batches, och, r, cap_h, params.reduction_arity_bits, cfg.proof_of_work_bits,
+                                 cfg.num_query_rounds)
+        assert_same_proof(got, want)
+        assert ch.get_challenge() == och.get_challenge()
+        assert fr.verify_fri_proof(batches, openings, verifier_ch, [cap], as_oracle_proof(got), r, cap_h,
+                                   params.reduction_arity_bits, cfg.proof_of_work_bits, cfg.num_query_rounds, lg_d)
+        fin = final_poly(inst, [b], want["_alpha"])
+        try:
+            assert np.array_equal(fin.coeffs, want["_final_poly_full"])
+            assert np.array_equal(fin.lde_coset_fft(r), want["_lde_values"])
+        finally:
+            fin.free()
     finally:
-        L.pcs_batch_free(h)
+        b.free()

@@ -86,9 +86,9 @@ def test_two_to_one(pcs):
 # ---------------------------------------------------------------------------------------------
 # NTT / LDE (reference properties: fft.rs:219-253, polynomial/mod.rs:478-518)
 # ---------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("lg_n", [0, 1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11, 12, 13, 14, 15, 16, 17, 18, 19, 20, 21, 22])
+@pytest.mark.parametrize("lg_n", [0, 1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11, 12, 13, 14, 15, 16, 17, 18, 19, 20, 21, 22, 23, 24])
 def test_ntt_forward_inverse(pcs, lg_n):
-    # every pass-kernel instantiation (1..10 stages per pass) and the 1-, 2- and 3-pass plans
+    # every pass-kernel instantiation (1..10 stages per pass) and the 1-, 2- and 3-pass plans (lg 23: [7, 8, 8], 24: [8, 8, 8])
     from plonky2_demo_b200.polynomial import ntt_batch
 
     w = 2 if lg_n > 16 else 3 if lg_n > 12 else 9
