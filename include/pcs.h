@@ -88,8 +88,7 @@ PCS_API int pcs_synchronize(void);
 typedef enum {
     PCS_OP_ADD = 0,       /* goldilocks_field.rs:199-221                                              */
     PCS_OP_SUB = 1,       /* :223-243                                                                 */
-    PCS_OP_MUL = 2,       /* :267-274, reduce128 :356-369 (the Poseidon kernels' reduction)           */
-    PCS_OP_MUL_MAD = 3,   /* the same product through the NTT kernels' multiply-add reduction         */
+    PCS_OP_MUL = 2,       /* :267-274, reduce128 :356-369 (the kernels' reduction); 3 is unused       */
     PCS_OP_SQUARE = 4,
     PCS_OP_CANON = 5,     /* to_canonical_u64 :171-178                                                */
     PCS_OP_NEG = 6,       /* :245-255                                                                 */

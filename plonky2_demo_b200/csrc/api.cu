@@ -365,7 +365,8 @@ int pcs_field_op(int op, const uint64_t* a, const uint64_t* b, size_t n, uint64_
     if (int rc = need_init()) return rc;
     if (n == 0) return PCS_OK;
     if (!a || !out) return fail(PCS_ERR_ARG, "NULL pointer");
-    if (op < PCS_OP_ADD || op > PCS_OP_MUL_2EXP) return fail(PCS_ERR_ARG, "unknown field operation");
+    if (op < PCS_OP_ADD || op > PCS_OP_MUL_2EXP || op == 3 /* no operation has this value */)
+        return fail(PCS_ERR_ARG, "unknown field operation");
     const bool binary = op != PCS_OP_SQUARE && op != PCS_OP_CANON && op != PCS_OP_NEG;
     if (binary && !b) return fail(PCS_ERR_ARG, "second operand is NULL");
     cudaStream_t st = g_ctx.stream;

@@ -1,7 +1,7 @@
 // Element-wise Goldilocks field operations on the device (pcs_field_op): the device counterpart of the reference's
 // field-arithmetic grid test (field/src/prime_field_testing.rs:7-17,78-125, instantiated goldilocks_field.rs:405-411).
-// Every arithmetic routine of gl64.cuh that the kernels build on is reachable here, including BOTH 128-bit reductions
-// (reduce128 in the form the Poseidon S-boxes and the NTT butterflies are built with, and the multiply-add form reduce128_mad), so the tests can compare each of them with
+// Every arithmetic routine of gl64.cuh that the kernels build on is reachable here, including the 128-bit reduction that
+// the Poseidon S-boxes and the NTT butterflies are built with, so the tests can compare each of them with
 // big-int arithmetic on the boundary inputs {0..9, 2^31+-10, 2^32+-10, 2^63+-10, p-10..p-1, non-canonical values}.
 #include "common.cuh"
 #include "gl64.cuh"
@@ -18,7 +18,6 @@ __global__ void k_field_op(int op, const uint64_t* __restrict__ a, const uint64_
         case PCS_OP_ADD: r = gl::add_lc(x, gl::canon(y)); break;             // loose + canonical, goldilocks_field.rs:199-221
         case PCS_OP_SUB: r = gl::sub_lc(x, gl::canon(y)); break;             // :223-243
         case PCS_OP_MUL: r = gl::mul(x, y); break;                            // :267-274 + reduce128 :356-369
-        case PCS_OP_MUL_MAD: r = gl::mul_mad(x, y); break;                    // the NTT butterfly's reduction
         case PCS_OP_SQUARE: r = gl::sqr(x); break;
         case PCS_OP_CANON: r = x; break;                                      // to_canonical_u64 :171-178
         case PCS_OP_NEG: r = gl::sub_lc(0, gl::canon(x)); break;              // :245-255

@@ -244,34 +244,9 @@ __device__ __forceinline__ uint64_t& tile_at(uint64_t* tile, uint32_t base_bytes
     return *reinterpret_cast<uint64_t*>(reinterpret_cast<char*>(tile) + (base_bytes ^ (sw(c) << 3)));
 }
 
-// The butterfly's modular multiplication and addition.  PCS_NTT_MUL: 0 = the multiply-add reduction (gl::mul_mad, rounds 1-2:
-// 17 SASS), 2 = the wide reduction (gl::reduce128_wide: 14 SASS, the same number on the ALU pipe and three fewer on the IMAD
-// pipe; LDE of 135 x 2^20 at rate 3: 20.16 -> 19.61 ms, profiles/r02_forms.md).  PCS_NTT_ADD: 0 = gl::add_lc (7 SASS, 4 of them
-// ALU), 1 = gl::add_lc_wide (5 SASS, all ALU: one more on the pipe that bounds the kernel, 128 registers and spills -- not used).
-#ifndef PCS_NTT_MUL
-#define PCS_NTT_MUL 2
-#endif
-#ifndef PCS_NTT_ADD
-#define PCS_NTT_ADD 0
-#endif
-__device__ __forceinline__ uint64_t ntt_mul(uint64_t a, uint64_t b) {
-#if PCS_NTT_MUL == 2
-    unsigned __int128 q = (unsigned __int128)a * b;
-    return gl::reduce128_wide((uint64_t)q, (uint64_t)(q >> 64));
-#else
-    return gl::mul_mad(a, b);
-#endif
-}
-__device__ __forceinline__ uint64_t ntt_add(uint64_t a, uint64_t b) {
-#if PCS_NTT_ADD == 1
-    return gl::add_lc_wide(a, b);
-#else
-    return gl::add_lc(a, b);
-#endif
-}
-
 // K stages on 32 registers; stage s pairs (j, j+16) with twiddle twp[s*16*STRIDE + j*STRIDE] and
-// rotates the register index left by one bit.
+// rotates the register index left by one bit.  The butterfly adds with gl::add_lc, not gl::add_lc_wide: the wide add puts one
+// more instruction on the ALU pipe, which bounds this kernel.
 template <int STRIDE>
 __device__ __forceinline__ void run_stages(uint64_t (&x)[32], const uint64_t* twp, int k) {
 #pragma unroll 1
@@ -279,8 +254,8 @@ __device__ __forceinline__ void run_stages(uint64_t (&x)[32], const uint64_t* tw
         uint64_t y[32];
 #pragma unroll
         for (int j = 0; j < 16; j++) {
-            uint64_t t = gl::canon(ntt_mul(x[j + 16], twp[j * STRIDE]));
-            y[2 * j] = ntt_add(x[j], t);
+            uint64_t t = gl::canon(gl::mul(x[j + 16], twp[j * STRIDE]));
+            y[2 * j] = gl::add_lc(x[j], t);
             y[2 * j + 1] = gl::sub_lc(x[j], t);
         }
 #pragma unroll

@@ -7,18 +7,17 @@
 // reference's own `consistency` test (poseidon.rs:777-790) licenses any algebraically equal
 // evaluation order, and tests/ pin this kernel to the reference KATs (poseidon_goldilocks.rs:461-482).
 //
-// Design for the B200 integer pipes (no tensor cores: 64-bit modular arithmetic).  Measured rates
-// (profiles/r01_intpipe.md): IADD3 128/clk/SM, IMAD/LOP3/SHF 64, IMAD.WIDE 32 -- so the wide
-// multiplier is the scarce unit and is reserved for the S-boxes (4 IMAD.WIDE per modmul):
-//  * MDS layer = add/shift network, zero multiplies.  Each lane is split in 32-bit halves; the
-//    12-point circulant product of a half is computed exactly in int64 through the factorisation
-//    x^12 - 1 = prod over zeta in {1,-1,i,-i} of (x^3 - zeta) with x^4 = zeta (three 4-point integer
-//    DFTs, three 3x3 twisted products whose constants are (2+i), (-4-i), (16-i), [16,32,16],
-//    [-1,-8,2] -- the MDS matrix was designed to have these -- and three inverse DFTs).  Same
-//    mathematics as the reference's x86 path (poseidon_goldilocks.rs:217-248,307-441), derived
-//    and verified independently in tests/golden/make_golden.py:mds_network_check.
-//    The next round's constant is folded into the network's additions (3-input IADD3), so
-//    constant_layer costs nothing; one 96-bit fold per lane brings the result back to 64 bits.
+// Design for the B200 integer and FP64 pipes.  Measured rates (profiles/r01_intpipe.md): IADD3 128/clk/SM,
+// IMAD/LOP3/SHF 64, IMAD.WIDE 32 -- so the wide multiplier is the scarce unit and is reserved for the S-boxes
+// (4 IMAD.WIDE per modmul):
+//  * MDS layer = add/shift network, zero multiplies, run on the FP64 pipe (mds_layer_fp64).  Each lane is split in
+//    32-bit halves; the 12-point circulant product of a half is computed exactly in doubles through the factorisation
+//    x^12 - 1 = prod over zeta in {1,-1,i,-i} of (x^3 - zeta) with x^4 = zeta (three 4-point DFTs, three 3x3 twisted
+//    products whose constants are (2+i), (-4-i), (16-i), [16,32,16], [-1,-8,2] -- the MDS matrix was designed to have
+//    these -- and three inverse DFTs).  Same mathematics as the reference's x86 path (poseidon_goldilocks.rs:217-248,
+//    307-441), derived and verified independently in tests/golden/make_golden.py:mds_network_check.
+//    The next round's constant is folded into the network's last additions, so constant_layer costs nothing; one
+//    96-bit fold per lane (gl::fold_halves_biased) brings the result back to 64 bits.
 //  * partial rounds use the same network's middle stage alone, with the state kept in its transform
 //    domain (crt_mid_half) and the scalar FAST_PARTIAL_ROUND_CONSTANTS[r] added to lane 0 after
 //    its S-box; the sparse "fast" matrices of poseidon.rs:584-596 would need 23 full 64x64
@@ -28,13 +27,6 @@
 #include "poseidon_constants.cuh"
 
 namespace pcs {
-
-#ifndef PCS_MDS_FP64
-#define PCS_MDS_FP64 1
-#endif
-#ifndef PCS_SBOX_GROUP
-#define PCS_SBOX_GROUP 12
-#endif
 
 constexpr int SPONGE_WIDTH = 12;
 constexpr int SPONGE_RATE = 8;
@@ -46,66 +38,8 @@ __device__ __forceinline__ uint64_t sbox7(uint64_t x) {
     return gl::mul(x3, x4);
 }
 
-// y = circ-correlation(s) + 8*s0*e0 + add, for 12 non-negative 32-bit inputs; exact in int64
-// (|intermediates| < 2^40, results < 2^43 + add).
-__device__ __forceinline__ void mds_half(const uint32_t (&s)[12], const uint32_t (&add)[12], uint64_t (&y)[12]) {
-    int64_t A[3], B[3], P[3], Q[3];
-#pragma unroll
-    for (int j = 0; j < 3; j++) {
-        int64_t s0 = s[j], s3 = s[j + 3], s6 = s[j + 6], s9 = s[j + 9];
-        int64_t u = s0 + s6, v = s3 + s9;
-        A[j] = u + v;    // S_j(1)
-        B[j] = u - v;    // S_j(-1)
-        P[j] = s0 - s6;  // Re S_j(i)
-        Q[j] = s3 - s9;  // Im S_j(i)
-    }
-    // zeta = 1: cyclic 3-product with [16, 32, 16]
-    int64_t t = A[0] + A[1] + A[2];
-    int64_t Ya[3] = {(t + A[2]) << 4, (t + A[0]) << 4, (t + A[1]) << 4};
-    // zeta = -1: negacyclic 3-product with [-1, -8, 2]
-    int64_t Yb[3] = {(B[2] << 3) - (B[1] << 1) - B[0],
-                     -(B[0] << 3) - B[1] - (B[2] << 1),
-                     (B[0] << 1) - (B[1] << 3) - B[2]};
-    // zeta = i: i-twisted 3-product with (2+i), (-4-i), (16-i)
-    int64_t re[3], im[3];
-    re[0] = (P[0] << 1) - Q[0] + P[1] - (Q[1] << 4) + P[2] + (Q[2] << 2);
-    im[0] = P[0] + (Q[0] << 1) + (P[1] << 4) + Q[1] - (P[2] << 2) + Q[2];
-    re[1] = -(P[0] << 2) + Q[0] + (P[1] << 1) - Q[1] + P[2] - (Q[2] << 4);
-    im[1] = -P[0] - (Q[0] << 2) + P[1] + (Q[1] << 1) + (P[2] << 4) + Q[2];
-    re[2] = (P[0] << 4) + Q[0] - (P[1] << 2) + Q[1] + (P[2] << 1) - Q[2];
-    im[2] = -P[0] + (Q[0] << 4) - P[1] - (Q[1] << 2) + P[2] + (Q[2] << 1);
-#pragma unroll
-    for (int j = 0; j < 3; j++) {
-        int64_t e1 = Ya[j] + Yb[j], e2 = Ya[j] - Yb[j];
-        y[j] = (uint64_t)(e1 + re[j] + (int64_t)add[j]);
-        y[j + 3] = (uint64_t)(e2 + im[j] + (int64_t)add[j + 3]);
-        y[j + 6] = (uint64_t)(e1 - re[j] + (int64_t)add[j + 6]);
-        y[j + 9] = (uint64_t)(e2 - im[j] + (int64_t)add[j + 9]);
-    }
-    y[0] += (uint64_t)s[0] << 3;  // MDS_MATRIX_DIAG[0] = 8
-}
-
-// s <- MDS * s + rc   (rc = nullptr: no constant; lane0_only: rc[0] is added to lane 0 only)
-template <int RC_MODE /*0 none, 1 all 12 lanes, 2 lane 0 only*/>
-__device__ __forceinline__ void mds_layer(uint64_t (&s)[12], const uint64_t* __restrict__ rc) {
-    uint32_t lo[12], hi[12], alo[12], ahi[12];
-#pragma unroll
-    for (int i = 0; i < 12; i++) {
-        lo[i] = (uint32_t)s[i];
-        hi[i] = (uint32_t)(s[i] >> 32);
-        uint64_t c = (RC_MODE == 1 || (RC_MODE == 2 && i == 0)) ? rc[i] : 0;
-        alo[i] = (uint32_t)c;
-        ahi[i] = (uint32_t)(c >> 32);
-    }
-    uint64_t L[12], H[12];
-    mds_half(lo, alo, L);
-    mds_half(hi, ahi, H);
-#pragma unroll
-    for (int r = 0; r < 12; r++) s[r] = gl::fold_halves(L[r], H[r]);
-}
-
 // ------------------------------------------------------------------------------------------------
-// The same network on the FP64 pipe.
+// The MDS network on the FP64 pipe.
 //
 // B200 has a full-rate FP64 pipe (measured 61 DFMA/clk/SM, co-issuing with the integer pipes at
 // 121 instr/clk/SM, profiles/r01_fp64pipe.md) that integer code leaves idle, while the integer
@@ -167,7 +101,7 @@ __device__ __forceinline__ void mds_half_fp64(const uint32_t (&s)[12], const dou
     }
 }
 
-// s <- MDS * s + ROUND_ADD[r]  on the FP64 pipe; rcd = &ROUND_ADD_D[24 * r]
+// s <- MDS * s + add[r]  on the FP64 pipe; rcd = &ROUND_ADD_D[24 * r] (add[r]: see full_round)
 __device__ __forceinline__ void mds_layer_fp64(uint64_t (&s)[12], const uint64_t* __restrict__ rcd) {
     const double* addb = reinterpret_cast<const double*>(rcd);
     uint32_t lo[12], hi[12];
@@ -337,7 +271,7 @@ __device__ __forceinline__ uint64_t fold_signed_d(double lo, double hi) {
 // (el, eh): ext of the current U, (xl, xh): x_prev, becomes x; rc = PARTIAL_RC[r].
 __device__ __forceinline__ void lane0_crt(double el, double eh, double& xl, double& xh, uint64_t rc, double& gl, double& gh) {
     const uint64_t s0 = fold_signed_d(fma(xl, 8.0, el), fma(xh, 8.0, eh));
-    const uint64_t x = gl::add_lc_p(sbox7(s0), rc);
+    const uint64_t x = gl::add_lc_wide(sbox7(s0), rc);
     // x - ext = (x - s_0) + 8 x_prev
     gl = fma(xl, 8.0, u32_biased((uint32_t)x) - u32_biased((uint32_t)s0));
     gh = fma(xh, 8.0, u32_biased((uint32_t)(x >> 32)) - u32_biased((uint32_t)(s0 >> 32)));
@@ -345,51 +279,26 @@ __device__ __forceinline__ void lane0_crt(double el, double eh, double& xl, doub
     xh = u32_as_double((uint32_t)(x >> 32));
 }
 
-#ifndef PCS_PARTIAL_FP64
-#define PCS_PARTIAL_FP64 1
-#endif
-
 // The permutation.  Input lanes: any u64 (loose); output lanes: canonical (CANON_OUT) or loose -- a sponge feeds the state
 // straight into the next permutation and canonicalises only the digest it finally emits.
 //
-// ONE round loop for all 30 rounds (the body is ~22 KB of SASS and must stay resident in the SM's
-// instruction cache: with separate full/partial loop bodies the kernel was instruction-fetch bound,
-// profiles/r01_leafhash_v2.md).  Every round is  "s-box ; s = M s + ROUND_ADD[r]"  where the s-box
-// covers all lanes in the 8 full rounds and lane 0 only in the 22 partial rounds (warp-uniform
-// branch) and ROUND_ADD[r] is the constant needed by the NEXT s-box layer moved behind the linear
-// layer (tests/golden/make_golden.py:round_addends); it is absorbed by 3-input adds of the network.
+// A full round is  "12 s-boxes ; s = M s + add[r]"  where add[r] is the constant needed by the NEXT s-box layer moved behind
+// the linear layer (tests/golden/make_golden.py:round_addends), held as biased doubles in ROUND_ADD_D and absorbed by the
+// network's last additions.  The code must stay resident in the SM's instruction cache (with separate loop bodies for
+// every round group the kernel was instruction-fetch bound, profiles/r01_leafhash_v2.md), so the two groups of full rounds
+// share one loop body.
 __device__ __forceinline__ void full_round(uint64_t (&s)[12], int r) {
     using namespace pconst;
-#if PCS_SBOX_GROUP == 12
 #pragma unroll
     for (int i = 0; i < 12; i++) s[i] = sbox7(s[i]);
-#else
-    // S-box layer as a rolled loop over groups of lanes (the state rotates by one group per pass): smaller code for
-    // the instruction cache at the price of 2 register moves per lane per pass
-#pragma unroll 1
-    for (int g = 0; g < 12 / PCS_SBOX_GROUP; g++) {
-        uint64_t t[PCS_SBOX_GROUP];
-#pragma unroll
-        for (int i = 0; i < PCS_SBOX_GROUP; i++) t[i] = sbox7(s[i]);
-#pragma unroll
-        for (int i = 0; i < 12 - PCS_SBOX_GROUP; i++) s[i] = s[i + PCS_SBOX_GROUP];
-#pragma unroll
-        for (int i = 0; i < PCS_SBOX_GROUP; i++) s[12 - PCS_SBOX_GROUP + i] = t[i];
-    }
-#endif
-#if PCS_MDS_FP64
     mds_layer_fp64(s, &ROUND_ADD_D[24 * r]);
-#else
-    mds_layer<1>(s, &ROUND_ADD[12 * r]);
-#endif
 }
 
 template <bool CANON_OUT = true>
 __device__ __forceinline__ void poseidon12(uint64_t (&s)[12]) {
     using namespace pconst;
 #pragma unroll
-    for (int i = 0; i < 12; i++) s[i] = gl::add_lc_p(s[i], RC[i]);
-#if PCS_PARTIAL_FP64 && PCS_MDS_FP64
+    for (int i = 0; i < 12; i++) s[i] = gl::add_lc_wide(s[i], RC[i]);
     // rounds 0..3 (full), 4..25 (partial, FP64 transform domain), 26..29 (full): the two full-round groups share
     // ONE loop body (phase 0 and phase 1) so that the code stays small enough for the instruction cache
 #pragma unroll 1
@@ -411,7 +320,7 @@ __device__ __forceinline__ void poseidon12(uint64_t (&s)[12]) {
             }
             double el = u32_as_double((uint32_t)s[0]), eh = u32_as_double((uint32_t)(s[0] >> 32));
             double xl = 0.0, xh = 0.0;
-            // the 22nd round runs G then H (the lanes, + RC[26] as 2^52 + halves of ROUND_ADD[25]) instead of S G
+            // the 22nd round runs G then H (the lanes, + RC[26] as 2^52 + halves of add[25]) instead of S G
             const double* rcd = reinterpret_cast<const double*>(&ROUND_ADD_D[24 * 25]);
 #pragma unroll 1
             for (int k = 0; k < 11; k++) {
@@ -444,22 +353,6 @@ __device__ __forceinline__ void poseidon12(uint64_t (&s)[12]) {
             }
         }
     }
-#else
-#pragma unroll 1
-    for (int r = 0; r < 30; r++) {
-        if (r < 4 || r >= 26) {
-#pragma unroll
-            for (int i = 0; i < 12; i++) s[i] = sbox7(s[i]);
-        } else {
-            s[0] = sbox7(s[0]);
-        }
-#if PCS_MDS_FP64
-        mds_layer_fp64(s, &ROUND_ADD_D[24 * r]);
-#else
-        mds_layer<1>(s, &ROUND_ADD[12 * r]);
-#endif
-    }
-#endif
     if (CANON_OUT) {
 #pragma unroll
         for (int i = 0; i < 12; i++) s[i] = gl::canon(s[i]);

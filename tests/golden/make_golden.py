@@ -18,7 +18,6 @@ Outputs (all committed):
        - field-op input grid               field/src/prime_field_testing.rs:7-17,78-125 (rule, restated)
   oracle/poseidon_constants.h                         C arrays for the CPU oracle
   plonky2_demo_b200/csrc/poseidon_constants.cuh       __constant__ arrays for the CUDA kernels
-      (includes the derived "lazy partial round" tables, see derive_lazy_tables())
 
 Poseidon parameters are data, not code: they cannot be re-derived (round constants
 come from a seeded RNG run, plonky2/src/bin/generate_constants.rs). The FAST_PARTIAL_*
@@ -368,7 +367,7 @@ def poseidon_dense_partial(params, state):
 
 
 def round_addends(params):
-    """Unified per-round additive constants for the GPU's single round loop (csrc/poseidon.cuh):
+    """Unified per-round additive constants (csrc/poseidon.cuh: full_round, and the exit of the partial rounds):
         s += RC[0]; for r in 0..29: { s-box (all lanes if full round else lane 0); s = M s + ADD[r] }
     ADD[r] is the constant the NEXT s-box layer needs, moved behind the linear layer:
       r = 0..2   : RC[r+1]
@@ -415,7 +414,7 @@ def poseidon_unified(params, add, state):
 
 
 def mds_network(circ, s):
-    """Add/shift network for y_r = sum_i circ[i] * s[(r+i) % 12] on integers (csrc/poseidon.cuh:mds_half).
+    """Add/shift network for y_r = sum_i circ[i] * s[(r+i) % 12] on integers (csrc/poseidon.cuh:mds_half_fp64).
     x^12 - 1 = prod_{zeta^4=1} (x^3 - zeta): 4-point DFTs of the three stride-3 subsequences, one
     zeta-twisted 3x3 product per frequency, inverse DFTs.  The frequency-domain constants are
     derived here from `circ` (not copied): K = DFT4(c')(1)/4, N = DFT4(c')(-1)/4, Z = DFT4(c')(i)/2."""
@@ -461,7 +460,7 @@ def c_array(name, vals, per_line=4, ctype="uint64_t", qual="static const"):
     return "\n".join(out)
 
 
-def write_headers(params, C, add):
+def write_headers(params, add, root=ROOT):
     banner = (
         "// GENERATED by tests/golden/make_golden.py from tests/golden/poseidon_params.json -- do not edit.\n"
         "// Poseidon-12 / Goldilocks parameters (data, scraped from the reference:\n"
@@ -477,7 +476,7 @@ def write_headers(params, C, add):
     h.append(c_array("FAST_PARTIAL_ROUND_VS", params["fast_partial_round_vs"]))
     h.append(c_array("FAST_PARTIAL_ROUND_W_HATS", params["fast_partial_round_w_hats"]))
     h.append(c_array("FAST_PARTIAL_ROUND_INITIAL_MATRIX", params["fast_partial_round_initial_matrix"]))
-    with open(os.path.join(ROOT, "oracle", "poseidon_constants.h"), "w") as f:
+    with open(os.path.join(root, "oracle", "poseidon_constants.h"), "w") as f:
         f.write("\n".join(h) + "\n")
 
     # --- CUDA header ---
@@ -485,33 +484,19 @@ def write_headers(params, C, add):
     h = [banner, "#pragma once", "#include <stdint.h>", ""]
     h.append("namespace pcs { namespace pconst {")
     h.append(c_array("RC", params["all_round_constants"], qual=q))
-    h.append("// ROUND_ADD[12*r + i]: see make_golden.round_addends (constants moved behind the linear layer)")
-    h.append(c_array("ROUND_ADD", [x for row in add for x in row], qual=q))
-    # the same addends split in 32-bit halves and pre-biased as doubles 2^52 + half (bit pattern
-    # 0x43300000_hhhhhhhh): the FP64 MDS network adds them last, which also converts its exact
-    # integer result back to "integer in the mantissa" form for free.
+    # the round addends (round_addends: constants moved behind the linear layer), split in 32-bit halves and
+    # pre-biased as doubles 2^52 + half (bit pattern 0x43300000_hhhhhhhh): the FP64 MDS network adds them last,
+    # which also converts its exact integer result back to "integer in the mantissa" form for free.
     biased = []
     for row in add:
         for x in row:
             biased.append((0x43300000 << 32) | (x & 0xFFFFFFFF))
             biased.append((0x43300000 << 32) | (x >> 32))
-    h.append("// ROUND_ADD_D[24*r + 2*i + {0,1}] = bits of the double 2^52 + {low, high} 32-bit half of ROUND_ADD[12*r + i]")
+    h.append("// ROUND_ADD_D[24*r + 2*i + {0,1}] = bits of the double 2^52 + {low, high} 32-bit half of make_golden.round_addends[r][i]")
     h.append(c_array("ROUND_ADD_D", biased, qual=q))
-    h.append(c_array("FIRST_RC", params["fast_partial_first_round_constant"], qual=q))
     h.append(c_array("PARTIAL_RC", params["fast_partial_round_constants"], qual=q))
-    h.append(c_array("VS", params["fast_partial_round_vs"], qual=q))
-    h.append(c_array("W_HATS", params["fast_partial_round_w_hats"], qual=q))
-    # initial matrix stored TRANSPOSED ([c][r]) so one output lane reads a contiguous row
-    im = params["fast_partial_round_initial_matrix"]
-    imt = [im[r * 11 + c] for c in range(11) for r in range(11)]
-    h.append("// INIT_T[c*11 + r] = FAST_PARTIAL_ROUND_INITIAL_MATRIX[r][c]")
-    h.append(c_array("INIT_T", imt, qual=q))
-    # lazy table: packed lower triangle, row k has k entries at offset k(k-1)/2
-    tri = [C[k][r] for k in range(N_PARTIAL) for r in range(k)]
-    h.append("// LAZY_C[k(k-1)/2 + r] = sum_i W_HATS[k][i]*VS[r][i]  (r<k), see make_golden.derive_lazy_tables")
-    h.append(c_array("LAZY_C", tri, qual=q))
     h.append("}}  // namespace pcs::pconst")
-    with open(os.path.join(ROOT, "plonky2_demo_b200", "csrc", "poseidon_constants.cuh"), "w") as f:
+    with open(os.path.join(root, "plonky2_demo_b200", "csrc", "poseidon_constants.cuh"), "w") as f:
         f.write("\n".join(h) + "\n")
 
 
@@ -555,7 +540,7 @@ def main():
         json.dump(params, f, indent=0)
     with open(os.path.join(HERE, "reference_kats.json"), "w") as f:
         json.dump(kat, f, indent=0)
-    write_headers(params, C, add)
+    write_headers(params, add)
     print("golden fixtures + headers written; derived FAST_* tables match the reference")
 
 

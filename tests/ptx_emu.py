@@ -1,6 +1,6 @@
 """A tiny interpreter for the PTX subset used by the inline-asm field arithmetic in csrc/gl64.cuh (integer add / sub with the
 carry flag, 32x32 wide multiplies, shifts, 64-bit packs).  It lets the CPU test-suite check the ALGORITHM of every device
-reduction -- all PCS_REDUCE_FORM variants -- against big-int arithmetic without a GPU (ptxas and the hardware are then
+reduction against big-int arithmetic without a GPU (ptxas and the hardware are then
 covered by the `-m gpu` field-grid and Poseidon KAT tests).  Test infrastructure only."""
 import re
 import subprocess
@@ -9,7 +9,7 @@ M32, M64 = (1 << 32) - 1, (1 << 64) - 1
 
 
 def preprocess(path, defines):
-    """Run the C preprocessor over a header so that #if PCS_REDUCE_FORM ... picks one variant."""
+    """Run the C preprocessor over a header (comments dropped, `defines` applied) so that only code is left to parse."""
     cmd = ["cpp", "-P", "-x", "c++", "-undef"] + [f"-D{k}={v}" for k, v in defines.items()] + [path]
     return subprocess.run(cmd, capture_output=True, text=True, check=True).stdout
 

@@ -218,7 +218,7 @@ def _loop_bodies(sass, kernel):
 
 
 def test_leaf_hash_kernel_instruction_budget(built_lib):
-    """The reduction forms of csrc/gl64.cuh are chosen for what ptxas makes of them (profiles/r02_forms.md): the compiled
+    """The reductions of csrc/gl64.cuh are written for what ptxas makes of them (profiles/r02_forms.md): the compiled
     leaf-hash kernel must keep the instruction counts the measurements were taken with -- one full Poseidon round in ~1018
     SASS instructions (1255 with the round 1-2 reductions), a partial-round pair in ~568 (610), five IMAD.WIDE per modular
     multiplication, the FP64 MDS network intact, and no spills."""

@@ -30,7 +30,7 @@ def _gpu_count():
 
 # ---------------------------------------------------------------------------------------------
 # K1: GoldilocksField ops on the device vs big-int arithmetic on the reference's input grid
-# (field/src/prime_field_testing.rs:7-17,78-125) -- both 128-bit reductions
+# (field/src/prime_field_testing.rs:7-17,78-125)
 # ---------------------------------------------------------------------------------------------
 def _field_op(op, a, b=None):
     from plonky2_demo_b200 import _ffi
@@ -42,14 +42,14 @@ def _field_op(op, a, b=None):
     return out
 
 
-def test_device_field_grid(pcs):
+def test_device_field_grid_vs_bigint(pcs):
     g = field_grid()
     # the reference's grid is canonical; add the non-canonical representatives the engine must accept (goldilocks_field.rs:33-37)
     g = sorted(set(g + [P, P + 1, P + 9, (1 << 64) - 1, (1 << 64) - 2, (1 << 64) - (1 << 32), 0xFFFFFFFF, 0xFFFFFFFF00000000]))
     a = np.array([x for x in g for _ in g], dtype=np.uint64)
     b = np.array([y for _ in g for y in g], dtype=np.uint64)
     ai, bi = [int(x) for x in a], [int(y) for y in b]
-    ops = {0: lambda x, y: (x + y) % P, 1: lambda x, y: (x - y) % P, 2: lambda x, y: x * y % P, 3: lambda x, y: x * y % P}
+    ops = {0: lambda x, y: (x + y) % P, 1: lambda x, y: (x - y) % P, 2: lambda x, y: x * y % P}
     for op, f in ops.items():
         want = np.array([f(x, y) for x, y in zip(ai, bi)], dtype=np.uint64)
         got = _field_op(op, a, b)
@@ -70,23 +70,26 @@ def test_device_field_grid(pcs):
     for x in (1, 7, P - 1, (1 << 63) + 5, (1 << 64) - 1):
         got = _field_op(8, np.full(192, x, dtype=np.uint64), ks)
         assert np.array_equal(got, np.array([x * pow(2, int(k), P) % P for k in ks], dtype=np.uint64))
+    # 3 names no operation (it was retired without renumbering the others): refused like any unknown op
+    from plonky2_demo_b200 import _ffi
+
+    for op in (3, 9, -1):
+        with pytest.raises(_ffi.PcsError, match=r"pcs error -5: unknown field operation"):
+            _field_op(op, ga, ga)
 
 
-def test_device_field_random_products(pcs):
+def test_device_field_random_products_vs_bigint(pcs):
     rng = np.random.default_rng(5)
     a = rng.integers(0, 1 << 64, size=200_000, dtype=np.uint64)
     b = rng.integers(0, 1 << 64, size=200_000, dtype=np.uint64)
-    want = np.array([int(x) * int(y) % P for x, y in zip(a[:20_000], b[:20_000])], dtype=np.uint64)
-    m, mm = _field_op(2, a, b), _field_op(3, a, b)
-    assert np.array_equal(m[:20_000], want)
-    assert np.array_equal(m, mm)                      # the two reductions agree everywhere
+    want = np.array([int(x) * int(y) % P for x, y in zip(a, b)], dtype=np.uint64)
+    assert np.array_equal(_field_op(2, a, b), want)
     # products whose high limbs stress the borrow / carry fix-ups: (2^32 - 1) * 2^32 multiples, p - 1 squares, tiny * huge
     edge = np.array([0xFFFFFFFF, 0xFFFFFFFF00000000, P - 1, P - 2, 1 << 32, (1 << 32) + 1, (1 << 63), 1, 0, (1 << 64) - 1], dtype=np.uint64)
     ea = np.repeat(edge, edge.size)
     eb = np.tile(edge, edge.size)
     want = np.array([int(x) * int(y) % P for x, y in zip(ea, eb)], dtype=np.uint64)
     assert np.array_equal(_field_op(2, ea, eb), want)
-    assert np.array_equal(_field_op(3, ea, eb), want)
 
 
 # ---------------------------------------------------------------------------------------------

@@ -30,7 +30,7 @@ MG = importlib.util.module_from_spec(_spec)
 _spec.loader.exec_module(MG)
 with open(os.path.join(HERE, "golden", "poseidon_params.json")) as _f:
     PARAMS = json.load(_f)
-ADD = MG.round_addends(PARAMS)                   # ROUND_ADD[r] (ROUND_ADD_D holds its halves as 2^52 + half)
+ADD = MG.round_addends(PARAMS)                   # add[r] (ROUND_ADD_D holds its halves as 2^52 + half)
 RC0 = PARAMS["all_round_constants"][:12]
 PARTIAL_RC = PARAMS["fast_partial_round_constants"]
 M = MG.mds_matrix(PARAMS)
@@ -317,7 +317,7 @@ def crt_forward_int(s):
 
 
 def test_beta_recurrence_matches_direct_partial_rounds():
-    """22 transform-domain rounds with the kernel's constants (PARTIAL_RC after the S-box, ROUND_ADD[25] at the exit)
+    """22 transform-domain rounds with the kernel's constants (PARTIAL_RC after the S-box, ADD[25] at the exit)
     against s_0 = sbox(s_0) + PARTIAL_RC[r]; s = M s, mod p, without the double arithmetic"""
     rnd = random.Random(10)
     inv4 = pow(4, -1, P)
@@ -428,3 +428,15 @@ def test_replay_matches_oracle_on_random_states():
     rnd = random.Random(12)
     states = [[rnd.getrandbits(64) for _ in range(12)] for _ in range(10_000)]
     assert [poseidon_mirror(s) for s in states] == _oracle(states)
+
+
+def test_constant_headers_regenerate_from_params(tmp_path):
+    """Both generated headers (the kernels' __constant__ tables and the oracle's) come out of poseidon_params.json byte
+    for byte, so the constants the kernels and the oracle read are the parameters the golden tests pin."""
+    rels = [("oracle", "poseidon_constants.h"), ("plonky2_demo_b200", "csrc", "poseidon_constants.cuh")]
+    for rel in rels:
+        os.makedirs(os.path.join(tmp_path, *rel[:-1]))
+    MG.write_headers(PARAMS, ADD, root=str(tmp_path))
+    for rel in rels:
+        with open(os.path.join(tmp_path, *rel), "rb") as f, open(os.path.join(HERE, "..", *rel), "rb") as g:
+            assert f.read() == g.read(), os.path.join(*rel)

@@ -1,7 +1,7 @@
-"""CPU check of the device field reductions' ALGORITHMS (csrc/gl64.cuh inline PTX, every PCS_REDUCE_FORM) against big-int
+"""CPU check of the device field reductions' ALGORITHMS (csrc/gl64.cuh inline PTX) against big-int
 arithmetic, through the PTX-subset interpreter in tests/ptx_emu.py.  The reference's reduce128 / reduce96 / add / sub
 (field/src/goldilocks_field.rs:199-274,347-369) and its input grid (prime_field_testing.rs:7-17) are the model; ptxas and the
-hardware are covered by the `-m gpu` tests (test_device_field_grid, Poseidon KATs)."""
+hardware are covered by the `-m gpu` tests (test_device_field_grid_vs_bigint, Poseidon KATs)."""
 import os
 import random
 
@@ -54,42 +54,24 @@ def src(tmp_path_factory):
     return _src(str(tmp_path_factory.mktemp("ptx")))
 
 
-REDUCE128 = ["reduce128_limbs", "reduce128_limbs_sub", "reduce128_wide", "reduce128_mad"]   # forms 0, 1, 2 and the NTT's
+def test_reduce128(src):
+    red = E.extract_asm(src, "reduce128")
 
+    def reduce128(lo, hi):
+        return E.run_asm(*red, {"lo": lo, "r2": hi & M32, "r3": hi >> 32})["z"]
 
-def _reduce128(src, func, lo, hi):
-    a = E.extract_asm(src, func)
-    if func == "reduce128_wide":
-        return E.run_asm(*a, {"lo": lo, "r2": hi & M32, "r3": hi >> 32})["z"]
-    if func == "reduce128_mad":
-        env = E.run_asm(*a, {"q0": lo & M32, "q1": lo >> 32, "q2": hi & M32, "q3": hi >> 32})
-        return env["x0"] | (env["x1"] << 32)
-    env = E.run_asm(*a, {"r0": lo & M32, "r1": lo >> 32, "r2": hi & M32, "r3": hi >> 32})
-    return env["r0"] | (env["r1"] << 32)
-
-
-@pytest.mark.parametrize("func", REDUCE128)
-def test_reduce128_every_form(src, func):
     rng = random.Random(0xC0FFEE)
     grid = _grid64()
     pairs = [(a, b) for a in grid for b in grid[::37]] + [(a, b) for a in grid[::53] for b in grid]
     pairs += list(zip(_rand64(rng, 2500), _rand64(rng, 2500)))
     for a, b in pairs:                               # every 128-bit value a product of two u64 can take ...
         q = a * b
-        r = _reduce128(src, func, q & M64, q >> 64)
-        assert 0 <= r <= M64 and r % P == q % P, (func, hex(a), hex(b), hex(r))
+        r = reduce128(q & M64, q >> 64)
+        assert 0 <= r <= M64 and r % P == q % P, (hex(a), hex(b), hex(r))
     for lo, hi in [(0, M64), (M64, M64), (0, M32 << 32), (M32, M32), (0, M32), (M64, 0), (1, 1 << 32), (M64, M32)] + \
                   list(zip(_rand64(rng, 1000), _rand64(rng, 1000))):     # ... and arbitrary limbs (the reduction accepts any)
-        r = _reduce128(src, func, lo, hi)
-        assert 0 <= r <= M64 and r % P == (lo + (hi << 64)) % P, (func, hex(lo), hex(hi), hex(r))
-
-
-def test_dispatch_macros(src):
-    # the dispatchers pick the forms by macro; the default build uses the forms the header documents
-    hdr = open(HDR).read()
-    for m in ("PCS_REDUCE_FORM", "PCS_SQR_FORM", "PCS_FOLD_FORM"):
-        assert f"#ifndef {m}" in hdr
-    assert "reduce128_form<PCS_REDUCE_FORM>" in hdr and "reduce128_form<PCS_SQR_FORM>" in hdr
+        r = reduce128(lo, hi)
+        assert 0 <= r <= M64 and r % P == (lo + (hi << 64)) % P, (hex(lo), hex(hi), hex(r))
 
 
 def test_reduce96(src):
@@ -102,11 +84,9 @@ def test_reduce96(src):
         assert r % P == (x + (top << 64)) % P
 
 
-@pytest.mark.parametrize("func", ["fold_halves_biased_limbs", "fold_halves_biased_limbs_sub", "fold_halves_biased_wide",
-                                  "fold_halves_biased_oneway"])
-def test_fold_halves_every_form(src, func):
+def test_fold_halves(src):
     rng = random.Random(99)
-    a = E.extract_asm(src, func)
+    a = E.extract_asm(src, "fold_halves_biased")
     c = E.extract_asm(src, "fold_halves")
     # full rounds: L, H < 2^45 (high words < 2^13); partial rounds (fold_d): < 2^52 (high words < 2^20)
     lim = [0, 1, (1 << 13) - 1, 1 << 13, (1 << 20) - 1]
@@ -117,8 +97,8 @@ def test_fold_halves_every_form(src, func):
     for l0, l1, h0, h1 in cases:
         want = (l0 + (l1 << 32) + ((h0 + (h1 << 32)) << 32)) % P          # L + H * 2^32
         env = E.run_asm(*a, {"l0": l0, "l1b": BIAS + l1, "h0": h0, "h1b": BIAS + h1})
-        r = env["z"] if func.endswith("wide") else env["w0"] | (env["w1"] << 32)
-        assert 0 <= r <= M64 and r % P == want, (func, l0, l1, h0, h1)
+        r = env["w0"] | (env["w1"] << 32)
+        assert 0 <= r <= M64 and r % P == want, (l0, l1, h0, h1)
         if l1 + h1 < (1 << 13):                                            # the integer network's fold: (L >> 32) + (H >> 32) < 2^13
             env = E.run_asm(*c, {"l0": l0, "l1": l1, "h0": h0, "h1": h1})
             r = env["w0"] | (env["w1"] << 32)

@@ -1,7 +1,7 @@
 // Experiment (not product): a radix-16 NTT register round with its butterflies on the FP64 pipe, against the integer round the
 // shipped kernel runs (run_stages in ntt.cu).  Question: can the idle FP64 pipe carry the add / sub / shift-twiddle work?
 //
-//   integer round (baseline): 4 constant-geometry stages, per butterfly  t = canon(mul_mad(v, w)); (u + t, u - t)
+//   integer round (baseline): 4 constant-geometry stages, per butterfly  t = canon(mul(v, w)); (u + t, u - t)
 //   FP64 round: x[a] *= g^a (one general multiplication per element), values -> pairs of exact doubles (lo + hi 2^32),
 //               16-point DFT whose twiddles are powers of 2 (2^12 is a primitive 16th root: 2^96 = -1 mod p):
 //               add / sub = 2 DADD each, x 2^e = exact scaling + floor-split (which renormalises), then back to u64.
@@ -133,7 +133,7 @@ __global__ void __launch_bounds__(256, 2) k_round(uint64_t* io, const uint64_t* 
                 uint64_t y[16];
 #pragma unroll
                 for (int j = 0; j < 8; j++) {
-                    const uint64_t tt = gl::canon(gl::mul_mad(x[j + 8], tw[s * 8 + j]));
+                    const uint64_t tt = gl::canon(gl::mul(x[j + 8], tw[s * 8 + j]));
                     y[2 * j] = gl::add_lc(x[j], tt);
                     y[2 * j + 1] = gl::sub_lc(x[j], tt);
                 }
@@ -142,7 +142,7 @@ __global__ void __launch_bounds__(256, 2) k_round(uint64_t* io, const uint64_t* 
             }
         } else {
 #pragma unroll
-            for (int a = 1; a < 16; a++) x[a] = gl::mul_mad(x[a], tw[32 + a]);      // pre-scale by g^a
+            for (int a = 1; a < 16; a++) x[a] = gl::mul(x[a], tw[32 + a]);      // pre-scale by g^a
             if (MODE == 1) {
                 D2 d[16];
 #pragma unroll

@@ -1,5 +1,5 @@
 // Times the Poseidon-12 permutation device function in isolation (17 chained permutations per
-// thread, like one 135-element leaf).  Build with different -D flags to compare variants:
+// thread, like one 135-element leaf).  -DTHREADS / -DMINBLOCKS set the launch bounds:
 //   nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -I plonky2_demo_b200/csrc -o pb tools/poseidon_bench.cu
 #include <cstdio>
 #include <cstdint>

@@ -1,5 +1,6 @@
-"""SHA-256 of a library's SASS listing (cuobjdump -sass, instruction text only: no encodings, so two builds of the same
-sources compare equal even though nvcc's temporary-file names differ).  Used to show that the in-tree libpcs.so is, instruction
+"""SHA-256 of a library's SASS listing (cuobjdump -sass, instruction text only: no encodings, and the anonymous-namespace
+hash that nvcc derives from the source path is masked in function names, so two builds of the same sources compare equal
+even at different paths and with different temporary-file names).  Used to show that the in-tree libpcs.so is, instruction
 for instruction, the binary a GPU run tested (profiles/r02_forms.md).
 
     python tools/sass_fingerprint.py [path/to/libpcs.so]
@@ -19,7 +20,7 @@ def fingerprint(lib):
     for line in out.split("\n"):
         m = re.search(r"Function : (\S+)", line)
         if m:
-            h.update(("F " + m.group(1) + "\n").encode())
+            h.update(("F " + re.sub(r"_GLOBAL__N__[0-9a-f]+_", "_GLOBAL__N__", m.group(1)) + "\n").encode())
             continue
         m = re.match(r"\s*/\*([0-9a-f]{4,6})\*/\s+(.*?);", line)
         if m:
