@@ -332,6 +332,32 @@ PCS_API int pcs_fri_commit_layer(const pcs_ext_poly* p, unsigned rate_bits, uint
  * (i+1)*arity], beta) = sum_j beta^j coeffs[i*arity + j] (plonk_common.rs:116-128); len /= 2^arity_bits.            */
 PCS_API int pcs_fri_fold(pcs_ext_poly* p, unsigned arity_bits, const uint64_t beta[2]);
 
+/* ---- the permutation argument between commitments #1 and #2 of prove() ---------------------------------------------------
+ * all_wires_permutation_partial_products (plonk/prover.rs): for every challenge c, wires_permutation_partial_products_and_zs
+ * (plonk/prover.rs) with beta = betas[c], gamma = gammas[c], n = 2^lg_n rows at x_i = w^i (w = primitive_root_of_unity(lg_n)),
+ * R = num_routed_wires, D = quotient_degree_factor, K = ceil(R / D) chunks of wires [kD, min((k+1)D, R)), P = K - 1:
+ *     q_j(i) = (wires[j][i] + beta k_is[j] x_i + gamma) / (wires[j][i] + beta sigmas[j][i] + gamma)
+ *     Q_k(i) = prod of q_j(i) over chunk k                           quotient_chunk_products (util/partial_products.rs)
+ *     Z(x_0) = 1,  Z(x_{i+1}) = Z(x_i) Q_0(i) .. Q_{K-1}(i),  pp_k(x_i) = Z(x_i) Q_0(i) .. Q_k(i), k < P
+ *                                                                    partial_products_and_z_gx + its swap (prover.rs)
+ * k_is = get_unique_coset_shifts(n, R) (field/src/cosets.rs), sigmas[j] = the j-th sigma polynomial's values
+ * (prover_data.sigmas[i][j] = sigmas[j][i]).
+ *   wires, sigmas : R pointers to n values each; HOST pointers, or with PCS_DEVICE_PTRS device pointers on the current
+ *                   context's device (contiguous or scattered; read, never written)
+ *   k_is [R], betas [C], gammas [C] : host arrays, always
+ *   out           : C (1 + P) pointers to n values each, in the order of prove()'s commitment #2: Z of challenge 0 .. C-1,
+ *                   then the partial products challenge-major (out[C + c P + k] = pp_k of challenge c), as
+ *                   PlonkOpeningShape zs_range / partial_products_range; host pointers, or device pointers with
+ *                   PCS_DEVICE_PTRS
+ * Any u64 is accepted as input; every output is canonical.  Synchronous: it reads back one device flag, and a zero
+ * denominator returns PCS_ERR_ARG "Tried to invert zero" (batch_multiplicative_inverse; the outputs are then undefined).
+ * quotient_degree_factor < 2, num_routed_wires == 0, num_challenges == 0 or a NULL pointer: PCS_ERR_ARG;
+ * lg_n > 32: PCS_ERR_TWO_ADICITY.  The context stays usable after every error.                                          */
+PCS_API int pcs_permutation_partial_products(const uint64_t* const* wires, const uint64_t* const* sigmas, size_t num_routed_wires,
+                                     unsigned lg_n, const uint64_t* k_is, const uint64_t* betas, const uint64_t* gammas,
+                                     size_t num_challenges, unsigned quotient_degree_factor, unsigned flags,
+                                     uint64_t* const* out);
+
 #ifdef __cplusplus
 }
 #endif

@@ -11,6 +11,7 @@ Names, argument meaning and error behaviour follow the reference:
     FriConfig / FriParams                 plonky2/src/fri/mod.rs:19-103
     PolynomialBatch                       plonky2/src/fri/oracle.rs:30-159 (+ prove_openings :162-219)
     Challenger                            plonky2/src/iop/challenger.rs:16-160
+    permutation Zs / partial products     plonky2/src/plonk/prover.rs (all_wires_permutation_partial_products)
     FriInstanceInfo / FriProof            plonky2/src/fri/structure.rs, fri/proof.rs
     Buffer (write_/read_polynomial_batch, _merkle_tree, _fri_proof)   plonky2/src/util/serialization/mod.rs
     PoseidonGoldilocksConfig              plonky2/src/plonk/config.rs:101-108
@@ -44,6 +45,12 @@ from .hashing import (  # noqa: F401
     PoseidonPermutation,
     verify_merkle_proof_to_cap,
 )
+from .permutation import (  # noqa: F401
+    all_wires_permutation_partial_products,
+    get_unique_coset_shifts,
+    wires_permutation_partial_products_and_zs,
+    zs_partial_products_values,
+)
 from .polynomial import (  # noqa: F401
     GOLDILOCKS_ORDER,
     PolynomialCoeffs,
@@ -62,5 +69,7 @@ __all__ = [
     "FriConfig", "FriParams", "FriReductionStrategy", "PoseidonGoldilocksConfig", "PoseidonHash",
     "PoseidonPermutation", "HashOut", "CircuitConfig", "fft_with_options", "ifft_with_options",
     "verify_merkle_proof_to_cap", "Challenger", "FriInstanceInfo", "FriBatchInfo", "FriPolynomialInfo", "FriOracleInfo",
-    "FriProof", "OpeningSet", "PlonkOpeningShape", "ExtensionPolynomial", "eval_commitment", "prove_openings", "init", "shutdown", "synchronize", "PcsError",
+    "FriProof", "OpeningSet", "PlonkOpeningShape", "ExtensionPolynomial", "eval_commitment", "prove_openings",
+    "get_unique_coset_shifts", "wires_permutation_partial_products_and_zs", "all_wires_permutation_partial_products",
+    "zs_partial_products_values", "init", "shutdown", "synchronize", "PcsError",
 ]

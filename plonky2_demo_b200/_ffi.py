@@ -88,6 +88,8 @@ SIGNATURES = {
     "pcs_ext_coset_lde": (C.c_int, [C.c_void_p, C.c_uint, C.c_uint64, u64p]),
     "pcs_fri_commit_layer": (C.c_int, [C.c_void_p, C.c_uint, C.c_uint64, C.c_uint, C.c_uint, u64p, C.POINTER(C.c_void_p)]),
     "pcs_fri_fold": (C.c_int, [C.c_void_p, C.c_uint, u64p]),
+    # the permutation argument's Zs and partial products
+    "pcs_permutation_partial_products": (C.c_int, [u64pp, u64pp, sz, C.c_uint, u64p, u64p, u64p, sz, C.c_uint, C.c_uint, u64pp]),
 }
 
 _lib = None

@@ -568,11 +568,6 @@ static void* pinned(void*& buf, size_t& cap, size_t bytes) {
     return buf;
 }
 
-// Device -> pageable host memory: D2H into one of two pinned buffers, then a multi-threaded copy into the caller's memory
-// (fresh Vecs / numpy arrays fault their pages on first touch: one thread moves ~5 GB/s, four ~15) while the next piece is
-// already crossing PCIe.  Synchronises the stream.
-static int d2h_pageable(void* dst, const void* src_dev, size_t bytes, cudaStream_t st);
-
 constexpr size_t RING_SLOT_BYTES = 16u << 20;
 constexpr unsigned STAGE_THREADS = 4;
 
@@ -686,7 +681,10 @@ static void host_copy_mt(char* dst, const char* src, size_t bytes) {
     for (unsigned t = 0; t < nt; t++) th[t].join();
 }
 
-static int d2h_pageable(void* dst, const void* src_dev, size_t bytes, cudaStream_t st) {
+// Device -> pageable host memory: D2H into one of two pinned buffers, then a multi-threaded copy into the caller's memory
+// (fresh Vecs / numpy arrays fault their pages on first touch: one thread moves ~5 GB/s, four ~15) while the next piece is
+// already crossing PCIe.  Synchronises the stream.
+int pcs::d2h_pageable(void* dst, const void* src_dev, size_t bytes, cudaStream_t st) {
     const size_t PIECE = 16u << 20;
     if (bytes <= (1u << 20) || !is_pageable_host(dst)) {
         PCS_CUDA(cudaMemcpyAsync(dst, src_dev, bytes, cudaMemcpyDeviceToHost, st));

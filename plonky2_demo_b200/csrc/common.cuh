@@ -70,6 +70,8 @@ static inline int check_shift(uint64_t shift) {   // a coset shift must be a uni
 // host polynomials (pageable memory) -> contiguous device block through the current context's pinned ring (api.cu)
 int stage_pageable(const uint64_t* const* polys, size_t count, size_t d, uint64_t* dst, cudaStream_t copy_st);
 bool is_pageable_host(const void* p);         // not page-locked or registered: plain copies stage through the driver (api.cu)
+// device -> host memory of any kind (pageable: through two pinned pieces and host threads); synchronises st (api.cu)
+int d2h_pageable(void* dst, const void* src_dev, size_t bytes, cudaStream_t st);
 void multi_shutdown_locked();                 // multi.cu: release the multi-GPU state (called by pcs_shutdown)
 pcs_batch* batch_new();                       // a batch bound to the calling thread's current context (api.cu)
 struct BatchFree {
