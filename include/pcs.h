@@ -358,6 +358,40 @@ PCS_API int pcs_permutation_partial_products(const uint64_t* const* wires, const
                                      size_t num_challenges, unsigned quotient_degree_factor, unsigned flags,
                                      uint64_t* const* out);
 
+/* ---- the quotient polynomials between commitments #2 and #3 of prove() ------------------------------------------------------
+ * compute_quotient_polys (plonk/prover.rs:576-744) without the gate constraints, followed by prove()'s trim_to_len(D n) and
+ * chunks(n): the C D polynomials prove() commits as #3 (all_quotient_poly_chunks).  With n = 2^lg_d of the batches,
+ * q = log2_ceil(D), D = quotient_degree_factor, R = num_routed_wires, C = num_challenges, K = ceil(R / D), P = K - 1, at every
+ * point x_i = 7 w^i of the size-n 2^q domain (w = primitive_root_of_unity(lg_d + q)):
+ *     terms = [L_0(x)(Z_c(x) - 1) for c < C]                                    L_0 = ZeroPolyOnCoset::eval_l_0
+ *           ++ [check_partial_products(num_c, den_c, pp_c, Z_c(x), Z_c(g x), D) for c < C]   (K terms each, util/partial_products.rs)
+ *     num_j = w_j + beta_c k_is[j] x + gamma_c,  den_j = w_j + beta_c sigma_j + gamma_c
+ *     quotient_a(x_i) = (sum_t terms_t alpha_a^t + alpha_a^(C (P + 2)) gate_terms[a][i]) / Z_H(x_i)    reduce_with_powers_multi
+ * then coset_ifft(7) of each of the C value vectors, coefficients [D n, n 2^q) checked to be zero and the first D n split into
+ * D chunks of n.  The LDE rows of the three batches are read in place (leaves [0, n 2^q) = the quotient domain):
+ *   constants_sigmas     : prover_data.constants_sigmas_commitment; sigma j = polynomial num_constants + j
+ *   wires                : commitment #1; wire j = polynomial j (j < R; wider batches are fine)
+ *   zs_partial_products  : commitment #2 in pcs_permutation_partial_products' output order: Z_c = polynomial c,
+ *                          pp_{c,k} = polynomial C + c P + k
+ * Other polynomials and the salt columns are not read.  All three must be resident, whole batches of the same context, degree
+ * and rate (committed without PCS_LDE_ON_DEMAND, not shards or pcs_multi_* shards).
+ *   k_is [R], betas [C], gammas [C], alphas [C] : host arrays, always (any u64)
+ *   gate_terms : NULL (zero), or C columns of n 2^q values in NATURAL order of the quotient domain: column a holds, at point i,
+ *                the alpha_a-reduced remainder of the vanishing terms sum_j constraint_j(x_i) alpha_a^j -- the gate constraints
+ *                (evaluate_gate_constraints_base_batch), preceded by any lookup terms the circuit has, i.e. what
+ *                reduce_with_powers_multi reduces after the permutation terms, restarted at alpha^0.  Any u64.
+ *   out        : C D pointers to n coefficients each, alpha-major (out[a D + k] = chunk k of quotient polynomial a).
+ * gate_terms and out are host pointers (pageable or pinned), or device pointers on the batches' device with PCS_DEVICE_PTRS;
+ * every output is canonical.  Synchronous: it reads back the trim check.  PCS_ERR_ARG (the context stays usable): NULL
+ * pointers, D < 2, R == 0, C == 0, q > rate_bits ("Having constraints of degree higher than the rate is not supported yet"),
+ * batches of different contexts, degrees or rates, a column range beyond its batch, an on-demand, shard or rows-only batch,
+ * and a failed trim ("Quotient has failed, the vanishing polynomial is not divisible by Z_H"; the outputs are then undefined). */
+PCS_API int pcs_quotient_polys(const pcs_batch* constants_sigmas, const pcs_batch* wires, const pcs_batch* zs_partial_products,
+                               size_t num_constants, size_t num_routed_wires, const uint64_t* k_is, const uint64_t* betas,
+                               const uint64_t* gammas, const uint64_t* alphas, size_t num_challenges,
+                               unsigned quotient_degree_factor, const uint64_t* const* gate_terms, unsigned flags,
+                               uint64_t* const* out);
+
 #ifdef __cplusplus
 }
 #endif

@@ -90,6 +90,9 @@ SIGNATURES = {
     "pcs_fri_fold": (C.c_int, [C.c_void_p, C.c_uint, u64p]),
     # the permutation argument's Zs and partial products
     "pcs_permutation_partial_products": (C.c_int, [u64pp, u64pp, sz, C.c_uint, u64p, u64p, u64p, sz, C.c_uint, C.c_uint, u64pp]),
+    # the quotient polynomials
+    "pcs_quotient_polys": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, sz, sz, u64p, u64p, u64p, u64p, sz, C.c_uint, u64pp,
+                                     C.c_uint, u64pp]),
 }
 
 _lib = None

@@ -492,7 +492,7 @@ static uint64_t host_inverse(uint64_t a) {  // a^(p-2) mod p
 }
 
 // coset_ifft in place on the device: values on shift * <w_n>, natural order -> coefficients
-static int coset_intt_dev(uint64_t* values, size_t w, unsigned lg_n, uint64_t shift, cudaStream_t st) {
+int pcs::coset_intt_dev(uint64_t* values, size_t w, unsigned lg_n, uint64_t shift, cudaStream_t st) {
     const size_t n = (size_t)1 << lg_n;
     if (int rc = ntt_dev(values, w, lg_n, true, st)) return rc;
     PCS_CUDA(launch_mul_powers(values, n, w, n, host_inverse(shift), st));   // c_i *= shift^-i  (mod.rs:68-72)

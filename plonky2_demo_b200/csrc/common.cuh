@@ -8,6 +8,7 @@
 #include <string>
 #include <vector>
 
+#include "gl64.cuh"
 #include "pcs.h"
 
 // Device-resident PolynomialBatch / MerkleTree (opaque in pcs.h)
@@ -72,6 +73,33 @@ int stage_pageable(const uint64_t* const* polys, size_t count, size_t d, uint64_
 bool is_pageable_host(const void* p);         // not page-locked or registered: plain copies stage through the driver (api.cu)
 // device -> host memory of any kind (pageable: through two pinned pieces and host threads); synchronises st (api.cu)
 int d2h_pageable(void* dst, const void* src_dev, size_t bytes, cudaStream_t st);
+// PolynomialValues::coset_ifft(shift) in place on a device matrix [w][2^lg_n], natural order in and out, asynchronous (api.cu)
+int coset_intt_dev(uint64_t* values, size_t w, unsigned lg_n, uint64_t shift, cudaStream_t st);
+// out[i] = base^i, i < n, canonical (permutation.cu)
+cudaError_t launch_pow_table(uint64_t base, size_t n, uint64_t* out, cudaStream_t st);
+struct DevBuf;
+// host column pointers -> a device table of them, stream-ordered (permutation.cu)
+int upload_table(const void* ptrs, size_t count, DevBuf& buf, cudaStream_t st);
+// host columns (R pointers, n values each, pageable or pinned) -> contiguous device block dst [R][n] (permutation.cu)
+int stage_host_columns(const uint64_t* const* cols, size_t R, size_t n, uint64_t* dst, cudaStream_t st);
+
+// a^(p-2) in the field: 64 squarings and 9 multiplications.  p - 2 = (2^31 - 1) 2^33 + (2^32 - 1).
+__device__ __forceinline__ uint64_t sqr_n(uint64_t a, int n) {
+    for (int i = 0; i < n; i++) a = gl::sqr(a);
+    return a;
+}
+__device__ __forceinline__ uint64_t inverse(uint64_t a) {
+    const uint64_t t2 = gl::mul(gl::sqr(a), a);         // a^(2^2 - 1)
+    const uint64_t t3 = gl::mul(gl::sqr(t2), a);        // a^(2^3 - 1)
+    const uint64_t t6 = gl::mul(sqr_n(t3, 3), t3);
+    const uint64_t t12 = gl::mul(sqr_n(t6, 6), t6);
+    const uint64_t t24 = gl::mul(sqr_n(t12, 12), t12);
+    const uint64_t t30 = gl::mul(sqr_n(t24, 6), t6);
+    const uint64_t t31 = gl::mul(gl::sqr(t30), a);
+    const uint64_t t32 = gl::mul(gl::sqr(t31), a);
+    return gl::mul(sqr_n(t31, 33), t32);
+}
+
 void multi_shutdown_locked();                 // multi.cu: release the multi-GPU state (called by pcs_shutdown)
 pcs_batch* batch_new();                       // a batch bound to the calling thread's current context (api.cu)
 struct BatchFree {

@@ -33,23 +33,6 @@ constexpr int SCAN_THREADS = 256, SCAN_ITEMS = 16, SCAN_TILE = SCAN_THREADS * SC
 constexpr int PART_THREADS = 1024;
 constexpr unsigned X_LO_BITS = 10;               // x_i = x_hi[i >> 10] * x_lo[i & 1023]
 
-// a^(p-2): 64 squarings and 9 multiplications.  p - 2 = (2^31 - 1) 2^33 + (2^32 - 1).
-__device__ __forceinline__ uint64_t sqr_n(uint64_t a, int n) {
-    for (int i = 0; i < n; i++) a = gl::sqr(a);
-    return a;
-}
-__device__ __forceinline__ uint64_t inverse(uint64_t a) {
-    const uint64_t t2 = gl::mul(gl::sqr(a), a);         // a^(2^2 - 1)
-    const uint64_t t3 = gl::mul(gl::sqr(t2), a);        // a^(2^3 - 1)
-    const uint64_t t6 = gl::mul(sqr_n(t3, 3), t3);
-    const uint64_t t12 = gl::mul(sqr_n(t6, 6), t6);
-    const uint64_t t24 = gl::mul(sqr_n(t12, 12), t12);
-    const uint64_t t30 = gl::mul(sqr_n(t24, 6), t6);
-    const uint64_t t31 = gl::mul(gl::sqr(t30), a);
-    const uint64_t t32 = gl::mul(gl::sqr(t31), a);
-    return gl::mul(sqr_n(t31, 33), t32);
-}
-
 // out[i] = base^i, i < n (canonical)
 __global__ void k_pow_table(uint64_t base, size_t n, uint64_t* out) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -244,21 +227,25 @@ cudaError_t launch_rows(int threads, size_t smem, const uint64_t* const* wires, 
     return cudaGetLastError();
 }
 
-// column pointers -> a device table (stream-ordered)
-int upload_table(const void* ptrs, size_t count, DevBuf& buf, cudaStream_t st) {
+}  // namespace
+
+cudaError_t pcs::launch_pow_table(uint64_t base, size_t n, uint64_t* out, cudaStream_t st) {
+    if (n == 0) return cudaSuccess;
+    k_pow_table<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(base, n, out);
+    return cudaGetLastError();
+}
+
+int pcs::upload_table(const void* ptrs, size_t count, DevBuf& buf, cudaStream_t st) {
     PCS_CUDA(buf.alloc(count * sizeof(uint64_t*), st));
     PCS_CUDA(cudaMemcpyAsync(buf.p, ptrs, count * sizeof(uint64_t*), cudaMemcpyHostToDevice, st));
     return PCS_OK;
 }
 
-// host columns (R pointers, n values each) -> contiguous device block dst [R][n]
-int stage_host_columns(const uint64_t* const* cols, size_t R, size_t n, uint64_t* dst, cudaStream_t st) {
+int pcs::stage_host_columns(const uint64_t* const* cols, size_t R, size_t n, uint64_t* dst, cudaStream_t st) {
     if (is_pageable_host(cols[0])) return stage_pageable(cols, R, n, dst, st);
     for (size_t j = 0; j < R; j++) PCS_CUDA(cudaMemcpyAsync(dst + j * n, cols[j], n * 8, cudaMemcpyHostToDevice, st));
     return PCS_OK;
 }
-
-}  // namespace
 
 extern "C" {
 
@@ -307,10 +294,8 @@ int pcs_permutation_partial_products(const uint64_t* const* wires, const uint64_
     PCS_CUDA(xt.alloc((n_lo + n_hi) * 8, st));
     PCS_CUDA(cb.alloc(consts.size() * 8, st));
     PCS_CUDA(cudaMemcpyAsync(cb.p, consts.data(), consts.size() * 8, cudaMemcpyHostToDevice, st));
-    k_pow_table<<<(unsigned)((n_lo + 255) / 256), 256, 0, st>>>(omega, n_lo, xt.u64());
-    PCS_CUDA(cudaGetLastError());
-    k_pow_table<<<(unsigned)((n_hi + 255) / 256), 256, 0, st>>>(glh::powmod(omega, n_lo), n_hi, xt.u64() + n_lo);
-    PCS_CUDA(cudaGetLastError());
+    PCS_CUDA(launch_pow_table(omega, n_lo, xt.u64(), st));
+    PCS_CUDA(launch_pow_table(glh::powmod(omega, n_lo), n_hi, xt.u64() + n_lo, st));
     PCS_CUDA(flag.alloc(sizeof(unsigned), st));
     PCS_CUDA(cudaMemsetAsync(flag.p, 0, sizeof(unsigned), st));
 
