@@ -392,6 +392,45 @@ PCS_API int pcs_quotient_polys(const pcs_batch* constants_sigmas, const pcs_batc
                                unsigned quotient_degree_factor, const uint64_t* const* gate_terms, unsigned flags,
                                uint64_t* const* out);
 
+/* ---- the gate constraints of the quotient step ------------------------------------------------------------------------------
+ * The gate-constraint tail of compute_quotient_polys (plonk/prover.rs:576-744): evaluate_gate_constraints_base_batch
+ * (plonk/vanishing_poly.rs) at every point x_i = 7 w^i, i < M = n 2^q, of the quotient domain, reduced with powers of each
+ * alpha:  out[a][i] = sum_j constraint_j(x_i) alphas[a]^j.  That is exactly pcs_quotient_polys' gate_terms, so the two chain on
+ * the device.  Slot j of the constraints sums constraint j of every gate g times its filter
+ *     compute_filter(g, groups[sel_g], s = local_constants[sel_g], num_selectors > 1)
+ *       = prod_{i in [start, end), i != g} (i - s) * (num_selectors > 1 ? (2^32 - 1) - s : 1);
+ * the gates read local_constants[num_selectors + k] and local_wires[k] (wire k = wires polynomial k).  The gates:
+ *     PCS_GATE_NOOP          NoopGate                      no constraint
+ *     PCS_GATE_CONSTANT      ConstantGate { num_consts }    c[k] - w[k], k < param
+ *     PCS_GATE_PUBLIC_INPUT  PublicInputGate               w[k] - public_inputs_hash[k], k < 4
+ *     PCS_GATE_ARITHMETIC    ArithmeticGate { num_ops }     w[4i+3] - (w[4i] w[4i+1] c[0] + w[4i+2] c[1]), i < param
+ *     PCS_GATE_POSEIDON      PoseidonGate                  the 123 constraints of gates/poseidon.rs over 135 wires
+ *   gates           : [num_gates][3] = { kind, param (num_consts / num_ops, else unused), selector_index }, in common_data.gates
+ *                     order
+ *   selector_groups : [num_selectors][2] = selectors_info.groups as [start, end) gate ranges
+ *   public_inputs_hash [4], alphas [C] : host arrays (any u64)
+ *   out             : C columns of M values in NATURAL order of the quotient domain, host pointers or, with PCS_DEVICE_PTRS,
+ *                     device pointers on the batches' device; every output is canonical.
+ * The LDE rows of constants_sigmas (constant k = polynomial k) and wires are read in place; both must be resident, whole,
+ * committed batches of the same context, degree and rate.  Synchronous for host outputs, asynchronous on pcs_stream() for device
+ * outputs.  PCS_ERR_ARG (the context stays usable): NULL pointers, C == 0, D < 2, q > rate_bits, an unknown gate kind, a
+ * selector_index >= num_selectors, a gate outside its own group, a group that is not a non-empty range in [0, num_gates),
+ * num_lookup_selectors > 0 (lookups are not built), batches too narrow for the gates (PoseidonGate needs 135 wires,
+ * ArithmeticGate num_selectors + 2 constants), batches of different contexts, degrees or rates, and an on-demand, shard or
+ * uncommitted batch. */
+enum {
+    PCS_GATE_NOOP = 0,
+    PCS_GATE_CONSTANT = 1,
+    PCS_GATE_PUBLIC_INPUT = 2,
+    PCS_GATE_ARITHMETIC = 3,
+    PCS_GATE_POSEIDON = 4
+};
+PCS_API int pcs_gate_constraint_terms(const pcs_batch* constants_sigmas, const pcs_batch* wires, const uint32_t* gates,
+                                      size_t num_gates, const size_t* selector_groups, size_t num_selectors,
+                                      size_t num_lookup_selectors, size_t num_constants, const uint64_t* public_inputs_hash,
+                                      const uint64_t* alphas, size_t num_challenges, unsigned quotient_degree_factor,
+                                      unsigned flags, uint64_t* const* out);
+
 #ifdef __cplusplus
 }
 #endif

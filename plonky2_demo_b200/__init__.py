@@ -13,6 +13,7 @@ Names, argument meaning and error behaviour follow the reference:
     Challenger                            plonky2/src/iop/challenger.rs:16-160
     permutation Zs / partial products     plonky2/src/plonk/prover.rs (all_wires_permutation_partial_products)
     quotient polynomials / chunks         plonky2/src/plonk/prover.rs:576-744 (compute_quotient_polys, no gate constraints)
+    gate constraints of the quotient step plonk/vanishing_poly.rs (evaluate_gate_constraints_base_batch), gates/*.rs
     FriInstanceInfo / FriProof            plonky2/src/fri/structure.rs, fri/proof.rs
     Buffer (write_/read_polynomial_batch, _merkle_tree, _fri_proof)   plonky2/src/util/serialization/mod.rs
     PoseidonGoldilocksConfig              plonky2/src/plonk/config.rs:101-108
@@ -52,6 +53,15 @@ from .permutation import (  # noqa: F401
     wires_permutation_partial_products_and_zs,
     zs_partial_products_values,
 )
+from .gates import (  # noqa: F401
+    ArithmeticGate,
+    ConstantGate,
+    NoopGate,
+    PoseidonGate,
+    PublicInputGate,
+    SelectorsInfo,
+    gate_constraint_terms,
+)
 from .quotient import compute_quotient_polys, quotient_poly_chunks  # noqa: F401
 from .polynomial import (  # noqa: F401
     GOLDILOCKS_ORDER,
@@ -73,5 +83,6 @@ __all__ = [
     "verify_merkle_proof_to_cap", "Challenger", "FriInstanceInfo", "FriBatchInfo", "FriPolynomialInfo", "FriOracleInfo",
     "FriProof", "OpeningSet", "PlonkOpeningShape", "ExtensionPolynomial", "eval_commitment", "prove_openings",
     "get_unique_coset_shifts", "wires_permutation_partial_products_and_zs", "all_wires_permutation_partial_products",
-    "zs_partial_products_values", "compute_quotient_polys", "quotient_poly_chunks", "init", "shutdown", "synchronize", "PcsError",
+    "zs_partial_products_values", "compute_quotient_polys", "quotient_poly_chunks", "NoopGate", "ConstantGate", "PublicInputGate", "ArithmeticGate", "PoseidonGate",
+    "SelectorsInfo", "gate_constraint_terms", "init", "shutdown", "synchronize", "PcsError",
 ]

@@ -17,6 +17,13 @@ PCS_KEEP_COEFFS = 2
 PCS_MULTI_CE_GATHER = 4
 PCS_LDE_ON_DEMAND = 8
 
+# gate kinds of pcs_gate_constraint_terms
+PCS_GATE_NOOP = 0
+PCS_GATE_CONSTANT = 1
+PCS_GATE_PUBLIC_INPUT = 2
+PCS_GATE_ARITHMETIC = 3
+PCS_GATE_POSEIDON = 4
+
 # every symbol include/pcs.h declares: name -> (restype, argtypes)
 SIGNATURES = {
     "pcs_init": (C.c_int, [C.c_int, C.c_void_p]),
@@ -93,6 +100,9 @@ SIGNATURES = {
     # the quotient polynomials
     "pcs_quotient_polys": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, sz, sz, u64p, u64p, u64p, u64p, sz, C.c_uint, u64pp,
                                      C.c_uint, u64pp]),
+    # the gate constraints of the quotient step
+    "pcs_gate_constraint_terms": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_uint32), sz, C.POINTER(sz), sz, sz, sz, u64p,
+                                            u64p, sz, C.c_uint, C.c_uint, u64pp]),
 }
 
 _lib = None

@@ -185,6 +185,19 @@ static inline int ilog2_strict(size_t n) {
     while ((n >> r) != 1) r++;
     return r;
 }
+static inline unsigned log2_ceil(size_t v) {
+    unsigned q = 0;
+    while (((size_t)1 << q) < v) q++;
+    return q;
+}
+
+// resident, whole, committed LDE rows (what the quotient-domain kernels read in place), or the reason why not
+static inline const char* unusable(const pcs_batch* b) {
+    if (b->on_demand) return "a PCS_LDE_ON_DEMAND batch keeps no LDE rows";
+    if (b->rows_only || b->coset_first != 0 || b->full_rate_bits != b->rate_bits) return "a shard batch holds part of the LDE";
+    if (!b->lde || !b->committed) return "the batch is not committed";
+    return nullptr;
+}
 
 // ------------------------------------------------------------------------------------------------
 // hash_kernels.cu

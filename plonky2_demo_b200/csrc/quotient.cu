@@ -208,20 +208,6 @@ __global__ void k_trim_check(const uint64_t* __restrict__ vals, size_t M, size_t
     if (i < M && vals[(size_t)blockIdx.y * M + i] != 0) *flag = 1;
 }
 
-unsigned log2_ceil(size_t v) {
-    unsigned q = 0;
-    while (((size_t)1 << q) < v) q++;
-    return q;
-}
-
-// resident, whole, committed LDE rows, or the reason why not
-const char* unusable(const pcs_batch* b) {
-    if (b->on_demand) return "a PCS_LDE_ON_DEMAND batch keeps no LDE rows";
-    if (b->rows_only || b->coset_first != 0 || b->full_rate_bits != b->rate_bits) return "a shard batch holds part of the LDE";
-    if (!b->lde || !b->committed) return "the batch is not committed";
-    return nullptr;
-}
-
 }  // namespace
 
 extern "C" {
