@@ -481,21 +481,11 @@ static int ntt_dev(uint64_t* polys, size_t w, unsigned lg_n, bool inverse, cudaS
     return PCS_OK;
 }
 
-static uint64_t host_inverse(uint64_t a) {  // a^(p-2) mod p
-    const uint64_t P = 0xFFFFFFFF00000001ULL;
-    unsigned __int128 acc = 1, b = a % P;
-    for (uint64_t e = P - 2; e; e >>= 1) {
-        if (e & 1) acc = acc * b % P;
-        b = b * b % P;
-    }
-    return (uint64_t)acc;
-}
-
 // coset_ifft in place on the device: values on shift * <w_n>, natural order -> coefficients
 int pcs::coset_intt_dev(uint64_t* values, size_t w, unsigned lg_n, uint64_t shift, cudaStream_t st) {
     const size_t n = (size_t)1 << lg_n;
     if (int rc = ntt_dev(values, w, lg_n, true, st)) return rc;
-    PCS_CUDA(launch_mul_powers(values, n, w, n, host_inverse(shift), st));   // c_i *= shift^-i  (mod.rs:68-72)
+    PCS_CUDA(launch_mul_powers(values, n, w, n, glh::inverse(shift), st));   // c_i *= shift^-i  (mod.rs:68-72)
     return PCS_OK;
 }
 

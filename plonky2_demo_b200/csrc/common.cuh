@@ -4,8 +4,10 @@
 #include <stddef.h>
 #include <stdint.h>
 
+#include <initializer_list>
 #include <memory>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "gl64.cuh"
@@ -78,8 +80,13 @@ int coset_intt_dev(uint64_t* values, size_t w, unsigned lg_n, uint64_t shift, cu
 // out[i] = base^i, i < n, canonical (permutation.cu)
 cudaError_t launch_pow_table(uint64_t base, size_t n, uint64_t* out, cudaStream_t st);
 struct DevBuf;
-// host column pointers -> a device table of them, stream-ordered (permutation.cu)
-int upload_table(const void* ptrs, size_t count, DevBuf& buf, cudaStream_t st);
+// The points x_i = root^i, i < n, of a subgroup as two tables read by subgroup_point: x_lo = root^j (j < 2^X_LO_BITS) at
+// buf.u64(), x_hi = root^(2^X_LO_BITS j) at buf.u64() + 2^X_LO_BITS, stream-ordered (permutation.cu)
+constexpr unsigned X_LO_BITS = 10;
+int point_tables(uint64_t root, size_t n, DevBuf& buf, cudaStream_t st);
+__device__ __forceinline__ uint64_t subgroup_point(const uint64_t* x_lo, const uint64_t* x_hi, size_t i) {
+    return gl::mul(x_hi[i >> X_LO_BITS], x_lo[i & ((1u << X_LO_BITS) - 1)]);
+}
 // host columns (R pointers, n values each, pageable or pinned) -> contiguous device block dst [R][n] (permutation.cu)
 int stage_host_columns(const uint64_t* const* cols, size_t R, size_t n, uint64_t* dst, cudaStream_t st);
 
@@ -98,6 +105,11 @@ __device__ __forceinline__ uint64_t inverse(uint64_t a) {
     const uint64_t t31 = gl::mul(gl::sqr(t30), a);
     const uint64_t t32 = gl::mul(gl::sqr(t31), a);
     return gl::mul(sqr_n(t31, 33), t32);
+}
+
+// the low `bits` bits of v in reverse order (0 when bits == 0)
+__device__ __forceinline__ size_t brev_bits(size_t v, unsigned bits) {
+    return bits ? (size_t)(__brevll((unsigned long long)v) >> (64 - bits)) : 0;
 }
 
 void multi_shutdown_locked();                 // multi.cu: release the multi-GPU state (called by pcs_shutdown)
@@ -175,6 +187,25 @@ struct DevBuf {
     ~DevBuf() { release(); }
 };
 
+// host array (pointer, constant or gate table) -> a stream-ordered device copy in buf
+template <class T>
+int upload_table(const T* host, size_t count, DevBuf& buf, cudaStream_t st) {
+    PCS_CUDA(buf.alloc(count * sizeof(T), st));
+    PCS_CUDA(cudaMemcpyAsync(buf.p, host, count * sizeof(T), cudaMemcpyHostToDevice, st));
+    return PCS_OK;
+}
+
+// f(std::integral_constant<int, N>()) with N = n for n in 1..4 (4 for larger n): the widths a kernel template is built for
+template <class F>
+cudaError_t dispatch_width(size_t n, F f) {
+    switch (n) {
+        case 1: return f(std::integral_constant<int, 1>());
+        case 2: return f(std::integral_constant<int, 2>());
+        case 3: return f(std::integral_constant<int, 3>());
+        default: return f(std::integral_constant<int, 4>());
+    }
+}
+
 // leaf digests + all node levels of MerkleTree::new over a poly-major matrix cols [width][n] (api.cu)
 int build_tree_dev(const uint64_t* cols, size_t n, size_t width, unsigned lg_n, unsigned cap_height, uint64_t* digests,
                    uint64_t* cap, cudaStream_t st, cudaEvent_t after_leaves);
@@ -185,19 +216,11 @@ static inline int ilog2_strict(size_t n) {
     while ((n >> r) != 1) r++;
     return r;
 }
-static inline unsigned log2_ceil(size_t v) {
-    unsigned q = 0;
-    while (((size_t)1 << q) < v) q++;
-    return q;
-}
-
-// resident, whole, committed LDE rows (what the quotient-domain kernels read in place), or the reason why not
-static inline const char* unusable(const pcs_batch* b) {
-    if (b->on_demand) return "a PCS_LDE_ON_DEMAND batch keeps no LDE rows";
-    if (b->rows_only || b->coset_first != 0 || b->full_rate_bits != b->rate_bits) return "a shard batch holds part of the LDE";
-    if (!b->lde || !b->committed) return "the batch is not committed";
-    return nullptr;
-}
+// The checks shared by the entry points that read committed batches on the quotient domain (quotient.cu, gates.cu), after
+// BatchScope and need_init(): the batches share one context, hold resident committed LDE rows of one degree and rate, and
+// quotient_degree_factor D >= 2 fits the rate; num_challenges C >= 1.  PCS_OK with lg_n = the batches' lg_d and
+// q = log2_ceil(D), or the reference's message and its code (quotient.cu).
+int check_quotient_domain(std::initializer_list<const pcs_batch*> batches, size_t D, size_t C, unsigned& lg_n, unsigned& q);
 
 // ------------------------------------------------------------------------------------------------
 // hash_kernels.cu
@@ -279,3 +302,21 @@ cudaError_t launch_lde_natural(const uint64_t* cols, size_t col_stride, uint32_t
 cudaError_t launch_mul_powers(uint64_t* data, size_t stride, size_t w, size_t n, uint64_t base, cudaStream_t st);
 
 }  // namespace pcs
+
+// ---- host-side base-field arithmetic (setup only: roots, shifts, powers of a few challenges) -------------
+namespace glh {
+constexpr uint64_t P = gl::P;
+static inline uint64_t mulmod(uint64_t a, uint64_t b) { return (uint64_t)((unsigned __int128)a * b % P); }
+static inline uint64_t powmod(uint64_t a, uint64_t e) {
+    uint64_t acc = 1;
+    a %= P;
+    for (; e; e >>= 1) {
+        if (e & 1) acc = mulmod(acc, a);
+        a = mulmod(a, a);
+    }
+    return acc;
+}
+static inline uint64_t inverse(uint64_t a) { return powmod(a, P - 2); }   // a^(p-2)
+// primitive_root_of_unity(lg) = POWER_OF_TWO_GENERATOR^(2^(32 - lg))   types.rs:268-272
+static inline uint64_t primitive_root_of_unity(unsigned lg) { return powmod(1753635133440165772ULL, (uint64_t)1 << (32 - lg)); }
+}  // namespace glh

@@ -7,6 +7,7 @@
 #pragma once
 #include <stdint.h>
 
+#include "common.cuh"
 #include "gl64.cuh"
 
 namespace gl {
@@ -163,23 +164,12 @@ __device__ __forceinline__ ext2 ext_pow(ext2 base, uint64_t e) {
 
 }  // namespace gl
 
-// ---- host-side scalar arithmetic (setup only: points, shifts, powers of a few challenges) -------------
+// ---- host-side extension arithmetic (setup only: powers of a few points and challenges; base field in common.cuh) -------
 namespace glh {
-constexpr uint64_t P = 0xFFFFFFFF00000001ULL;
 struct ext2 {
     uint64_t a, b;
 };
-static inline uint64_t mulmod(uint64_t a, uint64_t b) { return (uint64_t)((unsigned __int128)a * b % P); }
 static inline uint64_t addmod(uint64_t a, uint64_t b) { return (uint64_t)(((unsigned __int128)a + b) % P); }
-static inline uint64_t powmod(uint64_t a, uint64_t e) {
-    uint64_t acc = 1;
-    a %= P;
-    for (; e; e >>= 1) {
-        if (e & 1) acc = mulmod(acc, a);
-        a = mulmod(a, a);
-    }
-    return acc;
-}
 static inline ext2 ext_mul(ext2 x, ext2 y) {
     ext2 r;
     r.a = addmod(mulmod(x.a, y.a), mulmod(7, mulmod(x.b, y.b)));

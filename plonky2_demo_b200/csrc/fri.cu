@@ -57,7 +57,7 @@ __global__ void k_interleave(const uint64_t* in, size_t in_stride, size_t len, u
 __global__ void k_interleave_bitrev(const uint64_t* in, size_t n, unsigned lg_n, uint64_t* out) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) {
-        size_t r = lg_n ? (size_t)(__brevll((unsigned long long)i) >> (64 - lg_n)) : 0;
+        size_t r = brev_bits(i, lg_n);
         out[2 * r] = gl::canon(in[i]);
         out[2 * r + 1] = gl::canon(in[n + i]);
     }

@@ -23,7 +23,6 @@
 #include <vector>
 
 #include "common.cuh"
-#include "ext.cuh"
 #include "gl64.cuh"
 #include "poseidon.cuh"
 
@@ -185,13 +184,6 @@ __global__ void __launch_bounds__(GT_THREADS) k_gate_points(const GateArgs A, un
         if (a < (int)na) A.out[(size_t)(a0 + a) * M + l] = gl::canon(res[a]);
 }
 
-template <int N>
-cudaError_t launch_gate_points(const GateArgs& A, unsigned a0, unsigned na, cudaStream_t st) {
-    const size_t M = (size_t)1 << A.lg_m;
-    k_gate_points<N><<<(unsigned)((M + GT_THREADS - 1) / GT_THREADS), GT_THREADS, 0, st>>>(A, a0, na);
-    return cudaGetLastError();
-}
-
 }  // namespace
 
 extern "C" {
@@ -203,21 +195,13 @@ int pcs_gate_constraint_terms(const pcs_batch* constants_sigmas, const pcs_batch
     const pcs_batch *cs = constants_sigmas, *wb = wires;
     if (!cs || !wb || (num_gates && !gates) || (num_selectors && !selector_groups) || !public_inputs_hash || !alphas || !out)
         return fail(PCS_ERR_ARG, "NULL pointer");
-    if (cs->ctx != wb->ctx) return fail(PCS_ERR_ARG, "the batches belong to different contexts");
     BatchScope scope(cs);
     if (int rc = need_init()) return rc;
     const size_t C = num_challenges, D = quotient_degree_factor, G = num_gates, S = num_selectors;
-    if (D < 2) return fail(PCS_ERR_ARG, "quotient_degree_factor must be at least 2");
-    if (C == 0) return fail(PCS_ERR_ARG, "num_challenges is 0");
+    unsigned lg_n, q;
+    if (int rc = check_quotient_domain({cs, wb}, D, C, lg_n, q)) return rc;
     if (C > 0xFFFFu || G > 0xFFFFu) return fail(PCS_ERR_ARG, "num_challenges or num_gates too large");
     if (num_lookup_selectors) return fail(PCS_ERR_ARG, "lookups are not supported: num_lookup_selectors must be 0");
-    for (const pcs_batch* b : {cs, wb})
-        if (const char* why = unusable(b)) return fail(PCS_ERR_ARG, why);
-    if (wb->lg_d != cs->lg_d || wb->rate_bits != cs->rate_bits) return fail(PCS_ERR_ARG, "the batches differ in degree or rate");
-    const unsigned lg_n = cs->lg_d, q = log2_ceil(D);
-    if (q > cs->rate_bits)   // compute_quotient_polys' assertion
-        return fail(PCS_ERR_ARG, "Having constraints of degree higher than the rate is not supported yet. "
-                                 "quotient_degree_factor " + std::to_string(D) + " needs rate_bits >= " + std::to_string(q));
     if (num_constants > cs->w)
         return fail(PCS_ERR_ARG, "constants_sigmas has " + std::to_string(cs->w) + " polynomials, fewer than num_constants");
     if (S > num_constants) return fail(PCS_ERR_ARG, "num_selectors exceeds num_constants");
@@ -273,10 +257,8 @@ int pcs_gate_constraint_terms(const pcs_batch* constants_sigmas, const pcs_batch
         for (size_t k = 0; k < NK; k++, p = glh::mulmod(p, al)) consts[4 + a * NK + k] = p;
     }
     DevBuf cb, tb, pts, nat;   // released in stream order on every return
-    PCS_CUDA(cb.alloc(consts.size() * 8, st));
-    PCS_CUDA(cudaMemcpyAsync(cb.p, consts.data(), consts.size() * 8, cudaMemcpyHostToDevice, st));
-    PCS_CUDA(tb.alloc(table.size() * 4, st));
-    PCS_CUDA(cudaMemcpyAsync(tb.p, table.data(), table.size() * 4, cudaMemcpyHostToDevice, st));
+    if (int rc = upload_table(consts.data(), consts.size(), cb, st)) return rc;
+    if (int rc = upload_table(table.data(), table.size(), tb, st)) return rc;
 
     // 1. the point kernel, N <= 4 alphas per pass
     PCS_CUDA(pts.alloc(C * M * 8, st));
@@ -291,17 +273,12 @@ int pcs_gate_constraint_terms(const pcs_batch* constants_sigmas, const pcs_batch
     A.apow = cb.u64() + 4;
     A.lg_m = lg_m;
     A.out = pts.u64();
-    const unsigned N = (unsigned)std::min<size_t>(C, MAX_NA);
     for (size_t a0 = 0; a0 < C; a0 += MAX_NA) {
         const unsigned na = (unsigned)std::min<size_t>(C - a0, MAX_NA);
-        cudaError_t e;
-        switch (N) {
-            case 1: e = launch_gate_points<1>(A, (unsigned)a0, na, st); break;
-            case 2: e = launch_gate_points<2>(A, (unsigned)a0, na, st); break;
-            case 3: e = launch_gate_points<3>(A, (unsigned)a0, na, st); break;
-            default: e = launch_gate_points<4>(A, (unsigned)a0, na, st); break;
-        }
-        PCS_CUDA(e);
+        PCS_CUDA(dispatch_width(C, [&](auto N) {
+            k_gate_points<N><<<(unsigned)((M + GT_THREADS - 1) / GT_THREADS), GT_THREADS, 0, st>>>(A, (unsigned)a0, na);
+            return cudaGetLastError();
+        }));
     }
 
     // 2. leaf order -> natural order, straight into device outputs or through one staging block to the host

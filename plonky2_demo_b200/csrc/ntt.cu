@@ -89,20 +89,6 @@ __global__ void k_fill_psi(uint64_t* psi, unsigned nb, uint64_t root_2nb) {
     psi[q] = gl::pow(root_2nb, brev32(q, nb - 1));
 }
 
-static uint64_t h_mul(uint64_t a, uint64_t b) {
-    unsigned __int128 x = (unsigned __int128)a * b;
-    return (uint64_t)(x % gl::P);
-}
-static uint64_t h_pow(uint64_t b, uint64_t e) {
-    uint64_t acc = 1;
-    while (e) {
-        if (e & 1) acc = h_mul(acc, b);
-        b = h_mul(b, b);
-        e >>= 1;
-    }
-    return acc;
-}
-
 // Plan cache: one per CUDA device (twiddle tables live in that device's memory).  The commit path uses a handful of plans
 // (shift 7 and the inverse transform per degree); FRI layer shifts and caller-chosen shifts (pcs_coset_lde, pcs_coset_intt)
 // are arbitrary, so the cache is LRU-bounded.
@@ -143,9 +129,8 @@ NttPlan* ntt_plan_get(unsigned lg_d, unsigned r, bool inverse, uint64_t shift, c
         return p;
     }
     unsigned lg_n = lg_d + r;
-    // primitive_root_of_unity(lg_n) = POWER_OF_TWO_GENERATOR^(2^(32-lg_n))   types.rs:268-272
-    uint64_t root = h_pow(1753635133440165772ULL, 1ULL << (32 - lg_n));
-    if (inverse) root = h_pow(root, gl::P - 2);
+    uint64_t root = glh::primitive_root_of_unity(lg_n);
+    if (inverse) root = glh::inverse(root);
     NttPlan* p = new NttPlan();
     p->lg_d = lg_d;
     p->r = r;
@@ -173,7 +158,7 @@ NttPlan* ntt_plan_get(unsigned lg_d, unsigned r, bool inverse, uint64_t shift, c
         }
         size_t ng = (size_t)1 << gbits;
         k_fill_gamma<<<(unsigned)((ng + 255) / 256), 256, 0, st>>>(ps.gamma, gbits, root, p->shift, ps.L);
-        uint64_t root_2nb = h_pow(root, 1ULL << (lg_n - nb));
+        uint64_t root_2nb = glh::powmod(root, 1ULL << (lg_n - nb));
         size_t nq = (size_t)1 << (nb - 1);
         k_fill_psi<<<(unsigned)((nq + 255) / 256), 256, 0, st>>>(ps.psi, nb, root_2nb);
         s0 += nb;
@@ -538,7 +523,7 @@ __global__ void k_bitrev_permute(const uint64_t* __restrict__ in, size_t in_stri
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     size_t j = blockIdx.y;
     if (i >= ((size_t)1 << lg_n)) return;
-    size_t bi = lg_n ? (size_t)(__brevll((unsigned long long)i) >> (64 - lg_n)) : 0;
+    size_t bi = brev_bits(i, lg_n);
     uint64_t v = in[j * in_stride + i];
     if (scale != 1) v = gl::canon(gl::mul(v, scale));
     out[j * out_stride + bi] = v;
@@ -550,6 +535,7 @@ __global__ void k_bitrev_gather(const uint64_t* __restrict__ in, unsigned lg_n, 
                                 uint64_t* __restrict__ out) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= count) return;
+    // the sum inside the branch: brev_bits(first + i, lg_n) compiles to a select instead of this branch
     size_t src = lg_n ? (size_t)(__brevll((unsigned long long)(first + i)) >> (64 - lg_n)) : 0;
     out[i] = gl::canon(in[src]);
 }
@@ -581,7 +567,7 @@ __global__ void __launch_bounds__(256) k_bitrev_permute_tiled(const uint64_t* __
         t[hi][x] = v;
     }
     __syncthreads();
-    const size_t rmid = m ? (size_t)(__brevll((unsigned long long)mid) >> (64 - m)) : 0;
+    const size_t rmid = brev_bits(mid, m);
     const unsigned hi_src = __brev(x) >> 27;
     for (unsigned lo = threadIdx.y; lo < 32; lo += 8)
         dst[((size_t)(__brev(lo) >> 27) << (m + 5)) | (rmid << 5) | x] = t[hi_src][lo];
@@ -699,7 +685,7 @@ __global__ void __launch_bounds__(256) k_lde_natural(const uint64_t* __restrict_
     const size_t k = (size_t)blockIdx.x * 8 + threadIdx.y;
     if (k >= count) return;
     const size_t idx = (index_start + k) * step;
-    const size_t leaf = lg_n ? (size_t)(__brevll((unsigned long long)idx) >> (64 - lg_n)) : 0;
+    const size_t leaf = brev_bits(idx, lg_n);
     for (uint32_t j = threadIdx.x; j < width; j += 32) out[k * width + j] = __ldg(cols + (size_t)j * col_stride + leaf);
 }
 

@@ -19,7 +19,6 @@
 #include <vector>
 
 #include "common.cuh"
-#include "ext.cuh"
 #include "gl64.cuh"
 
 using namespace pcs;
@@ -31,7 +30,6 @@ constexpr size_t ROW_SMEM_TARGET = 64u << 10;   // per block: several blocks per
 constexpr int MAX_NC = 4;                        // challenges per pass over the inputs
 constexpr int SCAN_THREADS = 256, SCAN_ITEMS = 16, SCAN_TILE = SCAN_THREADS * SCAN_ITEMS;
 constexpr int PART_THREADS = 1024;
-constexpr unsigned X_LO_BITS = 10;               // x_i = x_hi[i >> 10] * x_lo[i & 1023]
 
 // out[i] = base^i, i < n (canonical)
 __global__ void k_pow_table(uint64_t base, size_t n, uint64_t* out) {
@@ -52,7 +50,7 @@ __global__ void __launch_bounds__(ROW_THREADS_MAX) k_perm_rows(
     const unsigned tid = threadIdx.x, bd = blockDim.x;
     const size_t i = (size_t)blockIdx.x * bd + tid;
     if (i >= n) return;
-    const uint64_t x = gl::mul(x_hi[i >> X_LO_BITS], x_lo[i & ((1u << X_LO_BITS) - 1)]);
+    const uint64_t x = subgroup_point(x_lo, x_hi, i);
     uint64_t np[NC], dp[NC], b[NC], g[NC];
 #pragma unroll
     for (int c = 0; c < NC; c++) {
@@ -213,20 +211,6 @@ __global__ void k_mul_z(uint64_t* const* __restrict__ cols, unsigned C, unsigned
     }
 }
 
-template <int NC>
-cudaError_t launch_rows(int threads, size_t smem, const uint64_t* const* wires, const uint64_t* const* sigmas, unsigned R,
-                        unsigned D, unsigned P, size_t n, const uint64_t* x_lo, const uint64_t* x_hi, const uint64_t* bk,
-                        const uint64_t* beta, const uint64_t* gamma, uint64_t* const* pp, uint64_t* T, unsigned* flag,
-                        cudaStream_t st) {
-    if (smem > (48u << 10)) {
-        cudaError_t e = cudaFuncSetAttribute(k_perm_rows<NC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-    }
-    const unsigned blocks = (unsigned)((n + threads - 1) / threads);
-    k_perm_rows<NC><<<blocks, threads, smem, st>>>(wires, sigmas, R, D, P, n, x_lo, x_hi, bk, beta, gamma, pp, T, flag);
-    return cudaGetLastError();
-}
-
 }  // namespace
 
 cudaError_t pcs::launch_pow_table(uint64_t base, size_t n, uint64_t* out, cudaStream_t st) {
@@ -235,9 +219,11 @@ cudaError_t pcs::launch_pow_table(uint64_t base, size_t n, uint64_t* out, cudaSt
     return cudaGetLastError();
 }
 
-int pcs::upload_table(const void* ptrs, size_t count, DevBuf& buf, cudaStream_t st) {
-    PCS_CUDA(buf.alloc(count * sizeof(uint64_t*), st));
-    PCS_CUDA(cudaMemcpyAsync(buf.p, ptrs, count * sizeof(uint64_t*), cudaMemcpyHostToDevice, st));
+int pcs::point_tables(uint64_t root, size_t n, DevBuf& buf, cudaStream_t st) {
+    const size_t n_lo = (size_t)1 << X_LO_BITS, n_hi = (n + n_lo - 1) / n_lo;
+    PCS_CUDA(buf.alloc((n_lo + n_hi) * 8, st));
+    PCS_CUDA(launch_pow_table(root, std::min(n, n_lo), buf.u64(), st));
+    PCS_CUDA(launch_pow_table(glh::powmod(root, n_lo), n_hi, buf.u64() + n_lo, st));
     return PCS_OK;
 }
 
@@ -281,8 +267,6 @@ int pcs_permutation_partial_products(const uint64_t* const* wires, const uint64_
         return fail(PCS_ERR_ARG, "too many partial products: " + std::to_string(P) + " per challenge");
 
     // small tables: x_lo / x_hi, beta_c k_j, beta, gamma (canonical)
-    const uint64_t omega = glh::powmod(1753635133440165772ULL, (uint64_t)1 << (32 - lg_n));   // primitive_root_of_unity(lg_n)
-    const size_t n_lo = (size_t)1 << X_LO_BITS, n_hi = (n + n_lo - 1) / n_lo;
     std::vector<uint64_t> consts(C * R + 2 * C);
     for (size_t c = 0; c < C; c++) {
         const uint64_t b = betas[c] % glh::P;
@@ -291,11 +275,8 @@ int pcs_permutation_partial_products(const uint64_t* const* wires, const uint64_
         consts[C * R + C + c] = gammas[c] % glh::P;
     }
     DevBuf xt, cb, tscr, part, flag, in_buf, out_buf, t_wires, t_sigmas, t_out;
-    PCS_CUDA(xt.alloc((n_lo + n_hi) * 8, st));
-    PCS_CUDA(cb.alloc(consts.size() * 8, st));
-    PCS_CUDA(cudaMemcpyAsync(cb.p, consts.data(), consts.size() * 8, cudaMemcpyHostToDevice, st));
-    PCS_CUDA(launch_pow_table(omega, n_lo, xt.u64(), st));
-    PCS_CUDA(launch_pow_table(glh::powmod(omega, n_lo), n_hi, xt.u64() + n_lo, st));
+    if (int rc = point_tables(glh::primitive_root_of_unity(lg_n), n, xt, st)) return rc;
+    if (int rc = upload_table(consts.data(), consts.size(), cb, st)) return rc;
     PCS_CUDA(flag.alloc(sizeof(unsigned), st));
     PCS_CUDA(cudaMemsetAsync(flag.p, 0, sizeof(unsigned), st));
 
@@ -327,16 +308,16 @@ int pcs_permutation_partial_products(const uint64_t* const* wires, const uint64_
         uint64_t* const* ppc = cols + C + c0 * P;
         uint64_t* T = tscr.u64() + c0 * n;
         const size_t smem = smem_of(threads, nc);
-        const auto* wt = (const uint64_t* const*)t_wires.p;
-        const auto* stb = (const uint64_t* const*)t_sigmas.p;
-        cudaError_t e;
-        switch (nc) {
-            case 1: e = launch_rows<1>(threads, smem, wt, stb, (unsigned)R, (unsigned)D, (unsigned)P, n, xt.u64(), xt.u64() + n_lo, bkc, beta, gamma, ppc, T, (unsigned*)flag.p, st); break;
-            case 2: e = launch_rows<2>(threads, smem, wt, stb, (unsigned)R, (unsigned)D, (unsigned)P, n, xt.u64(), xt.u64() + n_lo, bkc, beta, gamma, ppc, T, (unsigned*)flag.p, st); break;
-            case 3: e = launch_rows<3>(threads, smem, wt, stb, (unsigned)R, (unsigned)D, (unsigned)P, n, xt.u64(), xt.u64() + n_lo, bkc, beta, gamma, ppc, T, (unsigned*)flag.p, st); break;
-            default: e = launch_rows<4>(threads, smem, wt, stb, (unsigned)R, (unsigned)D, (unsigned)P, n, xt.u64(), xt.u64() + n_lo, bkc, beta, gamma, ppc, T, (unsigned*)flag.p, st); break;
-        }
-        PCS_CUDA(e);
+        PCS_CUDA(dispatch_width(nc, [&](auto NC) {
+            if (smem > (48u << 10)) {
+                cudaError_t e = cudaFuncSetAttribute(k_perm_rows<NC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+                if (e != cudaSuccess) return e;
+            }
+            k_perm_rows<NC><<<(unsigned)((n + threads - 1) / threads), threads, smem, st>>>(
+                (const uint64_t* const*)t_wires.p, (const uint64_t* const*)t_sigmas.p, (unsigned)R, (unsigned)D, (unsigned)P, n,
+                xt.u64(), xt.u64() + (1u << X_LO_BITS), bkc, beta, gamma, ppc, T, (unsigned*)flag.p);
+            return cudaGetLastError();
+        }));
     }
 
     // step 2: Z = exclusive product scan of T; step 3: partial products times Z

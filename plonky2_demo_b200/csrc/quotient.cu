@@ -27,7 +27,6 @@
 #include <vector>
 
 #include "common.cuh"
-#include "ext.cuh"
 #include "gl64.cuh"
 
 using namespace pcs;
@@ -37,11 +36,6 @@ namespace {
 constexpr int PT_THREADS = 128;
 constexpr int PT_ITEMS = 4;        // points per thread, strided by PT_THREADS (coalesced): one inversion for all of them
 constexpr int MAX_NC = 4;          // challenges (and alphas) per pass over the inputs
-constexpr unsigned X_LO_BITS = 10; // x_i = 7 * x_hi[i >> 10] * x_lo[i & 1023]
-
-__device__ __forceinline__ size_t brev_bits(size_t v, unsigned bits) {
-    return bits ? (size_t)(__brevll((unsigned long long)v) >> (64 - bits)) : 0;
-}
 
 struct PointArgs {
     const uint64_t* sigmas;   // sigma column j at sigmas[j * stride + l]
@@ -50,8 +44,8 @@ struct PointArgs {
     size_t stride;            // N = n << rate_bits (the batches' column length)
     unsigned R, D, K, C, lg_n, lg_m;
     uint64_t n_f;             // n as a field element
-    const uint64_t* x_lo;     // w_M^j, j < 1024
-    const uint64_t* x_hi;     // w_M^(1024 j)
+    const uint64_t* x_lo;     // point_tables of w_M: x_i = 7 w_M^i
+    const uint64_t* x_hi;
     const uint64_t* zh;       // [2^q] Z_H(x) of coset block b
     const uint64_t* zh_inv;   // [2^q] Z_H(x)^-1
     const uint64_t* bk;       // [C][R] beta_c k_j
@@ -81,7 +75,7 @@ __global__ void __launch_bounds__(PT_THREADS) k_quotient_points(const PointArgs 
         xs[k] = 0;
         if (l < M) {
             const size_t i = brev_bits(l, A.lg_m);
-            xs[k] = gl::mul(gl::mul(A.x_hi[i >> X_LO_BITS], A.x_lo[i & ((1u << X_LO_BITS) - 1)]), 7);
+            xs[k] = gl::mul(subgroup_point(A.x_lo, A.x_hi, i), 7);
             d = gl::mul(A.n_f, gl::canon(gl::sub_lc(xs[k], 1)));
         }
         pre[k] = acc;
@@ -195,20 +189,45 @@ __global__ void __launch_bounds__(PT_THREADS) k_quotient_points(const PointArgs 
     }
 }
 
-template <int N>
-cudaError_t launch_points(const PointArgs& A, unsigned c0, unsigned nc, unsigned a0, unsigned na, cudaStream_t st) {
-    const size_t M = (size_t)1 << A.lg_m, per_block = PT_THREADS * PT_ITEMS;
-    k_quotient_points<N><<<(unsigned)((M + per_block - 1) / per_block), PT_THREADS, 0, st>>>(A, c0, nc, a0, na);
-    return cudaGetLastError();
-}
-
 // trim_to_len(D n): coefficients [from, M) of every column of vals [C][M] must be zero
 __global__ void k_trim_check(const uint64_t* __restrict__ vals, size_t M, size_t from, unsigned* flag) {
     const size_t i = from + (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < M && vals[(size_t)blockIdx.y * M + i] != 0) *flag = 1;
 }
 
+// resident, whole, committed LDE rows (what the quotient-domain kernels read in place), or the reason why not
+const char* unusable(const pcs_batch* b) {
+    if (b->on_demand) return "a PCS_LDE_ON_DEMAND batch keeps no LDE rows";
+    if (b->rows_only || b->coset_first != 0 || b->full_rate_bits != b->rate_bits) return "a shard batch holds part of the LDE";
+    if (!b->lde || !b->committed) return "the batch is not committed";
+    return nullptr;
+}
+
+unsigned log2_ceil(size_t v) {
+    unsigned q = 0;
+    while (((size_t)1 << q) < v) q++;
+    return q;
+}
+
 }  // namespace
+
+int pcs::check_quotient_domain(std::initializer_list<const pcs_batch*> batches, size_t D, size_t C, unsigned& lg_n, unsigned& q) {
+    const pcs_batch* b0 = *batches.begin();
+    for (const pcs_batch* b : batches)
+        if (b->ctx != b0->ctx) return fail(PCS_ERR_ARG, "the batches belong to different contexts");
+    if (D < 2) return fail(PCS_ERR_ARG, "quotient_degree_factor must be at least 2");
+    if (C == 0) return fail(PCS_ERR_ARG, "num_challenges is 0");
+    for (const pcs_batch* b : batches)
+        if (const char* why = unusable(b)) return fail(PCS_ERR_ARG, why);
+    for (const pcs_batch* b : batches)
+        if (b->lg_d != b0->lg_d || b->rate_bits != b0->rate_bits) return fail(PCS_ERR_ARG, "the batches differ in degree or rate");
+    lg_n = b0->lg_d;
+    q = log2_ceil(D);
+    if (q > b0->rate_bits)   // compute_quotient_polys' assertion
+        return fail(PCS_ERR_ARG, "Having constraints of degree higher than the rate is not supported yet. "
+                                 "quotient_degree_factor " + std::to_string(D) + " needs rate_bits >= " + std::to_string(q));
+    return PCS_OK;
+}
 
 extern "C" {
 
@@ -218,22 +237,13 @@ int pcs_quotient_polys(const pcs_batch* constants_sigmas, const pcs_batch* wires
                        const uint64_t* const* gate_terms, unsigned flags, uint64_t* const* out) {
     const pcs_batch *cs = constants_sigmas, *wb = wires, *zb = zs_partial_products;
     if (!cs || !wb || !zb || !k_is || !betas || !gammas || !alphas || !out) return fail(PCS_ERR_ARG, "NULL pointer");
-    if (cs->ctx != wb->ctx || cs->ctx != zb->ctx) return fail(PCS_ERR_ARG, "the batches belong to different contexts");
     BatchScope scope(cs);
     if (int rc = need_init()) return rc;
     const size_t R = num_routed_wires, C = num_challenges, D = quotient_degree_factor;
-    if (D < 2) return fail(PCS_ERR_ARG, "quotient_degree_factor must be at least 2");
+    unsigned lg_n, q;
+    if (int rc = check_quotient_domain({cs, wb, zb}, D, C, lg_n, q)) return rc;
     if (R == 0) return fail(PCS_ERR_ARG, "num_routed_wires is 0");
-    if (C == 0) return fail(PCS_ERR_ARG, "num_challenges is 0");
     if (R > 0xFFFFFFFFu || C > 0xFFFFu) return fail(PCS_ERR_ARG, "num_routed_wires or num_challenges too large");
-    for (const pcs_batch* b : {cs, wb, zb})
-        if (const char* why = unusable(b)) return fail(PCS_ERR_ARG, why);
-    if (wb->lg_d != cs->lg_d || zb->lg_d != cs->lg_d || wb->rate_bits != cs->rate_bits || zb->rate_bits != cs->rate_bits)
-        return fail(PCS_ERR_ARG, "the batches differ in degree or rate");
-    const unsigned lg_n = cs->lg_d, q = log2_ceil(D);
-    if (q > cs->rate_bits)   // compute_quotient_polys' assertion
-        return fail(PCS_ERR_ARG, "Having constraints of degree higher than the rate is not supported yet. "
-                                 "quotient_degree_factor " + std::to_string(D) + " needs rate_bits >= " + std::to_string(q));
     const size_t K = (R + D - 1) / D, P = K - 1;
     if (num_constants + R > cs->w || num_constants > cs->w)
         return fail(PCS_ERR_ARG, "constants_sigmas has " + std::to_string(cs->w) + " polynomials, the sigmas end at " +
@@ -253,7 +263,7 @@ int pcs_quotient_polys(const pcs_batch* constants_sigmas, const pcs_batch* wires
     const size_t n = (size_t)1 << lg_n, M = (size_t)1 << lg_m, blocks = (size_t)1 << q;
 
     // small tables (canonical): bk [C][R], beta, gamma, alpha [C], apow [C][2C + 1], zh, zh_inv [2^q]
-    const uint64_t w_m = glh::powmod(1753635133440165772ULL, (uint64_t)1 << (32 - lg_m));   // primitive_root_of_unity(lg_m)
+    const uint64_t w_m = glh::primitive_root_of_unity(lg_m);
     std::vector<uint64_t> consts(C * R + 3 * C + C * (2 * C + 1) + 2 * blocks);
     uint64_t* h = consts.data();
     uint64_t *h_bk = h, *h_beta = h_bk + C * R, *h_gamma = h_beta + C, *h_alpha = h_gamma + C, *h_apow = h_alpha + C,
@@ -278,15 +288,11 @@ int pcs_quotient_polys(const pcs_batch* constants_sigmas, const pcs_batch* wires
         for (unsigned s = 0; s < q; s++) br |= ((b >> s) & 1) << (q - 1 - s);
         const uint64_t v = glh::mulmod(g_n, glh::powmod(w_q, br));
         h_zh[b] = v ? v - 1 : glh::P - 1;
-        h_zhi[b] = glh::powmod(h_zh[b], glh::P - 2);
+        h_zhi[b] = glh::inverse(h_zh[b]);
     }
-    const size_t n_lo = std::min<size_t>(M, (size_t)1 << X_LO_BITS), n_hi = (M + n_lo - 1) / n_lo;
     DevBuf cb, xt, flag, tails, t_tails, pts, nat;   // released in stream order on every return
-    PCS_CUDA(cb.alloc(consts.size() * 8, st));
-    PCS_CUDA(cudaMemcpyAsync(cb.p, consts.data(), consts.size() * 8, cudaMemcpyHostToDevice, st));
-    PCS_CUDA(xt.alloc(((size_t)1024 + n_hi) * 8, st));
-    PCS_CUDA(launch_pow_table(w_m, n_lo, xt.u64(), st));
-    PCS_CUDA(launch_pow_table(glh::powmod(w_m, 1024), n_hi, xt.u64() + 1024, st));
+    if (int rc = upload_table(consts.data(), consts.size(), cb, st)) return rc;
+    if (int rc = point_tables(w_m, M, xt, st)) return rc;
     PCS_CUDA(flag.alloc(sizeof(unsigned), st));
     PCS_CUDA(cudaMemsetAsync(flag.p, 0, sizeof(unsigned), st));
 
@@ -312,24 +318,21 @@ int pcs_quotient_polys(const pcs_batch* constants_sigmas, const pcs_batch* wires
     A.stride = cs->n;
     A.R = (unsigned)R, A.D = (unsigned)D, A.K = (unsigned)K, A.C = (unsigned)C, A.lg_n = lg_n, A.lg_m = lg_m;
     A.n_f = n % glh::P;
-    A.x_lo = xt.u64(), A.x_hi = xt.u64() + 1024;
+    A.x_lo = xt.u64(), A.x_hi = xt.u64() + (1u << X_LO_BITS);
     const uint64_t* dc = cb.u64();
     A.bk = dc, A.beta = dc + (h_beta - h), A.gamma = dc + (h_gamma - h), A.alpha = dc + (h_alpha - h);
     A.apow = dc + (h_apow - h), A.zh = dc + (h_zh - h), A.zh_inv = dc + (h_zhi - h);
     A.tail = tail_dev;
     A.out = pts.u64();
-    const unsigned N = (unsigned)std::min<size_t>(C, MAX_NC);
     for (size_t c0 = 0; c0 < C; c0 += MAX_NC)
         for (size_t a0 = 0; a0 < C; a0 += MAX_NC) {
             const unsigned nc = (unsigned)std::min<size_t>(C - c0, MAX_NC), na = (unsigned)std::min<size_t>(C - a0, MAX_NC);
-            cudaError_t e;
-            switch (N) {
-                case 1: e = launch_points<1>(A, (unsigned)c0, nc, (unsigned)a0, na, st); break;
-                case 2: e = launch_points<2>(A, (unsigned)c0, nc, (unsigned)a0, na, st); break;
-                case 3: e = launch_points<3>(A, (unsigned)c0, nc, (unsigned)a0, na, st); break;
-                default: e = launch_points<4>(A, (unsigned)c0, nc, (unsigned)a0, na, st); break;
-            }
-            PCS_CUDA(e);
+            PCS_CUDA(dispatch_width(C, [&](auto N) {
+                const size_t per_block = PT_THREADS * PT_ITEMS;
+                k_quotient_points<N><<<(unsigned)((M + per_block - 1) / per_block), PT_THREADS, 0, st>>>(A, (unsigned)c0, nc,
+                                                                                                       (unsigned)a0, na);
+                return cudaGetLastError();
+            }));
         }
     tails.release();
 

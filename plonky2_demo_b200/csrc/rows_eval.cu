@@ -28,7 +28,7 @@ __global__ void k_point_tables(const uint64_t* __restrict__ idx, size_t n, size_
     if (i >= n_pad * per) return;
     const size_t k = i / per, e = i % per;
     const size_t leaf = k < n ? idx[k] : 0;
-    const uint64_t br = lg_n ? (uint64_t)(__brevll((unsigned long long)leaf) >> (64 - lg_n)) : 0;
+    const uint64_t br = brev_bits(leaf, lg_n);
     const uint64_t x = gl::canon(gl::mul(7, gl::pow(root, br)));   // F::coset_shift() = 7 (types.rs:437)
     const uint64_t ex = e < TAB_K ? e : e < TAB_C ? (uint64_t)(e - TAB_K) * RE_THREADS : (uint64_t)(e - TAB_C) * RE_CHUNK;
     tabs[i] = gl::pow(x, ex);
@@ -113,8 +113,7 @@ int rows_eval(const pcs_batch* b, const uint64_t* idx_dev, size_t n, uint64_t* o
     const size_t d = (size_t)1 << b->lg_d, chunks = (d + RE_CHUNK - 1) / RE_CHUNK;
     const size_t tiles = (n + RE_POINTS - 1) / RE_POINTS, n_pad = tiles * RE_POINTS, per = TAB_C + chunks;
     const unsigned lg_n = b->lg_d + b->rate_bits;
-    // primitive_root_of_unity(lg_n) = POWER_OF_TWO_GENERATOR^(2^(32 - lg_n))   types.rs:268-272
-    const uint64_t root = glh::powmod(1753635133440165772ULL, (uint64_t)1 << (32 - lg_n));
+    const uint64_t root = glh::primitive_root_of_unity(lg_n);
     DevBuf tabs, partial;
     PCS_CUDA(tabs.alloc(n_pad * per * 8, st));
     PCS_CUDA(partial.alloc(n_pad * b->w * chunks * 8, st));

@@ -20,6 +20,7 @@ from dataclasses import dataclass
 import numpy as np
 
 from . import _ffi
+from .polynomial import log2_ceil
 
 
 @dataclass(frozen=True)
@@ -91,7 +92,7 @@ def gate_constraint_terms(constants_sigmas, wires, gates, selectors_info, num_co
         raise ValueError("public_inputs_hash: 4 elements")
     D = int(quotient_degree_factor)
     n = 1 << constants_sigmas.degree_log
-    out = np.empty((a.shape[0], n << (D - 1).bit_length()), dtype=np.uint64)
+    out = np.empty((a.shape[0], n << log2_ceil(D)), dtype=np.uint64)
     _ffi.check(_ffi.lib().pcs_gate_constraint_terms(
         constants_sigmas._h, wires._h, table.ctypes.data_as(_ffi.C.POINTER(_ffi.C.c_uint32)), table.shape[0],
         groups.ctypes.data_as(_ffi.C.POINTER(_ffi.sz)), groups.shape[0], 0, int(num_constants), _ffi.ptr(pih), _ffi.ptr(a),

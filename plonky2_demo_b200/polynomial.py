@@ -20,6 +20,11 @@ def log2_strict(n):
     return n.bit_length() - 1
 
 
+def log2_ceil(n):
+    """util/src/lib.rs log2_ceil: the least q with 2^q >= n."""
+    return (int(n) - 1).bit_length()
+
+
 def reverse_bits(n, num_bits):
     """plonky2/src/util/mod.rs:30-38"""
     return int(format(n, f"0{num_bits}b")[::-1], 2) if num_bits else 0

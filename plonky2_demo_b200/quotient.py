@@ -16,10 +16,7 @@ by Z_H", where the reference panics.
 import numpy as np
 
 from . import _ffi
-
-
-def _log2_ceil(v):
-    return (int(v) - 1).bit_length()
+from .polynomial import log2_ceil
 
 
 def quotient_poly_chunks(constants_sigmas, wires, zs_partial_products, num_constants, num_routed_wires, k_is, betas, gammas,
@@ -34,7 +31,7 @@ def quotient_poly_chunks(constants_sigmas, wires, zs_partial_products, num_const
     tails = None
     if gate_terms is not None:
         gt = _ffi.as_u64(gate_terms)
-        if gt.shape != (C, n << _log2_ceil(D)):
+        if gt.shape != (C, n << log2_ceil(D)):
             raise ValueError("gate_terms: [num_challenges][n 2^log2_ceil(quotient_degree_factor)]")
         tails = _ffi.ptr_array([gt[j] for j in range(C)])
     out = np.empty((C * max(D, 0), n), dtype=np.uint64)
@@ -52,6 +49,6 @@ def compute_quotient_polys(constants_sigmas, wires, zs_partial_products, num_con
                                   gammas, alphas, quotient_degree_factor, gate_terms)
     D, n = int(quotient_degree_factor), 1 << constants_sigmas.degree_log
     C = chunks.shape[0] // D
-    out = np.zeros((C, n << _log2_ceil(D)), dtype=np.uint64)
+    out = np.zeros((C, n << log2_ceil(D)), dtype=np.uint64)
     out[:, :D * n] = chunks.reshape(C, D * n)
     return out

@@ -1,40 +1,21 @@
 """ORACLE -- test infrastructure, NOT the product: ctypes front-end of gate_oracle.c, the CPU restatement of
 evaluate_gate_constraints_base_batch (plonk/vanishing_poly.rs) for NoopGate, ConstantGate, PublicInputGate, ArithmeticGate and
-PoseidonGate, reduced with powers of each alpha: the gate-constraint tail of compute_quotient_polys.  The library is compiled on
-first use with gcc into a per-user temporary directory keyed by the source's hash, so a read-only tree works too.  Its inputs are
-the batches' LDEs in natural order, as oracle.coset_lde returns them."""
+PoseidonGate, reduced with powers of each alpha: the gate-constraint tail of compute_quotient_polys.  The library is built by
+c_oracle.  Its inputs are the batches' LDEs in natural order, as oracle.coset_lde returns them."""
 import ctypes as C
-import hashlib
-import os
-import subprocess
-import tempfile
 
+import c_oracle
 import numpy as np
+from c_oracle import u64, u64p
 
-_HERE = os.path.dirname(os.path.abspath(__file__))
-_SRC = os.path.join(_HERE, "gate_oracle.c")
-_ORACLE_DIR = os.path.join(os.path.dirname(os.path.dirname(_HERE)), "oracle")   # gl64.h, poseidon_constants.h
 _lib = None
-u64p = C.POINTER(C.c_uint64)
 
 NOOP, CONSTANT, PUBLIC_INPUT, ARITHMETIC, POSEIDON = range(5)
 
 
 def build():
     """Compile (if needed) and return the path of the shared library."""
-    h = hashlib.sha256()
-    for f in (_SRC, os.path.join(_ORACLE_DIR, "gl64.h"), os.path.join(_ORACLE_DIR, "poseidon_constants.h")):
-        with open(f, "rb") as fh:
-            h.update(fh.read())
-    out_dir = os.path.join(tempfile.gettempdir(), f"pcs_gate_oracle_{os.getuid()}")
-    os.makedirs(out_dir, exist_ok=True)
-    so = os.path.join(out_dir, f"libgate_oracle_{h.hexdigest()[:16]}.so")
-    if not os.path.exists(so):
-        tmp = f"{so}.{os.getpid()}.tmp"
-        subprocess.check_call(["gcc", "-O3", "-march=x86-64-v3", "-fopenmp", "-fPIC", "-fvisibility=hidden", "-Wall", "-Wextra",
-                               "-std=gnu11", "-shared", "-I", _ORACLE_DIR, "-o", tmp, _SRC])
-        os.replace(tmp, so)
-    return so
+    return c_oracle.build("gate_oracle", ("gl64.h", "poseidon_constants.h"))
 
 
 def lib():
@@ -53,25 +34,16 @@ def lib():
 
 
 def use_all_cores():
-    try:
-        n = len(os.sched_getaffinity(0))
-    except AttributeError:
-        n = os.cpu_count() or 1
-    lib().ref_gate_set_num_threads(n)
-    return n
+    return c_oracle.use_all_cores(lib().ref_gate_set_num_threads)
 
 
 def set_num_threads(n):
     lib().ref_gate_set_num_threads(int(n))
 
 
-def _u64(a):
-    return np.ascontiguousarray(a, dtype=np.uint64)
-
-
 def poseidon_gate_constraints(wires_row):
     """PoseidonGate::eval_unfiltered on one row of 135 wire values (fast form) -> its 123 constraints"""
-    w = _u64(wires_row)
+    w = u64(wires_row)
     assert w.shape == (135,)
     out = np.empty(123, dtype=np.uint64)
     lib().ref_poseidon_gate_constraints(w.ctypes.data_as(u64p), out.ctypes.data_as(u64p))
@@ -81,7 +53,7 @@ def poseidon_gate_constraints(wires_row):
 def gate_terms(cs_lde, wires_lde, rate_bits, gates, groups, num_constants, public_inputs_hash, alphas, quotient_degree_factor):
     """Natural-order LDEs [w][n << rate_bits] of constants_sigmas and wires; gates [(kind, param, selector_index)], groups
     [(start, end)] -> [C][n 2^q] gate terms in natural order of the quotient domain"""
-    cs, w = _u64(cs_lde), _u64(wires_lde)
+    cs, w = u64(cs_lde), u64(wires_lde)
     N = cs.shape[1]
     assert w.shape[1] == N
     n = N >> rate_bits
@@ -89,7 +61,7 @@ def gate_terms(cs_lde, wires_lde, rate_bits, gates, groups, num_constants, publi
     M = n << q
     g = np.ascontiguousarray(np.array(gates, dtype=np.uint32).reshape(-1, 3))
     gr = np.ascontiguousarray(np.array(groups, dtype=np.uintp).reshape(-1, 2))
-    pih, a = _u64(np.asarray(public_inputs_hash).reshape(4)), _u64(np.atleast_1d(alphas))
+    pih, a = u64(np.asarray(public_inputs_hash).reshape(4)), u64(np.atleast_1d(alphas))
     out = np.empty((a.size, M), dtype=np.uint64)
     rc = lib().ref_gate_terms(cs.ctypes.data_as(u64p), cs.shape[0], w.ctypes.data_as(u64p), w.shape[0], n.bit_length() - 1,
                               rate_bits, g.ctypes.data_as(C.POINTER(C.c_uint32)), g.shape[0],

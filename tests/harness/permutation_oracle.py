@@ -1,36 +1,17 @@
 """ORACLE -- test infrastructure, NOT the product: ctypes front-end of permutation_oracle.c, the CPU restatement of
-all_wires_permutation_partial_products (plonk/prover.rs).  The library is compiled on first use with gcc into a
-per-user temporary directory keyed by the source's hash, so a read-only tree works too."""
+all_wires_permutation_partial_products (plonk/prover.rs).  The library is built by c_oracle."""
 import ctypes as C
-import hashlib
-import os
-import subprocess
-import tempfile
 
+import c_oracle
 import numpy as np
+from c_oracle import u64, u64p
 
-_HERE = os.path.dirname(os.path.abspath(__file__))
-_SRC = os.path.join(_HERE, "permutation_oracle.c")
-_ORACLE_DIR = os.path.join(os.path.dirname(os.path.dirname(_HERE)), "oracle")   # gl64.h
 _lib = None
-u64p = C.POINTER(C.c_uint64)
 
 
 def build():
     """Compile (if needed) and return the path of the shared library."""
-    h = hashlib.sha256()
-    for f in (_SRC, os.path.join(_ORACLE_DIR, "gl64.h")):
-        with open(f, "rb") as fh:
-            h.update(fh.read())
-    out_dir = os.path.join(tempfile.gettempdir(), f"pcs_permutation_oracle_{os.getuid()}")
-    os.makedirs(out_dir, exist_ok=True)
-    so = os.path.join(out_dir, f"libpermutation_oracle_{h.hexdigest()[:16]}.so")
-    if not os.path.exists(so):
-        tmp = f"{so}.{os.getpid()}.tmp"
-        subprocess.check_call(["gcc", "-O3", "-march=x86-64-v3", "-fopenmp", "-fPIC", "-fvisibility=hidden", "-Wall", "-Wextra",
-                               "-std=gnu11", "-shared", "-I", _ORACLE_DIR, "-o", tmp, _SRC])
-        os.replace(tmp, so)
-    return so
+    return c_oracle.build("permutation_oracle")
 
 
 def lib():
@@ -47,23 +28,14 @@ def lib():
 
 
 def use_all_cores():
-    try:
-        n = len(os.sched_getaffinity(0))
-    except AttributeError:
-        n = os.cpu_count() or 1
-    lib().ref_perm_set_num_threads(n)
-    return n
-
-
-def _u64(a):
-    return np.ascontiguousarray(a, dtype=np.uint64)
+    return c_oracle.use_all_cores(lib().ref_perm_set_num_threads)
 
 
 def all_wires_permutation_partial_products(wires, sigmas, k_is, betas, gammas, quotient_degree_factor):
     """wires, sigmas [R][n]; k_is [R]; betas, gammas [C] -> [C][P + 1][n]: per challenge [pp_0 .. pp_{P-1}, Z], the order
     wires_permutation_partial_products_and_zs returns.  Raises ZeroDivisionError("Tried to invert zero") where the
     reference panics."""
-    w, s, k, b, g = (_u64(a) for a in (wires, sigmas, k_is, betas, gammas))
+    w, s, k, b, g = (u64(a) for a in (wires, sigmas, k_is, betas, gammas))
     R, n = w.shape
     assert s.shape == (R, n) and k.shape == (R,) and b.shape == g.shape
     lg_n = n.bit_length() - 1

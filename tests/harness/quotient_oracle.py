@@ -1,39 +1,20 @@
 """ORACLE -- test infrastructure, NOT the product: ctypes front-end of quotient_oracle.c, the CPU restatement of
-compute_quotient_polys (plonk/prover.rs:576-744) without the gate constraints, and of prove()'s trim_to_len / chunks.  The
-library is compiled on first use with gcc into a per-user temporary directory keyed by the source's hash, so a read-only tree
-works too.  Its inputs are the batches' LDEs in natural order, as oracle.coset_lde returns them."""
+compute_quotient_polys (plonk/prover.rs:576-744) without the gate constraints, and of prove()'s trim_to_len / chunks.  The library is
+built by c_oracle.  Its inputs are the batches' LDEs in natural order, as oracle.coset_lde returns them."""
 import ctypes as C
-import hashlib
-import os
-import subprocess
-import tempfile
 
+import c_oracle
 import numpy as np
+from c_oracle import u64, u64p
 
-_HERE = os.path.dirname(os.path.abspath(__file__))
-_SRC = os.path.join(_HERE, "quotient_oracle.c")
-_ORACLE_DIR = os.path.join(os.path.dirname(os.path.dirname(_HERE)), "oracle")   # gl64.h
 _lib = None
-u64p = C.POINTER(C.c_uint64)
 
 QUOTIENT_FAILED = "Quotient has failed, the vanishing polynomial is not divisible by Z_H"
 
 
 def build():
     """Compile (if needed) and return the path of the shared library."""
-    h = hashlib.sha256()
-    for f in (_SRC, os.path.join(_ORACLE_DIR, "gl64.h")):
-        with open(f, "rb") as fh:
-            h.update(fh.read())
-    out_dir = os.path.join(tempfile.gettempdir(), f"pcs_quotient_oracle_{os.getuid()}")
-    os.makedirs(out_dir, exist_ok=True)
-    so = os.path.join(out_dir, f"libquotient_oracle_{h.hexdigest()[:16]}.so")
-    if not os.path.exists(so):
-        tmp = f"{so}.{os.getpid()}.tmp"
-        subprocess.check_call(["gcc", "-O3", "-march=x86-64-v3", "-fopenmp", "-fPIC", "-fvisibility=hidden", "-Wall", "-Wextra",
-                               "-std=gnu11", "-shared", "-I", _ORACLE_DIR, "-o", tmp, _SRC])
-        os.replace(tmp, so)
-    return so
+    return c_oracle.build("quotient_oracle")
 
 
 def lib():
@@ -52,16 +33,7 @@ def lib():
 
 
 def use_all_cores():
-    try:
-        n = len(os.sched_getaffinity(0))
-    except AttributeError:
-        n = os.cpu_count() or 1
-    lib().ref_quot_set_num_threads(n)
-    return n
-
-
-def _u64(a):
-    return np.ascontiguousarray(a, dtype=np.uint64)
+    return c_oracle.use_all_cores(lib().ref_quot_set_num_threads)
 
 
 def log2_ceil(v):
@@ -72,15 +44,15 @@ def compute_quotient_polys(cs_lde, wires_lde, zs_lde, rate_bits, num_constants, 
                            quotient_degree_factor, gate_terms=None):
     """Natural-order LDEs [w][n << rate_bits] of constants_sigmas, wires and zs_partial_products -> [C][n 2^q] coefficients of
     the quotient polynomials (coset_ifft(7) of the quotient values), before the trim."""
-    cs, w, z = _u64(cs_lde), _u64(wires_lde), _u64(zs_lde)
-    k, b, g, a = (_u64(np.atleast_1d(v)) for v in (k_is, betas, gammas, alphas))
+    cs, w, z = u64(cs_lde), u64(wires_lde), u64(zs_lde)
+    k, b, g, a = (u64(np.atleast_1d(v)) for v in (k_is, betas, gammas, alphas))
     N = cs.shape[1]
     assert w.shape[1] == N and z.shape[1] == N and b.shape == g.shape == a.shape
     n = N >> rate_bits
     lg_n = n.bit_length() - 1
     q = log2_ceil(quotient_degree_factor)
     M = n << q
-    tails = None if gate_terms is None else _u64(gate_terms)
+    tails = None if gate_terms is None else u64(gate_terms)
     assert tails is None or tails.shape == (b.size, M)
     out = np.empty((b.size, M), dtype=np.uint64)
     p = lambda x: x.ctypes.data_as(u64p) if x is not None else None  # noqa: E731
@@ -94,7 +66,7 @@ def compute_quotient_polys(cs_lde, wires_lde, zs_lde, rate_bits, num_constants, 
 def quotient_poly_chunks(quotient_polys, n, quotient_degree_factor):
     """prove(): trim_to_len(D n) of every quotient polynomial (ValueError with the reference's message when a coefficient
     beyond it is not zero), then chunks(n): [C D][n], alpha-major."""
-    qp = _u64(quotient_polys)
+    qp = u64(quotient_polys)
     D = quotient_degree_factor
     if qp[:, D * n:].any():
         raise ValueError(QUOTIENT_FAILED)

@@ -1,4 +1,6 @@
-"""Shared test helpers: seeded inputs (SURVEY 8d generator) and big-int field arithmetic."""
+"""Shared test helpers: seeded inputs (SURVEY 8d generator), big-int field arithmetic and device buffers for the GPU tests."""
+import ctypes as C
+
 import numpy as np
 
 P = 0xFFFFFFFF00000001
@@ -75,3 +77,94 @@ def as_oracle_proof(proof):
             for r in proof.query_round_proofs
         ],
     }
+
+
+def noncanonical(rng, shape):
+    """uniform u64 with a share of values in [p, 2^64) (the reference's loose representation)"""
+    a = rng.integers(0, 1 << 64, size=shape, dtype=np.uint64, endpoint=False)
+    hi = rng.random(shape) < 0.25
+    a[hi] = np.uint64(P) + (a[hi] % np.uint64((1 << 64) - P))
+    return a
+
+
+class Ext:
+    """a + b X in F[X] / (X^2 - 7), the reference's quadratic extension; % P is a no-op (values stay reduced)"""
+
+    def __init__(self, a, b=0):
+        self.a, self.b = int(a) % P, int(b) % P
+
+    def _c(self, o):
+        return o if isinstance(o, Ext) else Ext(o)
+
+    def __add__(self, o):
+        o = self._c(o)
+        return Ext(self.a + o.a, self.b + o.b)
+
+    __radd__ = __add__
+
+    def __sub__(self, o):
+        o = self._c(o)
+        return Ext(self.a - o.a, self.b - o.b)
+
+    def __rsub__(self, o):
+        return self._c(o) - self
+
+    def __mul__(self, o):
+        o = self._c(o)
+        return Ext(self.a * o.a + 7 * self.b * o.b, self.a * o.b + self.b * o.a)
+
+    __rmul__ = __mul__
+
+    def __mod__(self, _):
+        return self
+
+    def __eq__(self, o):
+        o = self._c(o)
+        return (self.a, self.b) == (o.a, o.b)
+
+    def __repr__(self):
+        return f"Ext({self.a}, {self.b})"
+
+    def pow(self, e):
+        r, x = Ext(1), self
+        while e:
+            if e & 1:
+                r = r * x
+            x = x * x
+            e >>= 1
+        return r
+
+    def inv(self):
+        ni = pow((self.a * self.a - 7 * self.b * self.b) % P, P - 2, P)
+        return Ext(self.a * ni, (P - self.b) * ni)
+
+
+def mem_available_bytes():
+    try:
+        with open("/proc/meminfo") as f:
+            for line in f:
+                if line.startswith("MemAvailable:"):
+                    return int(line.split()[1]) * 1024
+    except OSError:
+        pass
+    return 0
+
+
+def torch_u64(a):
+    """a u64 array as a device tensor of the same bits"""
+    import torch
+
+    return torch.from_numpy(np.ascontiguousarray(a).view(np.int64)).cuda()
+
+
+def dev_table(tensors):
+    """a host table of the tensors' device pointers"""
+    from plonky2_demo_b200 import _ffi
+
+    return (_ffi.u64p * len(tensors))(*[C.cast(C.c_void_p(t.data_ptr()), _ffi.u64p) for t in tensors])
+
+
+def free(*batches):
+    """free the batches now: a failing test's traceback would otherwise keep them alive past pcs_shutdown"""
+    for b in batches:
+        b.free()

@@ -30,7 +30,7 @@ sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "har
 import gate_oracle as go  # noqa: E402
 import permutation_oracle as po  # noqa: E402
 import quotient_oracle as qo  # noqa: E402
-from test_permutation_oracle import noncanonical  # noqa: E402
+from helpers import Ext, noncanonical  # noqa: E402
 from test_quotient_oracle import vanishing_at  # noqa: E402
 
 P = 0xFFFFFFFF00000001
@@ -50,45 +50,6 @@ def omega(lg):
 
 # ---- literal big-int restatement of the reference ------------------------------------------------------------------------
 # Written with + - * and % P only, so that it evaluates base-field ints and Ext elements (the verifier's openings) alike.
-class Ext:
-    """a + b X in F[X] / (X^2 - 7), the reference's quadratic extension; % P is a no-op (values stay reduced)"""
-
-    def __init__(self, a, b=0):
-        self.a, self.b = int(a) % P, int(b) % P
-
-    def _c(self, o):
-        return o if isinstance(o, Ext) else Ext(o)
-
-    def __add__(self, o):
-        o = self._c(o)
-        return Ext(self.a + o.a, self.b + o.b)
-
-    __radd__ = __add__
-
-    def __sub__(self, o):
-        o = self._c(o)
-        return Ext(self.a - o.a, self.b - o.b)
-
-    def __rsub__(self, o):
-        return self._c(o) - self
-
-    def __mul__(self, o):
-        o = self._c(o)
-        return Ext(self.a * o.a + 7 * self.b * o.b, self.a * o.b + self.b * o.a)
-
-    __rmul__ = __mul__
-
-    def __mod__(self, _):
-        return self
-
-    def __eq__(self, o):
-        o = self._c(o)
-        return (self.a, self.b) == (o.a, o.b)
-
-    def __repr__(self):
-        return f"Ext({self.a}, {self.b})"
-
-
 def _el(v):
     return v if isinstance(v, Ext) else int(v) % P
 

@@ -23,7 +23,7 @@ import numpy as np
 import pytest
 
 import oracle
-from helpers import P, as_oracle_proof, assert_same_proof, brev, seeded_polys
+from helpers import P, as_oracle_proof, assert_same_proof, brev, mem_available_bytes, seeded_polys
 from oracle import fri_ref as fr
 
 pytestmark = pytest.mark.gpu
@@ -36,17 +36,6 @@ MIN_FREE_HBM = 24 << 30
 MIN_HOST_MEM = 40 << 30      # the oracle's peak at the headline shape, plus the inputs and readbacks of a case
 
 
-def _mem_available_bytes():
-    try:
-        with open("/proc/meminfo") as f:
-            for line in f:
-                if line.startswith("MemAvailable:"):
-                    return int(line.split()[1]) * 1024
-    except OSError:
-        pass
-    return 0
-
-
 @pytest.fixture(scope="module")
 def L():
     import torch
@@ -54,7 +43,7 @@ def L():
     import plonky2_demo_b200 as p
     from plonky2_demo_b200 import _ffi
 
-    free_hbm, host = torch.cuda.mem_get_info()[0], _mem_available_bytes()
+    free_hbm, host = torch.cuda.mem_get_info()[0], mem_available_bytes()
     if free_hbm < MIN_FREE_HBM:
         pytest.skip(f"benchmark-size commits need {MIN_FREE_HBM >> 30} GiB of free HBM ({free_hbm >> 30} GiB free)")
     if host < MIN_HOST_MEM:

@@ -19,8 +19,9 @@ import oracle
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "harness"))
 import gate_oracle as go  # noqa: E402
 import quotient_oracle as qo  # noqa: E402
+from helpers import Ext, dev_table, free, mem_available_bytes, noncanonical, torch_u64  # noqa: E402
 from test_gate_oracle import (  # noqa: E402
-    ARITHMETIC, CONSTANT, DEMO_GATES, DEMO_GROUPS, NOOP, Ext, gate_slots, reduce_with_powers, satisfied_instance)
+    ARITHMETIC, CONSTANT, DEMO_GATES, DEMO_GROUPS, NOOP, gate_slots, reduce_with_powers, satisfied_instance)
 
 pytestmark = pytest.mark.gpu
 
@@ -38,24 +39,6 @@ SHAPES = [   # (lg_n, C, D, rate_bits, gate set, wires salt_w)
     (20, 2, 8, 3, "demo", 0),      # the standard shape
 ]
 OUT_MODES = ["host", "device"]
-
-
-def _mem_available_bytes():
-    try:
-        with open("/proc/meminfo") as f:
-            for line in f:
-                if line.startswith("MemAvailable:"):
-                    return int(line.split()[1]) * 1024
-    except OSError:
-        pass
-    return 0
-
-
-def noncanonical(rng, shape):
-    a = rng.integers(0, 1 << 64, size=shape, dtype=np.uint64, endpoint=False)
-    hi = rng.random(shape) < 0.25
-    a[hi] = np.uint64(P) + (a[hi] % np.uint64((1 << 64) - P))
-    return a
 
 
 def _gate_set(name):
@@ -102,18 +85,6 @@ def L():
     p.shutdown()
 
 
-def _torch_u64(a):
-    import torch
-
-    return torch.from_numpy(np.ascontiguousarray(a).view(np.int64)).cuda()
-
-
-def _dev_table(tensors):
-    from plonky2_demo_b200 import _ffi
-
-    return (_ffi.u64p * len(tensors))(*[C.cast(C.c_void_p(t.data_ptr()), _ffi.u64p) for t in tensors])
-
-
 def _batches(case):
     import plonky2_demo_b200 as p
 
@@ -121,12 +92,6 @@ def _batches(case):
     cap_h = min(4, case.shape[0] + rate_bits)
     return [p.PolynomialBatch.from_coeffs(case.cs, rate_bits, False, cap_h),
             p.PolynomialBatch.from_coeffs(case.wires, rate_bits, case.salts is not None, cap_h, salts=case.salts)]
-
-
-def _free(*batches):
-    """free the batches now: a failing test's traceback would otherwise keep them alive past pcs_shutdown"""
-    for b in batches:
-        b.free()
 
 
 def _call(L, cs, w, gates, groups, nc, pih, alphas, D, flags, outs, lookups=0):
@@ -150,7 +115,7 @@ def _run(L, case, batches, out_mode):
     flags = _ffi.PCS_DEVICE_PTRS if out_mode == "device" else 0
     if out_mode == "device":
         o = torch.zeros((C_, M), dtype=torch.int64, device="cuda")
-        outs = _dev_table(list(o))
+        outs = dev_table(list(o))
     else:
         o = np.full((C_, M), 0xDEAD, dtype=np.uint64)
         outs = _ffi.ptr_array(list(o))
@@ -165,7 +130,7 @@ def _run(L, case, batches, out_mode):
 
 def _skip_if_short(shape):
     if shape[0] >= 20:
-        if _mem_available_bytes() < MIN_HOST_MEM:
+        if mem_available_bytes() < MIN_HOST_MEM:
             pytest.skip("not enough host memory for the oracle at the standard shape")
         import torch
 
@@ -182,7 +147,7 @@ def test_equals_oracle(L, shape, out_mode):
     try:
         rc, got = _run(L, case, batches, out_mode)
     finally:
-        _free(*batches)
+        free(*batches)
     assert rc == 0, L.pcs_last_error()
     assert got.shape == case.want.shape
     assert (got < np.uint64(P)).all()
@@ -199,7 +164,7 @@ def test_python_api(L):
     try:
         got = p.gate_constraint_terms(*batches, gates, info, case.nc, case.pih, case.alphas, case.shape[2])
     finally:
-        _free(*batches)
+        free(*batches)
     assert np.array_equal(got, case.want)
 
 
@@ -210,21 +175,6 @@ def _openings(L, h, w, z):
     out = np.empty((w, 2), dtype=np.uint64)
     _ffi.check(L.pcs_batch_eval_ext(h, _ffi.ptr(np.array([z.a, z.b], dtype=np.uint64)), _ffi.ptr(out)))
     return [Ext(int(a), int(b)) for a, b in out]
-
-
-def _e_pow(x, e):
-    r = Ext(1)
-    while e:
-        if e & 1:
-            r = r * x
-        x = x * x
-        e >>= 1
-    return r
-
-
-def _e_inv(x):
-    ni = pow((x.a * x.a - 7 * x.b * x.b) % P, P - 2, P)
-    return Ext(x.a * ni, (P - x.b) * ni)
 
 
 @pytest.mark.parametrize("lg_n", [12, 15])
@@ -254,19 +204,19 @@ def test_device_resident_chain(L, lg_n):
     h2, h3 = C.c_void_p(), C.c_void_p()
     try:
         W = C_ * K
-        w_dev = _torch_u64(wires)
+        w_dev = torch_u64(wires)
         zs_dev = torch.zeros((W, n), dtype=torch.int64, device="cuda")
         _ffi.check(L.pcs_permutation_partial_products(_ffi.dev_ptr_array(w_dev.data_ptr(), R, n),
-                                                      _ffi.dev_ptr_array(_torch_u64(sigmas).data_ptr(), R, n), R, lg_n,
+                                                      _ffi.dev_ptr_array(torch_u64(sigmas).data_ptr(), R, n), R, lg_n,
                                                       _ffi.ptr(k_is), _ffi.ptr(betas), _ffi.ptr(gammas), C_, D,
                                                       _ffi.PCS_DEVICE_PTRS, _ffi.dev_ptr_array(zs_dev.data_ptr(), W, n)))
         _ffi.check(L.pcs_commit_from_values(_ffi.dev_ptr_array(zs_dev.data_ptr(), W, n), W, lg_n, rate_bits, cap_h, None, 0,
                                             _ffi.PCS_DEVICE_PTRS | _ffi.PCS_KEEP_COEFFS, None, None, C.byref(h2)))
         gt = torch.zeros((C_, M), dtype=torch.int64, device="cuda")
-        _ffi.check(_call(L, b_cs._h, b_w._h, gates, groups, nc, inst["pih"], alphas, D, _ffi.PCS_DEVICE_PTRS, _dev_table(list(gt))))
+        _ffi.check(_call(L, b_cs._h, b_w._h, gates, groups, nc, inst["pih"], alphas, D, _ffi.PCS_DEVICE_PTRS, dev_table(list(gt))))
         q_dev = torch.zeros((C_ * D, n), dtype=torch.int64, device="cuda")
         _ffi.check(L.pcs_quotient_polys(b_cs._h, b_w._h, h2, nc, R, _ffi.ptr(k_is), _ffi.ptr(betas), _ffi.ptr(gammas),
-                                        _ffi.ptr(alphas), C_, D, _dev_table(list(gt)), _ffi.PCS_DEVICE_PTRS,
+                                        _ffi.ptr(alphas), C_, D, dev_table(list(gt)), _ffi.PCS_DEVICE_PTRS,
                                         _ffi.dev_ptr_array(q_dev.data_ptr(), C_ * D, n)))
         _ffi.check(L.pcs_commit_from_coeffs(_ffi.dev_ptr_array(q_dev.data_ptr(), C_ * D, n), C_ * D, lg_n, rate_bits, cap_h, None,
                                             0, _ffi.PCS_DEVICE_PTRS | _ffi.PCS_KEEP_COEFFS, None, C.byref(h3)))
@@ -282,9 +232,9 @@ def test_device_resident_chain(L, lg_n):
         w_o, cs_o = _openings(L, b_w._h, 135, zeta), _openings(L, b_cs._h, nc + R, zeta)
         z_o, z_go = _openings(L, h2, W, zeta), _openings(L, h2, W, zeta * g)
         q_o = _openings(L, h3, C_ * D, zeta)
-        zn = _e_pow(zeta, n)
+        zn = zeta.pow(n)
         zh = zn - 1
-        l_0 = zh * _e_inv(Ext(n) * (zeta - 1))
+        l_0 = zh * (Ext(n) * (zeta - 1)).inv()
         Pn = K - 1
         terms = [l_0 * (z_o[c] - 1) for c in range(C_)]
         for c in range(C_):
@@ -312,16 +262,16 @@ def test_device_resident_chain(L, lg_n):
 
         # one changed wire: the gate terms no longer vanish on H, and the quotient's trim fails
         _ffi.check(_call(L, b_cs._h, b_bad._h, gates, groups, nc, inst["pih"], alphas, D, _ffi.PCS_DEVICE_PTRS,
-                         _dev_table(list(gt))))
+                         dev_table(list(gt))))
         rc = L.pcs_quotient_polys(b_cs._h, b_bad._h, h2, nc, R, _ffi.ptr(k_is), _ffi.ptr(betas), _ffi.ptr(gammas),
-                                  _ffi.ptr(alphas), C_, D, _dev_table(list(gt)), _ffi.PCS_DEVICE_PTRS,
+                                  _ffi.ptr(alphas), C_, D, dev_table(list(gt)), _ffi.PCS_DEVICE_PTRS,
                                   _ffi.dev_ptr_array(q_dev.data_ptr(), C_ * D, n))
         assert rc == -5
         assert L.pcs_last_error() == qo.QUOTIENT_FAILED.encode()
     finally:
         L.pcs_batch_free(h2)
         L.pcs_batch_free(h3)
-        _free(b_cs, b_w, b_bad)
+        free(b_cs, b_w, b_bad)
 
 
 # ---- argument errors ---------------------------------------------------------------------------------------------------------
@@ -331,7 +281,7 @@ def _normal_call_works(L):
     try:
         rc, got = _run(L, case, batches, "host")
     finally:
-        _free(*batches)
+        free(*batches)
     assert rc == 0, L.pcs_last_error()
     assert np.array_equal(got, case.want)
 
@@ -408,4 +358,4 @@ def test_argument_errors(L):
     finally:
         L.pcs_batch_free(shard)
         L.pcs_batch_free(rows_only)
-        _free(*bs, narrow, other_degree, other_rate, on_demand)
+        free(*bs, narrow, other_degree, other_rate, on_demand)

@@ -13,7 +13,7 @@ import numpy as np
 import pytest
 
 import oracle
-from helpers import P, as_oracle_proof, assert_same_proof, brev, seeded_polys, splitmix64_stream
+from helpers import P, as_oracle_proof, assert_same_proof, brev, mem_available_bytes, seeded_polys, splitmix64_stream
 from oracle import fri_ref as fr
 
 pytestmark = pytest.mark.gpu
@@ -367,17 +367,6 @@ def test_headline_shape_matches_resident_commit(L):
         L.pcs_batch_free(hr)
 
 
-def _mem_available_bytes():
-    try:
-        with open("/proc/meminfo") as f:
-            for line in f:
-                if line.startswith("MemAvailable:"):
-                    return int(line.split()[1]) * 1024
-    except OSError:
-        pass
-    return 0
-
-
 def test_large_commit_on_one_gpu(L):
     """135 x 2^24 at rate 3: 145 GB of LDE rows as a resident batch, which does not fit one B200.  Rows equal direct
     evaluation and Merkle paths verify against the cap.  Then configs[4]'s opening proof over it (bench.py's instance at
@@ -396,7 +385,7 @@ def test_large_commit_on_one_gpu(L):
 
     w, lg_d, r, cap_h = 135, 24, 3, 4
     d, n = 1 << lg_d, 1 << (lg_d + r)
-    free, host_mem = torch.cuda.mem_get_info()[0], _mem_available_bytes()
+    free, host_mem = torch.cuda.mem_get_info()[0], mem_available_bytes()
     if free < (80 << 30):
         pytest.skip(f"135 x 2^24 on demand needs 80 GiB of free HBM ({free >> 30} GiB free)")
     if host_mem < (40 << 30):

@@ -13,6 +13,7 @@ import oracle
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "harness"))
 import permutation_oracle as po  # noqa: E402
+from helpers import dev_table, noncanonical, torch_u64  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 
@@ -30,13 +31,6 @@ SHAPES = [   # (R, lg_n, C, D)
     (80, 20, 2, 8),    # the benchmark shape
 ]
 MODES = ["host", "device", "scattered"]
-
-
-def noncanonical(rng, shape):
-    a = rng.integers(0, 1 << 64, size=shape, dtype=np.uint64, endpoint=False)
-    hi = rng.random(shape) < 0.25
-    a[hi] = np.uint64(P) + (a[hi] % np.uint64((1 << 64) - P))
-    return a
 
 
 @functools.lru_cache(maxsize=2)
@@ -59,18 +53,6 @@ def L():
     p.shutdown()
 
 
-def _torch_u64(a):
-    import torch
-
-    return torch.from_numpy(np.ascontiguousarray(a).view(np.int64)).cuda()
-
-
-def _dev_table(tensors):
-    from plonky2_demo_b200 import _ffi
-
-    return (_ffi.u64p * len(tensors))(*[C.cast(C.c_void_p(t.data_ptr()), _ffi.u64p) for t in tensors])
-
-
 def _run(L, mode, wires, sigmas, k_is, betas, gammas, D, W):
     """-> (rc, [W][n] result as numpy)"""
     from plonky2_demo_b200 import _ffi
@@ -87,13 +69,13 @@ def _run(L, mode, wires, sigmas, k_is, betas, gammas, D, W):
     import torch
 
     if mode == "device":
-        w, s = _torch_u64(wires), _torch_u64(sigmas)
+        w, s = torch_u64(wires), torch_u64(sigmas)
         o = torch.zeros((W, n), dtype=torch.int64, device="cuda")
-        tw, ts, to = _dev_table(list(w)), _dev_table(list(s)), _dev_table(list(o))
+        tw, ts, to = dev_table(list(w)), dev_table(list(s)), dev_table(list(o))
     else:   # every column its own allocation
-        w, s = [_torch_u64(c) for c in wires], [_torch_u64(c) for c in sigmas]
+        w, s = [torch_u64(c) for c in wires], [torch_u64(c) for c in sigmas]
         o = [torch.zeros(n, dtype=torch.int64, device="cuda") for _ in range(W)]
-        tw, ts, to = _dev_table(w), _dev_table(s), _dev_table(o)
+        tw, ts, to = dev_table(w), dev_table(s), dev_table(o)
     rc = L.pcs_permutation_partial_products(tw, ts, R, lg_n, *scalars, _ffi.PCS_DEVICE_PTRS, to)
     torch.cuda.synchronize()
     res = (o if mode == "device" else torch.stack(o)).cpu().numpy().view(np.uint64)
@@ -140,8 +122,8 @@ def test_device_resident_chain(L):
     sigmas = noncanonical(rng, (R, n))
     k_is = p.get_unique_coset_shifts(n, R)
     betas, gammas = noncanonical(rng, C_), noncanonical(rng, C_)
-    w_dev = _torch_u64(wires)
-    s_dev = _torch_u64(sigmas)
+    w_dev = torch_u64(wires)
+    s_dev = torch_u64(sigmas)
     b1 = C.c_void_p()
     cap1 = np.empty((1 << cap_height, 4), dtype=np.uint64)
     _ffi.check(L.pcs_commit_from_values(_ffi.dev_ptr_array(w_dev.data_ptr(), num_wires, n), num_wires, lg_n, rate_bits, cap_height,

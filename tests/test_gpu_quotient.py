@@ -19,6 +19,7 @@ import oracle
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "harness"))
 import permutation_oracle as po  # noqa: E402
 import quotient_oracle as qo  # noqa: E402
+from helpers import Ext, dev_table, free, mem_available_bytes, noncanonical, torch_u64  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 
@@ -37,24 +38,6 @@ SHAPES = [   # (R, lg_n, C, D, rate_bits, num_constants, wires_w, salt_w)
     (80, 20, 2, 8, 3, 0, 80, 0),     # the standard shape
 ]
 MODES = [("none", "host"), ("host", "host"), ("device", "device"), ("none", "device")]   # (tail, outputs)
-
-
-def _mem_available_bytes():
-    try:
-        with open("/proc/meminfo") as f:
-            for line in f:
-                if line.startswith("MemAvailable:"):
-                    return int(line.split()[1]) * 1024
-    except OSError:
-        pass
-    return 0
-
-
-def noncanonical(rng, shape):
-    a = rng.integers(0, 1 << 64, size=shape, dtype=np.uint64, endpoint=False)
-    hi = rng.random(shape) < 0.25
-    a[hi] = np.uint64(P) + (a[hi] % np.uint64((1 << 64) - P))
-    return a
 
 
 def _m(lg_n, D):
@@ -98,18 +81,6 @@ def L():
     p.shutdown()
 
 
-def _torch_u64(a):
-    import torch
-
-    return torch.from_numpy(np.ascontiguousarray(a).view(np.int64)).cuda()
-
-
-def _dev_table(tensors):
-    from plonky2_demo_b200 import _ffi
-
-    return (_ffi.u64p * len(tensors))(*[C.cast(C.c_void_p(t.data_ptr()), _ffi.u64p) for t in tensors])
-
-
 def _batches(case):
     import plonky2_demo_b200 as p
 
@@ -117,12 +88,6 @@ def _batches(case):
     cap_h = min(4, case.shape[1] + rate_bits)
     return [p.PolynomialBatch.from_coeffs(c, rate_bits, s is not None, cap_h, salts=s)
             for c, s in zip((case.cs, case.wires, case.zs), case.salts)]
-
-
-def _free(*batches):
-    """free the batches now: a failing test's traceback would otherwise keep them alive past pcs_shutdown"""
-    for b in batches:
-        b.free()
 
 
 def _call(L, batches, case, betas, gammas, alphas, tail, out_tables, flags, D=None):
@@ -147,13 +112,13 @@ def _run(L, case, batches, tail_mode, out_mode):
     flags = _ffi.PCS_DEVICE_PTRS if out_mode == "device" else 0
     if out_mode == "device":
         o = torch.zeros((W, n), dtype=torch.int64, device="cuda")
-        outs = _dev_table(list(o))
+        outs = dev_table(list(o))
     else:
         o = np.full((W, n), 0xDEAD, dtype=np.uint64)
         outs = _ffi.ptr_array(list(o))
     if tail_mode == "device":
-        t_dev, d_dev = _torch_u64(case.tail), _torch_u64(decoy_tail)
-        tails, dtails = _dev_table(list(t_dev)), _dev_table(list(d_dev))
+        t_dev, d_dev = torch_u64(case.tail), torch_u64(decoy_tail)
+        tails, dtails = dev_table(list(t_dev)), dev_table(list(d_dev))
     elif tail_mode == "host":
         tails, dtails = _ffi.ptr_array(list(case.tail)), _ffi.ptr_array(list(decoy_tail))
     else:
@@ -168,7 +133,7 @@ def _run(L, case, batches, tail_mode, out_mode):
 
 def _skip_if_short(shape):
     if shape[1] >= 20:
-        if _mem_available_bytes() < MIN_HOST_MEM:
+        if mem_available_bytes() < MIN_HOST_MEM:
             pytest.skip("not enough host memory for the oracle at the standard shape")
         import torch
 
@@ -185,7 +150,7 @@ def test_equals_oracle(L, shape, mode):
     try:
         rc, got = _run(L, case, batches, *mode)
     finally:
-        _free(*batches)
+        free(*batches)
     assert rc == 0, L.pcs_last_error()
     want = case.want[mode[0] != "none"]
     assert got.shape == want.shape
@@ -204,7 +169,7 @@ def test_python_api(L):
         chunks = p.quotient_poly_chunks(*batches, *args, gate_terms=case.tail)
         full = p.compute_quotient_polys(*batches, *args)
     finally:
-        _free(*batches)
+        free(*batches)
     assert np.array_equal(chunks, case.want[True])
     assert full.shape == (C_, _m(lg_n, D))
     assert np.array_equal(full[:, :D << lg_n].reshape(C_ * D, -1), case.want[False])
@@ -212,44 +177,12 @@ def test_python_api(L):
 
 
 # ---- extension-field arithmetic for the verifier's identity: F[X] / (X^2 - 7) ---------------------------------------------
-def e_add(a, b):
-    return ((a[0] + b[0]) % P, (a[1] + b[1]) % P)
-
-
-def e_sub(a, b):
-    return ((a[0] - b[0]) % P, (a[1] - b[1]) % P)
-
-
-def e_mul(a, b):
-    return ((a[0] * b[0] + 7 * a[1] * b[1]) % P, (a[0] * b[1] + a[1] * b[0]) % P)
-
-
-def e_pow(a, e):
-    r = (1, 0)
-    while e:
-        if e & 1:
-            r = e_mul(r, a)
-        a = e_mul(a, a)
-        e >>= 1
-    return r
-
-
-def e_inv(a):
-    norm = (a[0] * a[0] - 7 * a[1] * a[1]) % P
-    ni = pow(norm, P - 2, P)
-    return (a[0] * ni % P, (P - a[1]) * ni % P)
-
-
-def e_base(v):
-    return (int(v) % P, 0)
-
-
 def _openings(L, batch, z):
     from plonky2_demo_b200 import _ffi
 
     out = np.empty((batch.n_polys, 2), dtype=np.uint64)
-    _ffi.check(L.pcs_batch_eval_ext(batch._h, _ffi.ptr(np.array(z, dtype=np.uint64)), _ffi.ptr(out)))
-    return [(int(a), int(b)) for a, b in out]
+    _ffi.check(L.pcs_batch_eval_ext(batch._h, _ffi.ptr(np.array([z.a, z.b], dtype=np.uint64)), _ffi.ptr(out)))
+    return [Ext(int(a), int(b)) for a, b in out]
 
 
 def test_device_resident_chain(L):
@@ -269,14 +202,14 @@ def test_device_resident_chain(L):
     betas, gammas, alphas = (rng.integers(1, P, C_, dtype=np.uint64) for _ in range(3))
     consts = rng.integers(0, P, (nc, n), dtype=np.uint64)
     b_cs = p.PolynomialBatch.from_values(np.vstack([consts, sigmas]), rate_bits, False, cap_h)
-    w_dev = _torch_u64(wires)
+    w_dev = torch_u64(wires)
     b_w = p.PolynomialBatch.from_values(wires, rate_bits, False, cap_h)   # commitment #1
     h2, h3 = C.c_void_p(), C.c_void_p()
     try:
         W = C_ * K
         zs_dev = torch.zeros((W, n), dtype=torch.int64, device="cuda")
         _ffi.check(L.pcs_permutation_partial_products(_ffi.dev_ptr_array(w_dev.data_ptr(), R, n),
-                                                      _ffi.dev_ptr_array(_torch_u64(sigmas).data_ptr(), R, n), R, lg_n,
+                                                      _ffi.dev_ptr_array(torch_u64(sigmas).data_ptr(), R, n), R, lg_n,
                                                       _ffi.ptr(k_is), _ffi.ptr(betas), _ffi.ptr(gammas), C_, D,
                                                       _ffi.PCS_DEVICE_PTRS, _ffi.dev_ptr_array(zs_dev.data_ptr(), W, n)))
         _ffi.check(L.pcs_commit_from_values(_ffi.dev_ptr_array(zs_dev.data_ptr(), W, n), W, lg_n, rate_bits, cap_h, None, 0,
@@ -295,9 +228,9 @@ def test_device_resident_chain(L):
         assert np.array_equal(cap3, oracle.commit_from_coeffs(chunks, rate_bits, cap_h)["cap"])
 
         # vanishing(zeta) = Z_H(zeta) sum_k zeta^(k n) chunk_k(zeta), every value an opening of a committed batch
-        zeta = (int(rng.integers(2, P, dtype=np.uint64)), int(rng.integers(1, P, dtype=np.uint64)))
+        zeta = Ext(int(rng.integers(2, P, dtype=np.uint64)), int(rng.integers(1, P, dtype=np.uint64)))
         g = pow(1753635133440165772, 1 << (32 - lg_n), P)
-        zeta_g = e_mul(zeta, e_base(g))
+        zeta_g = zeta * g
         w_o, s_o = _openings(L, b_w, zeta)[:R], _openings(L, b_cs, zeta)[nc:nc + R]
 
         class _B:   # the raw commitment #2 / #3 handles
@@ -306,41 +239,39 @@ def test_device_resident_chain(L):
 
         z_o, z_go = _openings(L, _B(h2, W), zeta), _openings(L, _B(h2, W), zeta_g)
         q_o = _openings(L, _B(h3, C_ * D), zeta)
-        zh = e_sub(e_pow(zeta, n), (1, 0))
-        l_0 = e_mul(zh, e_inv(e_mul(e_base(n), e_sub(zeta, (1, 0)))))
+        zn = zeta.pow(n)
+        zh = zn - 1
+        l_0 = zh * (Ext(n) * (zeta - 1)).inv()
         Pn = K - 1
-        terms = []
+        terms = [l_0 * (z_o[c] - 1) for c in range(C_)]
         for c in range(C_):
-            terms.append(e_mul(l_0, e_sub(z_o[c], (1, 0))))
-        for c in range(C_):
-            b, gm = e_base(betas[c]), e_base(gammas[c])
-            num = [e_add(e_add(w_o[j], e_mul(b, e_mul(e_base(k_is[j]), zeta))), gm) for j in range(R)]
-            den = [e_add(e_add(w_o[j], e_mul(b, s_o[j])), gm) for j in range(R)]
+            b, gm = int(betas[c]), int(gammas[c])
+            num = [w_o[j] + b * (int(k_is[j]) * zeta) + gm for j in range(R)]
+            den = [w_o[j] + b * s_o[j] + gm for j in range(R)]
             acc, chain = z_o[c], z_o[C_ + c * Pn:C_ + (c + 1) * Pn] + [z_go[c]]
             for k in range(K):
-                nk, dk = (1, 0), (1, 0)
+                nk, dk = Ext(1), Ext(1)
                 for v in num[k * D:(k + 1) * D]:
-                    nk = e_mul(nk, v)
+                    nk = nk * v
                 for v in den[k * D:(k + 1) * D]:
-                    dk = e_mul(dk, v)
-                terms.append(e_sub(e_mul(acc, nk), e_mul(chain[k], dk)))
+                    dk = dk * v
+                terms.append(acc * nk - chain[k] * dk)
                 acc = chain[k]
-        zn = e_pow(zeta, n)
         for a in range(C_):
-            al = e_base(alphas[a])
-            van = (0, 0)
+            al = int(alphas[a])
+            van = Ext(0)
             for t in reversed(terms):
-                van = e_add(e_mul(van, al), t)
-            tq, zk = (0, 0), (1, 0)
+                van = van * al + t
+            tq, zk = Ext(0), Ext(1)
             for k in range(D):
-                tq = e_add(tq, e_mul(zk, q_o[a * D + k]))
-                zk = e_mul(zk, zn)
-            assert van == e_mul(zh, tq), a
+                tq = tq + zk * q_o[a * D + k]
+                zk = zk * zn
+            assert van == zh * tq, a
         assert np.array_equal(w_dev.cpu().numpy().view(np.uint64), wires)
     finally:
         L.pcs_batch_free(h2)
         L.pcs_batch_free(h3)
-        _free(b_cs, b_w)
+        free(b_cs, b_w)
 
 
 def _normal_call_works(L):
@@ -349,7 +280,7 @@ def _normal_call_works(L):
     try:
         rc, got = _run(L, case, batches, "host", "host")
     finally:
-        _free(*batches)
+        free(*batches)
     assert rc == 0, L.pcs_last_error()
     assert np.array_equal(got, case.want[True])
 
@@ -405,7 +336,7 @@ def test_argument_errors(L):
     finally:
         L.pcs_batch_free(shard)
         L.pcs_batch_free(rows_only)
-        _free(*bs, other_degree, other_rate, on_demand)
+        free(*bs, other_degree, other_rate, on_demand)
 
 
 @pytest.mark.parametrize("out_mode", ["host", "device"])
@@ -427,7 +358,7 @@ def test_trim_failure(L, out_mode):
         import torch
 
         o = torch.zeros((C_ * D, n), dtype=torch.int64, device="cuda")
-        outs, flags = _dev_table(list(o)), _ffi.PCS_DEVICE_PTRS
+        outs, flags = dev_table(list(o)), _ffi.PCS_DEVICE_PTRS
     else:
         o = np.empty((C_ * D, n), dtype=np.uint64)
         outs, flags = _ffi.ptr_array(list(o)), 0
@@ -435,7 +366,7 @@ def test_trim_failure(L, out_mode):
         rc = L.pcs_quotient_polys(bs[0]._h, bs[1]._h, bs[2]._h, 0, R, _ffi.ptr(k_is), _ffi.ptr(betas), _ffi.ptr(gammas),
                                   _ffi.ptr(alphas), C_, D, None, flags, outs)
     finally:
-        _free(*bs)
+        free(*bs)
     assert rc == -5
     assert L.pcs_last_error() == b"Quotient has failed, the vanishing polynomial is not divisible by Z_H"
     _normal_call_works(L)

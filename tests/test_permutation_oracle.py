@@ -16,6 +16,7 @@ import pytest
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "harness"))
 
 import permutation_oracle as po  # noqa: E402
+from helpers import noncanonical  # noqa: E402
 
 P = 0xFFFFFFFF00000001
 GEN = 1753635133440165772   # POWER_OF_TWO_GENERATOR
@@ -72,14 +73,6 @@ def wires_permutation_partial_products_and_zs(wires, sigmas, k_is, beta, gamma, 
 def big_reference(wires, sigmas, k_is, betas, gammas, degree_factor):
     return np.stack([wires_permutation_partial_products_and_zs(wires, sigmas, k_is, int(b) % P, int(g) % P, degree_factor)
                      for b, g in zip(betas, gammas)])
-
-
-def noncanonical(rng, shape):
-    """uniform u64 with a share of values in [p, 2^64) (the reference's loose representation)"""
-    a = rng.integers(0, 1 << 64, size=shape, dtype=np.uint64, endpoint=False)
-    hi = rng.random(shape) < 0.25
-    a[hi] = np.uint64(P) + (a[hi] % np.uint64((1 << 64) - P))
-    return a
 
 
 SHAPES = [   # (R, lg_n, C, D)

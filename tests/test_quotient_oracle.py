@@ -19,7 +19,8 @@ sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "har
 
 import permutation_oracle as po  # noqa: E402
 import quotient_oracle as qo  # noqa: E402
-from test_permutation_oracle import copy_constrained_witness, noncanonical  # noqa: E402
+from helpers import noncanonical  # noqa: E402
+from test_permutation_oracle import copy_constrained_witness  # noqa: E402
 
 P = 0xFFFFFFFF00000001
 GEN = 1753635133440165772   # POWER_OF_TWO_GENERATOR
